@@ -2,7 +2,7 @@
 """bench.py - particle events/s of neutral's particle-history hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
-                    [--deck csp] [--particles P] [--scaling weak|strong]
+                    [--deck csp] [--particles P] [--scaling weak|strong] [--dump-outputs DIR]
 
 One "step" = one complete run of the deck named in ``config.workload`` (default csp: 4000 x
 4000 mesh, 1e6 particles per GPU, 10 timesteps of solve_transport_2d) from the freshly
@@ -53,6 +53,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the source tree
 
 METRIC = "particle_events_per_sec"
 UNIT = "events/s"
@@ -80,7 +81,12 @@ def parse_args():
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--no-decks", action="store_true")
     ap.add_argument("--opts", default="", help="library options, e.g. pipeline=0,fast_div=0")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    return args
 
 
 def workload_config(deck, nglobal: int, world: int, scaling: str):
@@ -353,6 +359,34 @@ def parity_report(deck, nglobal, counts_global, tally, bank_hashes, live):
     return rep
 
 
+DUMP_SAMPLE = 1 << 18  # particles and tally cells sampled per dump (fixed seed): ~20 MB in all
+
+
+def dump_outputs(out_dir, deck, last_run, bank, tally):
+    """Writes what the last timed step returned to its caller as DIR/<name>.npy (float64): the
+    per-timestep counts, the tally and every bank field - the larger arrays as a fixed, seeded
+    sample of indices (written beside them) plus the tally's 64 x 64 block sums, so that two
+    builds can be compared output for output on the same inputs."""
+    os.makedirs(out_dir, exist_ok=True)
+
+    def sample(n):
+        if n <= DUMP_SAMPLE:
+            return np.arange(n)
+        return np.sort(np.random.default_rng(0).choice(n, DUMP_SAMPLE, replace=False))
+
+    out = {"counts": np.array([[r.facets, r.collisions, r.processed, r.census, r.deaths]
+                               for r in last_run], dtype=np.float64),
+           "tally_block_sums": block_sums(tally, deck.nx, deck.ny)}
+    cells = sample(tally.size)
+    out["tally_sample_index"], out["tally_sample"] = cells.astype(np.float64), tally[cells]
+    pids = sample(len(bank))
+    out["bank_sample_index"] = pids.astype(np.float64)
+    for k, a in bank.arrays.items():
+        out[f"bank_{k}"] = a[pids].astype(np.float64)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def connect_group(lib, dist, torch, world, rank, ncells):
     """One library-side tally group over the ranks of this job: every rank allocates its slab,
     the CUDA-IPC handles travel through torch.distributed, every rank maps its peers."""
@@ -525,6 +559,9 @@ def run_b200_arm(args, rank: int, local_rank: int, world: int):
     alg_bytes = algorithmic_bytes(timed)
     reductions = sum(r.facets + r.census + r.deaths for r in timed)
     collisions = sum(r.collisions for r in timed)
+    if args.dump_outputs and rank == 0:  # a sharded run dumps rank 0's part of the bank
+        dump_outputs(args.dump_outputs, d, timed[-d.iterations:], sim.bank_to_host(),
+                     sim.tally_to_host())
 
     stage("parity")
     # ---- parity of the timed runs themselves (outside the timed region) ----------------

@@ -1,7 +1,7 @@
-"""Parity of the CUDA path (through the C-ABI) against the oracle port, the committed golden
-vectors of the reference build and - when its prebuilt library travelled - the unmodified
-reference itself. Bars (BASELINE.json north_star): per-particle event counts and every
-particle field bit-exact; tally within 1e-10 relative per cell (atomic summation order)."""
+"""Parity of the CUDA path (through the C-ABI) against the oracle port and the committed golden
+vectors of the reference build (whole runs and step by step). Bars (BASELINE.json north_star):
+per-particle event counts and every particle field bit-exact; tally within 1e-10 relative per
+cell (atomic summation order)."""
 import hashlib
 import os
 
@@ -12,6 +12,7 @@ from conftest import SMALL_DECKS
 from neutral_b200.bank import ALL_FIELDS, HostBank
 from neutral_b200.decks import build_problem
 from neutral_b200.host import NB200_BAD_OPTION, Simulation, solve_transport_2d_host
+from recorded import field_hashes, reference_run
 
 pytestmark = pytest.mark.gpu
 
@@ -107,19 +108,21 @@ def test_device_flavour_matches_golden(gpu_lib, deck, mode):
 
 
 @pytest.mark.parametrize("deck", ["mixed_small", "csp_small"])
-def test_host_flavour_is_a_drop_in_for_omp3(gpu_lib, port, ref, deck):
-    """Same call, same host arrays: reference omp3 library vs nb200_solve_transport_2d_host."""
+def test_host_flavour_is_a_drop_in_for_omp3(gpu_lib, port, deck):
+    """Same call, same host arrays: nb200_solve_transport_2d_host against the reference omp3
+    run recorded in tests/golden/steps.json, timestep by timestep."""
     prob = build_problem(deck)
     d = prob.deck
-    aos_ref = ref.inject(prob)
-    aos_gpu = aos_ref.copy()
-    t_ref, t_gpu = np.zeros(d.nx * d.ny), np.zeros(d.nx * d.ny)
+    want = reference_run(deck)
+    aos_gpu = port.inject(prob).to_aos()
+    assert field_hashes(HostBank.from_aos(aos_gpu)) == want["hashes"][0]
+    t_gpu = np.zeros(d.nx * d.ny)
     for tt in range(1, d.iterations + 1):
-        want = ref.step(prob, aos_ref, tt, t_ref)
         got = solve_transport_2d_host(prob, aos_gpu, tt, t_gpu)
-        assert want == got
-        assert sum(HostBank.from_aos(aos_ref).bit_equal(HostBank.from_aos(aos_gpu)).values()) == 0
-        assert tally_close(t_ref, t_gpu)
+        assert list(got) == want["counts"][tt - 1]
+        assert field_hashes(HostBank.from_aos(aos_gpu)) == want["hashes"][tt]
+        assert tally_close(np.array([t_gpu.sum()]), np.array([want["tally_sums"][tt - 1]]))
+    assert tally_close(np.load(os.path.join(GOLDEN, f"{deck}.npz"))["tally"], t_gpu)
 
 
 def test_host_flavour_matches_oracle(gpu_lib, port):
@@ -221,13 +224,13 @@ def test_deferred_step_and_async_fold(gpu_lib, port):
 
 
 @pytest.mark.parametrize("deck", ["csp_small", "split_small"])
-def test_device_inject_equals_host_inject(gpu_lib, port, ref, deck):
-    """inject_particles on the device (default), on the host with libm (device_inject=0), the
-    oracle port and the unmodified reference all produce the same bank, bit for bit - whole
-    and as shards (global RNG keys)."""
+def test_device_inject_equals_host_inject(gpu_lib, port, deck):
+    """inject_particles on the device (default), on the host with libm (device_inject=0) and
+    the oracle port, whose bank is pinned by tests/golden/steps.json, all produce the same
+    bank, bit for bit - whole and as shards (global RNG keys)."""
     prob = build_problem(deck, nparticles=50_000)
     want = port.inject(prob)
-    assert sum(HostBank.from_aos(ref.inject(prob)).bit_equal(want).values()) == 0
+    assert field_hashes(want) == reference_run(f"{deck}@50000")["hashes"][0]
     for device_inject in (1, 0):
         gpu_lib.nb200_set_option(b"device_inject", device_inject)
         try:

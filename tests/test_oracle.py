@@ -1,6 +1,6 @@
-"""Pins the oracle port: against the UNMODIFIED reference omp3 build (when its prebuilt
-library is present) and against the committed golden vectors generated from that build
-(tests/golden/make_golden.py) - bit-exact particle state, exact counts, tally to 1e-12."""
+"""Pins the oracle port against the committed golden vectors of the UNMODIFIED reference omp3
+build (tests/golden/make_golden.py, make_golden_steps.py) - bit-exact particle state, exact
+counts, tally to 1e-12."""
 import hashlib
 import os
 
@@ -8,8 +8,9 @@ import numpy as np
 import pytest
 
 from conftest import SMALL_DECKS
-from neutral_b200.bank import ALL_FIELDS, HostBank
+from neutral_b200.bank import ALL_FIELDS
 from neutral_b200.decks import build_problem, shard_range
+from recorded import field_hashes, reference_run
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
@@ -49,18 +50,22 @@ def test_port_matches_golden(port, deck):
 
 
 @pytest.mark.parametrize("deck", SMALL_DECKS)
-def test_port_matches_reference_build(port, ref, deck):
+def test_port_matches_reference_build(port, deck):
+    """Every timestep against the reference run recorded in tests/golden/steps.json: exact
+    counts, every particle field bit for bit, the tally's sum; the final tally cell by cell to
+    1e-12."""
     prob = build_problem(deck)
     d = prob.deck
-    aos = ref.inject(prob)
+    want = reference_run(deck)
     bank = port.inject(prob)
-    assert sum(HostBank.from_aos(aos).bit_equal(bank).values()) == 0
-    t_ref, t_port = np.zeros(d.nx * d.ny), np.zeros(d.nx * d.ny)
+    assert field_hashes(bank) == want["hashes"][0]
+    t_port = np.zeros(d.nx * d.ny)
     for tt in range(1, d.iterations + 1):
-        f, c = ref.step(prob, aos, tt, t_ref)
         pf, pc, _ = port.step(prob, bank, tt, t_port)
-        assert (f, c) == (pf, pc)
-        assert sum(HostBank.from_aos(aos).bit_equal(bank).values()) == 0
+        assert [pf, pc] == want["counts"][tt - 1]
+        assert field_hashes(bank) == want["hashes"][tt]
+        assert abs(t_port.sum() - want["tally_sums"][tt - 1]) <= 1e-12 * abs(t_port.sum())
+    t_ref = np.load(os.path.join(GOLDEN, f"{deck}.npz"))["tally"]
     assert np.all(np.abs(t_ref - t_port) <= 1e-12 * np.maximum(np.abs(t_ref), np.abs(t_port)))
 
 
