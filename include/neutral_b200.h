@@ -127,7 +127,9 @@ size_t inject_particles(const int nparticles, const int global_nx, const int loc
  * (neutral_interface.h:35-36 / omp3/neutral.c:520-557); same printed lines. When the
  * environment names a file in NB200_RESULTS_JSON the verdict is also written there as JSON:
  * deck, tally total, expected value, relative error, PASSED / FAILED / NOT_VALIDATED and the
- * per-timestep counts the library saw (SURVEY.md 8f 1). */
+ * per-timestep counts the library saw (SURVEY.md 8f 1). When the tally was deposited by a bank
+ * with tally batches (section 6) the JSON also has "tally_batches": B and
+ * "tally_total_relative_error": R of the total. */
 void validate(const int nx, const int ny, const char* params_filename, const int rank,
               double* energy_tally);
 
@@ -270,12 +272,16 @@ int nb200_accumulate_clear_async(double* dst_device, double* src_device, size_t 
  * kernels, same order, same results; 0: the ~23 driver calls are issued one by one. The
  * occupancy / L2 probes "history_smem_pad", "l2_persist" and "pipeline" = 0 always take the
  * call-by-call path).
+ * "tally_batches" (0, default: off; 2..64: the NEXT inject_particles / nb200_bank_create makes a
+ * bank whose tally carries B independent batch estimates, section 6; environment
+ * NB200_TALLY_BATCHES=<B> sets the default; 1 is refused: one batch has no spread).
  * "tally_prereduce" = 1 implies "fast_div" = 1 (it has no separate IEEE-division build); it
  * is an experiment kept for the record (measured slower): its peer mask is the opportunistic
  * __activemask() pattern, which CUDA does not guarantee to be the converged set.
  * Options are process-wide defaults; nb200_bank_set_option overrides one for one bank (the
- * creation-time options ngpus / host_mirror / headroom_pct / device_inject apply when the bank
- * is created). Returns the previous value, or NB200_BAD_OPTION for an unknown name or a value
+ * creation-time options ngpus / host_mirror / headroom_pct / device_inject / tally_batches
+ * apply when the bank is created; nb200_bank_set_option refuses tally_batches, and pipeline = 0
+ * or tally_prereduce = 1 on a bank with tally batches). Returns the previous value, or NB200_BAD_OPTION for an unknown name or a value
  * outside the option's range (nb200_last_error says which). */
 int nb200_set_option(const char* name, int value);
 int nb200_get_option(const char* name);
@@ -330,6 +336,35 @@ int nb200_tally_sync(double* tally_device);
  * caller has changed such an array in place. */
 int nb200_update_replicas(void);
 
+/* ------------------------------------------------------------------------------------
+ * 6. Tally batches: a relative error beside every tally cell. A bank created with option
+ *    "tally_batches" = B splits its N particles into B contiguous ranges of global particle
+ *    index, omp3's thread split (batch b starts at b*(N/B) + min(b, N%B) and holds
+ *    n_b = N/B + (b < N%B) particles). Every deposit goes to the partial tally S_b of the
+ *    depositing particle's batch; histories, counts and the bank are exactly those of the
+ *    unbatched run. The caller's tally receives what the batches gained lazily, wherever a
+ *    sharded run's tally would (validate, copy_buffer RECV, nb200_memcpy_* / nb200_memset_d of
+ *    it, nb200_tally_sync, nb200_bank_free, and the two calls below); afterwards it equals the
+ *    unbatched run's tally up to summation order. The batches belong to the first tally and
+ *    mesh a timestep of the bank deposits into; a timestep into another tally or mesh flushes
+ *    and starts over. With x_b = S_b * N / n_b (an independent estimate of the whole tally),
+ *    m = mean of x_b, s^2 = sum_b (x_b - m)^2 / (B - 1): R = sqrt(s^2 / B) / |m|, 0 where
+ *    m == 0, per cell and for the tally total.
+ *    Refused (error code, or a fatal error from inject_particles / solve_transport_2d): banks
+ *    sharded over several GPUs or in a multi-process group, banks that do not hold particles
+ *    [0, ntotal_particles) of the timestep, B > N, nb200_bank_append, pipeline = 0 and
+ *    tally_prereduce = 1, and B * nx * ny >= 2^31. The host flavour
+ *    nb200_solve_transport_2d_host has no batches.
+ * ---------------------------------------------------------------------------------- */
+/* Flushes, then writes the B cumulative partial tallies S_b as B consecutive arrays of ncells
+ * doubles (batch-major) to device memory. Returns B, or a negative code (nb200_last_error):
+ * not a batched bank, no timestep deposited yet, ncells not the batches' mesh. */
+int nb200_bank_tally_batches(nb200_particle_soa* particles, double* out_device, size_t ncells);
+/* Flushes, then writes R of every cell to relerr_device (ncells doubles, device memory) and R of
+ * the tally total to *total_relerr_host. Either may be null. Returns 0 or a negative code. */
+int nb200_bank_tally_relerr(nb200_particle_soa* particles, double* relerr_device,
+                            double* total_relerr_host);
+
 /* What the history kernel is bound by on facet-dominated decks, measured in place: FP64
  * reductions per second the L2 retires (csrc/microbench.cu; pattern 3 = the peak, 1 = a
  * particle's mesh walk, 0 = random cells, 5 / 6 = 32 / 4 lanes on consecutive cells) into a
@@ -370,6 +405,10 @@ void nb200_host_sincos(const double* x, long long n, double* sin_out, double* co
 unsigned nb200_selftest_dispatch_group(unsigned cta, unsigned n_live, unsigned n_coll,
                                        int stagger_at, int stagger_share, int stagger_min);
 long long nb200_selftest_host_sincos(const double* x, long long n, double* bad_x);
+/* The batch of global particle `pid` among `nbatches` batches of n particles (host evaluation
+ * of the history kernel's own map, nb_bank.cuh: batch_of); UINT_MAX outside 1 <= nbatches <= n,
+ * pid < n < 2^31. */
+unsigned nb200_selftest_batch_of(uint64_t pid, uint64_t n, int nbatches);
 
 #ifdef __cplusplus
 }

@@ -16,8 +16,8 @@ CSRC = os.path.join(HERE, "csrc")
 # NB200_LIB / NB200_DEFINES build and load an experiment variant next to the product library
 # (e.g. NB200_DEFINES=-DNB_HISTORY_MIN_BLOCKS=5 NB200_LIB=libneutral_b200.mb5.so).
 LIB = os.path.join(HERE, os.environ.get("NB200_LIB", "libneutral_b200.so"))
-SOURCES = ["transport.cu", "stage.cu", "pipeline.cu", "history.cu", "group.cu", "microbench.cu",
-           "capi.cu"]
+SOURCES = ["transport.cu", "stage.cu", "pipeline.cu", "history.cu", "group.cu",
+           "tally_batches.cu", "microbench.cu", "capi.cu"]
 HEADERS = ["transport.cuh", "nb_device.cuh", "nb_bank.cuh", "nb_math.cuh", "nb_history.cuh",
            "nb_sincos.cuh", "nb_fastmath.cuh", "nb_group.cuh", "nb_nccl_dyn.cuh", "engine.cuh", "glibc_log_table.inc", "glibc_sincos_table.inc",
            os.path.join("..", "..", "include", "neutral_b200.h")]

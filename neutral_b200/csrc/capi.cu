@@ -50,6 +50,7 @@ const OptionSpec kOptionSpecs[] = {
     {"stagger_at", &Options::stagger_at, 0, 95},
     {"stagger_share", &Options::stagger_share, 0, 100},
     {"stagger_min", &Options::stagger_min, 0, 1000},
+    {"tally_batches", &Options::tally_batches, 0, kMaxTallyBatches},  // 1 is refused too
 };
 const int kNumOptionSpecs = (int)(sizeof(kOptionSpecs) / sizeof(kOptionSpecs[0]));
 
@@ -77,6 +78,7 @@ std::vector<TallyGroup*> g_groups;     // every live group (tally-access hooks w
 uint64_t g_replica_generation = 1;     // bumped by nb200_update_replicas
 int g_shard_first = 0, g_shard_count = -1;  // nb200_set_shard
 std::unordered_set<const void*> g_handles;  // every live bank handle (what `Particle*` may be)
+std::vector<Bank*> g_batched;          // every live bank with tally batches
 
 // What `validate` reports besides the reference's printed lines (SURVEY.md 8f 1).
 struct StepLog {
@@ -168,6 +170,15 @@ void read_environment() {
   if (const char* s = getenv("NB200_COLLECTIVE")) g_opt.collective = strcmp(s, "nccl") == 0 ? 0 : 1;
   if (const char* s = getenv("NB200_HOST_MIRROR")) g_opt.host_mirror = atoi(s) != 0;
   if (const char* s = getenv("NB200_HEADROOM_PCT")) g_opt.headroom_pct = std::max(0, atoi(s));
+  // NB200_TALLY_BATCHES: batches of the drop-in binary's tally statistics (option tally_batches)
+  if (const char* s = getenv("NB200_TALLY_BATCHES")) {
+    const int b = atoi(s);
+    if (b == 0 || (b >= 2 && b <= kMaxTallyBatches))
+      g_opt.tally_batches = b;
+    else
+      fprintf(stderr, "neutral_b200: NB200_TALLY_BATCHES=%s ignored (0 or 2..%d)\n", s,
+              kMaxTallyBatches);
+  }
 }
 
 // The context of CUDA device `dev`, initialised on first use (`dev` must be current).
@@ -264,6 +275,11 @@ int opt_of(const Bank* bank, int Options::*slot) {
     for (const auto& o : bank->overrides)
       if (kOptionSpecs[o.first].slot == slot) return o.second;
   return g_opt.*slot;
+}
+
+// A value the option's range admits but the option does not: one batch has no spread.
+bool option_value_invalid(const OptionSpec& spec, int value) {
+  return spec.slot == &Options::tally_batches && value == 1;
 }
 
 // --------------------------------------------------------------------------- allocation --
@@ -421,6 +437,133 @@ Bank* bank_of(nb200_particle_soa* particles) {
 nb200_particle_soa* handle_of(Bank* bank) { return views_of(bank->header); }
 
 bool single_shard(const Bank* bank) { return bank->shards.size() == 1; }
+
+// ------------------------------------------------------------------------ tally batches --
+// Why a bank of n particles with global pids [pid0, pid0 + n) cannot have B tally batches under
+// the current defaults, or nullptr. The batches are ranges of the whole run's pids: the bank
+// must hold all of them, on one GPU, and be stepped by the batched history kernel.
+const char* why_no_batches(int B, int n, uint64_t pid0, int ngpus) {
+  static char why[256];
+  if (B <= 0) return nullptr;
+  if (ngpus > 1 || g_mp)
+    return "tally_batches: a bank sharded over several GPUs or in a multi-process group has no "
+           "batched tally";
+  if (pid0 != 0) {
+    snprintf(why, sizeof(why), "tally_batches: the bank starts at particle %llu; batches need "
+             "the whole run's particles from 0", (unsigned long long)pid0);
+    return why;
+  }
+  if (B > n) {
+    snprintf(why, sizeof(why), "tally_batches=%d exceeds the bank's %d particles", B, n);
+    return why;
+  }
+  if (!g_opt.pipeline) return "tally_batches: needs option pipeline=1 (the direct kernel has no batches)";
+  if (g_opt.tally_prereduce) return "tally_batches: cannot be combined with tally_prereduce=1";
+  return nullptr;
+}
+
+void batches_attach(Bank* bank, int B) {
+  if (B <= 0) return;
+  bank->batches.B = B;
+  g_batched.push_back(bank);
+}
+
+// Brings the caller's tally up to date: target += sum_b S_b - F, F = sum_b S_b. Synchronous.
+void batches_flush(Bank* bank) {
+  TallyBatches& tb = bank->batches;
+  if (!tb.dirty || !tb.target) return;
+  const Shard& sh = bank->shards[0];
+  DeviceGuard guard(sh.dev);
+  DeviceCtx& c = ctx_on(sh.dev);
+  c.launches += launch_batch_flush(tb.slab, tb.B, tb.ncells, tb.target, c.stream);
+  CU_FATAL(cudaGetLastError());
+  CU_FATAL(cudaStreamSynchronize(c.stream));
+  tb.dirty = false;
+}
+
+void batches_release(Bank* bank) {
+  TallyBatches& tb = bank->batches;
+  if (tb.B <= 0) return;
+  batches_flush(bank);
+  if (tb.slab) {
+    DeviceGuard guard(bank->shards[0].dev);
+    cudaFree(tb.slab);
+  }
+  tb = TallyBatches{};
+  g_batched.erase(std::remove(g_batched.begin(), g_batched.end(), bank), g_batched.end());
+}
+
+// Binds the batches to the tally and mesh of a timestep (before it is enqueued): another tally
+// or mesh flushes into the old target and starts over, as enqueue_step does for a group.
+// Terminates on a step the batches cannot serve.
+void batches_bind(Bank* bank, const StepRequest& rq) {
+  TallyBatches& tb = bank->batches;
+  const size_t ncells = (size_t)rq.nx * (size_t)rq.ny;
+  if (!single_shard(bank) || bank->pid0 != 0 || rq.ntotal != bank->n)
+    terminate("solve_transport_2d: a bank with tally_batches must hold the whole run on one GPU "
+              "(bank: %d particles from %llu on %zu GPU(s); ntotal_particles = %d)", bank->n,
+              (unsigned long long)bank->pid0, bank->shards.size(), rq.ntotal);
+  if (g_mp) terminate("solve_transport_2d: tally_batches in a multi-process group");
+  if (!opt_of(bank, &Options::pipeline) || opt_of(bank, &Options::tally_prereduce))
+    terminate("solve_transport_2d: tally_batches needs pipeline=1 and tally_prereduce=0");
+  if ((unsigned long long)ncells * (unsigned long long)tb.B >= (1ull << 31))
+    terminate("solve_transport_2d: tally_batches=%d over %zu cells needs 2^31 or more tally "
+              "slots (the history kernel indexes them with 32 bits)", tb.B, ncells);
+  if (tb.target == rq.tally && tb.ncells == ncells) return;
+  batches_flush(bank);
+  const Shard& sh = bank->shards[0];
+  DeviceGuard guard(sh.dev);
+  DeviceCtx& c = ctx_on(sh.dev);
+  const size_t bytes = sizeof(double) * (size_t)(tb.B + 1) * ncells;
+  if (tb.ncells != ncells || !tb.slab) {
+    if (tb.slab) {
+      CU_FATAL(cudaStreamSynchronize(c.stream));
+      cudaFree(tb.slab);
+    }
+    CU_FATAL(cudaMalloc(&tb.slab, bytes));
+    tb.ncells = ncells;
+  }
+  CU_FATAL(cudaMemsetAsync(tb.slab, 0, bytes, c.stream));
+  tb.target = rq.tally;
+}
+
+// R of the tally total: the B batch totals through a fixed-order device reduction, then the
+// estimator in FP64 on the host.
+double batches_total_relerr(Bank* bank) {
+  TallyBatches& tb = bank->batches;
+  const Shard& sh = bank->shards[0];
+  DeviceGuard guard(sh.dev);
+  DeviceCtx& c = ctx_on(sh.dev);
+  const size_t np = (size_t)tb.B * kBatchSumBlocks;
+  double* d_partial = nullptr;
+  CU_FATAL(cudaMalloc(&d_partial, sizeof(double) * np));
+  c.launches += launch_batch_sums(tb.slab, tb.B, tb.ncells, d_partial, c.stream);
+  std::vector<double> h(np);
+  CU_FATAL(cudaMemcpyAsync(h.data(), d_partial, sizeof(double) * np, cudaMemcpyDeviceToHost,
+                           c.stream));
+  CU_FATAL(cudaStreamSynchronize(c.stream));
+  cudaFree(d_partial);
+  std::vector<double> x(tb.B);
+  double sum = 0.0;
+  for (int b = 0; b < tb.B; ++b) {
+    double t = 0.0;
+    for (int k = 0; k < kBatchSumBlocks; ++k) t += h[(size_t)b * kBatchSumBlocks + k];
+    const int nb = bank->n / tb.B + (b < bank->n % tb.B ? 1 : 0);
+    x[b] = t * (double)bank->n / (double)nb;
+    sum += x[b];
+  }
+  const double m = sum / (double)tb.B;
+  double ss = 0.0;
+  for (int b = 0; b < tb.B; ++b) ss += (x[b] - m) * (x[b] - m);
+  const double var = ss / (double)(tb.B - 1);
+  return m == 0.0 ? 0.0 : sqrt(var / (double)tb.B) / fabs(m);
+}
+
+Bank* batched_bank_of_tally(const double* tally) {
+  for (Bank* b : g_batched)
+    if (b->batches.target == tally && b->batches.slab) return b;
+  return nullptr;
+}
 
 // Uploads host SoA slices into the shards of `bank` (origins from 0 within each shard).
 void upload_host_soa(Bank* bank, const SoaView& host) {
@@ -674,6 +817,7 @@ struct ShardIO {
   const double *density, *edgex, *edgey, *s_keys, *s_vals, *a_keys, *a_vals;
   double* tally;
   uint64_t *r0, *r1, *r2;
+  BatchArgs batches;
 };
 
 // An event the host will wait on or read a time from. While a timestep is being recorded into
@@ -800,7 +944,7 @@ void record_shard_step(DeviceCtx& c, const Bank* bank, Shard& sh, const StepRequ
     a.stagger_share = opt_of(bank, &Options::stagger_share);
     a.stagger_min = opt_of(bank, &Options::stagger_min);
     const bool fast_div = opt_of(bank, &Options::fast_div) != 0;
-    c.launches += launch_history(a, c.d_n_live, s.n_upper, fast_div,
+    c.launches += launch_history(a, io.batches, c.d_n_live, s.n_upper, fast_div,
                                  opt_of(bank, &Options::tally_prereduce) != 0,
                                  opt_l2 == 2 ? (const void*)io.tally
                                  : opt_l2    ? (const void*)c.d_cs_stage : nullptr,
@@ -1161,6 +1305,14 @@ void group_flush(TallyGroup& g) {
 // Any library-mediated look at memory that a group's unflushed contributions belong to
 // flushes first (validate, copy_buffer, the nb200_memcpy / memset helpers).
 void flush_groups_touching(const void* ptr, size_t bytes) {
+  for (Bank* b : g_batched) {
+    const TallyBatches& tb = b->batches;
+    if (!tb.dirty || !tb.target) continue;
+    const char* lo = (const char*)tb.target;
+    const char* hi = lo + tb.ncells * 8;
+    const char* p = (const char*)ptr;
+    if (p < hi && p + bytes > lo) batches_flush(b);
+  }
   for (TallyGroup* g : g_groups) {
     if (!g->dirty || !g->target) continue;
     const char* lo = (const char*)g->target;
@@ -1243,6 +1395,7 @@ void enqueue_step(Bank* bank, const StepRequest& rq) {
     closes = group->reduce_every > 0 && group->steps_deposited + 1 >= group->reduce_every;
     epoch = group->epoch + 1;
   }
+  if (bank->batches.B > 0) batches_bind(bank, rq);
   PendingStep ps;
   ps.pipeline = opt_of(bank, &Options::pipeline) != 0;
   ps.print = opt_of(bank, &Options::print) != 0;
@@ -1266,6 +1419,7 @@ void enqueue_step(Bank* bank, const StepRequest& rq) {
     io.a_keys = replica_of(c, sh, pd, rq.a_keys, (size_t)rq.a_n);
     io.a_vals = replica_of(c, sh, pd, rq.a_vals, (size_t)rq.a_n);
     io.tally = rq.tally;
+    io.batches = BatchArgs{bank->batches.slab, bank->batches.B, bank->n};
     // per-particle counters live on the primary GPU, indexed in injection order: a secondary
     // shard reaches its part of them through peer access (one 8-byte update per particle-step)
     const bool counters_ok = sh.dev == pd || (group && group->collective);
@@ -1286,6 +1440,7 @@ void enqueue_step(Bank* bank, const StepRequest& rq) {
       enqueue_shard_step(c, bank, sh, rq, io, slot, nullptr, 0);
     }
   }
+  if (bank->batches.B > 0) bank->batches.dirty = true;
   if (group) {
     group->steps_deposited++;
     group->dirty = true;
@@ -1416,8 +1571,11 @@ double device_sum(DeviceCtx& c, const double* v, size_t n) {
 
 // The machine-readable side of `validate` (SURVEY.md 8f 1): written when NB200_RESULTS_JSON
 // names a file. Same verdict as the printed lines, plus what the library saw of the run.
+// `batches` > 0: the tally came from a bank with tally batches, whose total has relative error
+// `total_relerr`.
 void write_results_json(const char* path, const char* deck, int nx, int ny, double total,
-                        bool have_expected, double expected, const char* verdict) {
+                        bool have_expected, double expected, const char* verdict, int batches,
+                        double total_relerr) {
   FILE* fp = fopen(path, "w");
   if (!fp) {
     fprintf(stderr, "neutral_b200: cannot write %s\n", path);
@@ -1430,6 +1588,9 @@ void write_results_json(const char* path, const char* deck, int nx, int ny, doub
   fprintf(fp, "{\"deck\": \"%s\", \"nx\": %d, \"ny\": %d, \"device\": \"%s\",\n", deck, nx, ny,
           prop.name);
   fprintf(fp, " \"tally_total\": %.17e, ", total);
+  if (batches > 0)
+    fprintf(fp, "\"tally_batches\": %d, \"tally_total_relative_error\": %.17e, ", batches,
+            total_relerr);
   if (have_expected)
     fprintf(fp, "\"expected\": %.17e, \"relative_error\": %.6e, \"tolerance\": 1e-3, ", expected,
             fabs(expected - total) / (fabs(expected) > 0.0 ? fabs(expected) : 1.0));
@@ -1518,9 +1679,12 @@ extern "C" size_t inject_particles(
     terminate("inject_particles: shard [%d, %d) outside [0, %d)", first, first + count,
               nparticles);
 
+  if (const char* why = why_no_batches(g_opt.tally_batches, count, (uint64_t)first, g_opt.ngpus))
+    terminate("inject_particles: %s", why);
   size_t bytes = 0;
   Bank* bank = new_bank(count, (uint64_t)first, g_opt.ngpus, g_opt.headroom_pct,
                         g_opt.host_mirror != 0, &bytes);
+  batches_attach(bank, g_opt.tally_batches);
   for (Shard& sh : bank->shards) {  // per-mesh scratch of every GPU involved, ahead of timestep 1
     DeviceGuard guard(sh.dev);
     int shift = g_opt.tile_shift, tx = 1, nt = 1;
@@ -1619,13 +1783,22 @@ extern "C" void validate(const int nx, const int ny, const char* params_filename
   flush_groups_touching(energy_tally, sizeof(double) * (size_t)nx * ny);
   const double total = device_sum(c, energy_tally, (size_t)nx * ny);
   if (rank != 0) return;
+  const char* json = getenv("NB200_RESULTS_JSON");
+  int batches = 0;
+  double total_relerr = 0.0;
+  if (json && *json) {
+    if (Bank* b = batched_bank_of_tally(energy_tally)) {
+      batches = b->batches.B;
+      total_relerr = batches_total_relerr(b);
+    }
+  }
   printf("\nFinal global_energy_tally %.15e\n", total);
   double expected = 0.0;
-  const char* json = getenv("NB200_RESULTS_JSON");
   if (!find_expected("problems/neutral.tests", params_filename, &expected)) {
     printf("Warning. Test entry was not found, could NOT validate.\n");
     if (json && *json)
-      write_results_json(json, params_filename, nx, ny, total, false, 0.0, "NOT_VALIDATED");
+      write_results_json(json, params_filename, nx, ny, total, false, 0.0, "NOT_VALIDATED",
+                         batches, total_relerr);
     return;
   }
   printf("Expected %.12e, result was %.12e.\n", expected, total);
@@ -1636,7 +1809,7 @@ extern "C" void validate(const int nx, const int ny, const char* params_filename
   printf(pass ? "PASSED validation.\n" : "FAILED validation.\n");
   if (json && *json)
     write_results_json(json, params_filename, nx, ny, total, true, expected,
-                       pass ? "PASSED" : "FAILED");
+                       pass ? "PASSED" : "FAILED", batches, total_relerr);
 }
 
 // ======================================================================================
@@ -1668,6 +1841,8 @@ extern "C" void deallocate_data(double* buf) {
     flush_groups_touching(buf, sizeof(double));
     for (TallyGroup* g : g_groups)
       if (g->target == buf) g->target = nullptr;
+    for (Bank* b : g_batched)
+      if (b->batches.target == buf) b->batches.target = nullptr;
   }
   cudaFree(buf);
 }
@@ -1856,8 +2031,14 @@ extern "C" int nb200_bank_create(const nb200_particle_soa* host, int count, int 
     set_error("nb200_bank_create: bad arguments");
     return -3;
   }
+  if (const char* why = why_no_batches(g_opt.tally_batches, count, (uint64_t)pid_first,
+                                     g_opt.ngpus)) {
+    set_error("nb200_bank_create: %s", why);
+    return -3;
+  }
   Bank* bank = new_bank(count, (uint64_t)pid_first, g_opt.ngpus, g_opt.headroom_pct,
                         g_opt.host_mirror != 0, nullptr);
+  batches_attach(bank, g_opt.tally_batches);
   if (count > 0) upload_host_soa(bank, as_soa_view(*host));
   refresh_mirror(bank);
   *particles = handle_of(bank);
@@ -2055,6 +2236,11 @@ extern "C" int nb200_bank_append(nb200_particle_soa* particles, const nb200_part
     set_error("nb200_bank_append: banks with a host mirror cannot grow");
     return -3;
   }
+  if (bank->batches.B > 0) {
+    set_error("nb200_bank_append: a bank with tally_batches cannot grow (its batches are ranges "
+              "of the particles it was created with)");
+    return -3;
+  }
   if (sh.n + count > sh.capacity) {
     set_error("nb200_bank_append: %d particles do not fit the head-room (%d of %d slots used; "
               "option headroom_pct)", count, sh.n, sh.capacity);
@@ -2095,6 +2281,7 @@ extern "C" int nb200_bank_free(nb200_particle_soa* particles) {
   Bank* bank = bank_of(particles);
   if (!bank) return -3;
   finish_all(bank);
+  batches_release(bank);
   if (bank->group) {
     group_flush(*bank->group);
     group_free(bank->group);
@@ -2180,8 +2367,9 @@ extern "C" int nb200_set_option(const char* name, int value) {
     return NB200_BAD_OPTION;
   }
   const OptionSpec& spec = kOptionSpecs[i];
-  if (value < spec.lo || value > spec.hi) {
-    set_error("nb200_set_option: %s=%d is outside [%d, %d]", name, value, spec.lo, spec.hi);
+  if (value < spec.lo || value > spec.hi || option_value_invalid(spec, value)) {
+    set_error("nb200_set_option: %s=%d is outside [%d, %d]%s", name, value, spec.lo, spec.hi,
+              option_value_invalid(spec, value) ? " (1: one batch has no spread)" : "");
     return NB200_BAD_OPTION;
   }
   const int prev = g_opt.*(spec.slot);
@@ -2209,6 +2397,17 @@ extern "C" int nb200_bank_set_option(nb200_particle_soa* particles, const char* 
   const OptionSpec& spec = kOptionSpecs[i];
   if (value < spec.lo || value > spec.hi) {
     set_error("nb200_bank_set_option: %s=%d is outside [%d, %d]", name, value, spec.lo, spec.hi);
+    return NB200_BAD_OPTION;
+  }
+  if (spec.slot == &Options::tally_batches) {
+    set_error("nb200_bank_set_option: tally_batches is fixed when the bank is created "
+              "(nb200_set_option before inject_particles / nb200_bank_create)");
+    return NB200_BAD_OPTION;
+  }
+  if (bank->batches.B > 0 && ((spec.slot == &Options::pipeline && value == 0) ||
+                              (spec.slot == &Options::tally_prereduce && value != 0))) {
+    set_error("nb200_bank_set_option: %s=%d on a bank with tally_batches (only the pipelined "
+              "kernel without tally_prereduce has batches)", name, value);
     return NB200_BAD_OPTION;
   }
   const int prev = opt_of(bank, spec.slot);
@@ -2262,9 +2461,72 @@ extern "C" uint64_t nb200_kernel_launches(void) {
 extern "C" int nb200_tally_sync(double* tally_device) {
   CTX_OR_RETURN(c);
   (void)c;
+  for (Bank* b : g_batched)
+    if (!tally_device || b->batches.target == tally_device) batches_flush(b);
   for (TallyGroup* g : g_groups)
     if (!tally_device || g->target == tally_device) group_flush(*g);
   return 0;
+}
+
+// ------------------------------------------------------------------------ tally batches --
+// The bank's batched state, flushed into the caller's tally; nullptr (error set) if there is none.
+static Bank* flushed_batches(nb200_particle_soa* particles, const char* who) {
+  Bank* bank = bank_of(particles);
+  if (!bank || bank->batches.B <= 0) {
+    set_error("%s: not a bank handle created with tally_batches", who);
+    return nullptr;
+  }
+  if (!bank->batches.slab) {
+    set_error("%s: no timestep of this bank has deposited into its batches yet", who);
+    return nullptr;
+  }
+  batches_flush(bank);
+  return bank;
+}
+
+extern "C" int nb200_bank_tally_batches(nb200_particle_soa* particles, double* out_device,
+                                        size_t ncells) {
+  CTX_OR_RETURN(c0);
+  (void)c0;
+  Bank* bank = flushed_batches(particles, "nb200_bank_tally_batches");
+  if (!bank) return -3;
+  const TallyBatches& tb = bank->batches;
+  if (!out_device || ncells != tb.ncells) {
+    set_error("nb200_bank_tally_batches: the batches cover %zu cells, %zu were asked for",
+              tb.ncells, ncells);
+    return -3;
+  }
+  DeviceGuard guard(bank->shards[0].dev);
+  DeviceCtx& c = ctx_on(bank->shards[0].dev);
+  c.launches += launch_batch_export(tb.slab, tb.B, tb.ncells, out_device, c.stream);
+  CU_TRY(cudaGetLastError());
+  CU_TRY(cudaStreamSynchronize(c.stream));
+  return tb.B;
+}
+
+extern "C" int nb200_bank_tally_relerr(nb200_particle_soa* particles, double* relerr_device,
+                                       double* total_relerr_host) {
+  CTX_OR_RETURN(c0);
+  (void)c0;
+  Bank* bank = flushed_batches(particles, "nb200_bank_tally_relerr");
+  if (!bank) return -3;
+  const TallyBatches& tb = bank->batches;
+  DeviceGuard guard(bank->shards[0].dev);
+  DeviceCtx& c = ctx_on(bank->shards[0].dev);
+  if (relerr_device) {
+    c.launches += launch_batch_relerr(tb.slab, tb.B, tb.ncells, bank->n, relerr_device, c.stream);
+    CU_TRY(cudaGetLastError());
+    CU_TRY(cudaStreamSynchronize(c.stream));
+  }
+  if (total_relerr_host) *total_relerr_host = batches_total_relerr(bank);
+  return 0;
+}
+
+// Host-side evaluation of the history kernel's pid -> batch map (pure integer arithmetic), for
+// the tests: it has to reproduce shard_split's ranges for any n and B.
+extern "C" unsigned nb200_selftest_batch_of(uint64_t pid, uint64_t n, int nbatches) {
+  if (nbatches < 1 || n > 0x7fffffffull || (uint64_t)nbatches > n || pid >= n) return UINT_MAX;
+  return batch_of((unsigned)pid, (unsigned)n, (unsigned)nbatches);
 }
 
 extern "C" int nb200_update_replicas(void) {

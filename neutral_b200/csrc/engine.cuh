@@ -54,7 +54,9 @@ struct Options {
   int stagger_share = 50;  // percent of the collider CTAs that are delayed
   int stagger_min = 35;    // colliders' share of the live bank (per mille) from which on it is done
   int step_graph = 1;    // submit a timestep as one CUDA graph launch instead of ~23 driver calls
+  int tally_batches = 0; // batches of the next bank's tally statistics (0: none, else 2..64)
 };
+constexpr int kMaxTallyBatches = 64;
 
 struct OptionSpec {
   const char* name;
@@ -206,8 +208,20 @@ struct HostMirror {  // pinned host copy of the bank in injection order (visit_d
   bool present = false;
 };
 
+// Option tally_batches of a single-GPU bank (tally_batches.cu): the history kernel deposits into
+// B partial tallies; the caller's tally is brought up to date lazily, where a sharded run's
+// would be (flush_groups_touching), by adding what the batches gained since the last flush.
+struct TallyBatches {
+  int B = 0;                 // 0: the bank deposits straight into the caller's tally
+  double* slab = nullptr;    // B partial tallies (batch_slot layout), then F = their sum at the last flush
+  size_t ncells = 0;
+  double* target = nullptr;  // the caller-visible tally the batches belong to
+  bool dirty = false;        // the batches hold deposits the target has not received
+};
+
 struct Bank {
   std::vector<Shard> shards;
+  TallyBatches batches;
   int n = 0;
   uint64_t pid0 = 0;
   int primary_dev = 0;

@@ -30,6 +30,11 @@
 //
 // Compiled with -fmad=false: the only fused operations are the explicit fma() of nb_log,
 // div_by_known and the cores.
+#include <type_traits>
+#ifdef NB_ASSERT_BATCH_SLOT
+#include <cassert>
+#endif
+
 #include "nb_history.cuh"
 
 namespace nb {
@@ -119,17 +124,43 @@ extern "C" unsigned nb200_selftest_dispatch_group(unsigned cta, unsigned n_live,
   return dispatch_group(a, cta, n_live, n_coll);
 }
 
-template <bool kFastDiv, bool kPreReduce>
+// kBatched (option tally_batches): every deposit goes to the partial tally of the particle's
+// batch (StepArgs::batch_slab). The batch follows from the global pid, once per history; it
+// is parked beside `origin` and turned into an address at each deposit.
+struct ParkedBatched : Parked {
+  int batch[kHistoryThreads];
+};
+
+template <bool kBatched, class P>
+__device__ __forceinline__ int parked_batch(const P& park) {
+  if constexpr (kBatched) return park.batch[threadIdx.x];
+  else return 0;
+}
+
+// Index of `cell` of batch b in the slab (32 bits: the host refuses B * ncells >= 2^31).
+__device__ __forceinline__ int batch_index(const StepArgs& a, const BatchArgs& bt, int b,
+                                           int cell) {
+  const int i = (int)batch_slot(b, (size_t)(unsigned)cell, bt.nbatches, (size_t)(a.nx * a.ny));
+#ifdef NB_ASSERT_BATCH_SLOT  // checking build: NB200_DEFINES=-DNB_ASSERT_BATCH_SLOT
+  assert(b >= 0 && b < bt.nbatches && cell >= 0 && cell < a.nx * a.ny && i >= 0 &&
+         i < bt.nbatches * a.nx * a.ny);
+#endif
+  return i;
+}
+
+template <bool kFastDiv, bool kPreReduce, bool kBatched>
 __global__ void NB_HISTORY_BOUNDS
-k_history(const StepArgs a, const unsigned* __restrict__ n_live) {
+k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs bt) {
 #if NB_PARK_SMEM
-  __shared__ Parked park;
+  __shared__ std::conditional_t<kBatched, ParkedBatched, Parked> park;
 #define PARKED(name) park.name[threadIdx.x]
+#define PARKED_BATCH parked_batch<kBatched>(park)
 #else
   double park_e, park_Sig_s, park_p_absorb, park_rho, park_edep;
-  int park_origin, park_slot;
+  int park_origin, park_slot, park_batch = 0;
   unsigned park_nc;
 #define PARKED(name) park_##name
+#define PARKED_BATCH park_batch
 #endif
   const unsigned live = n_live[0];
   unsigned nf = 0, census = 0, processed = 0, died = 0;
@@ -156,10 +187,22 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live) {
     double dtc = tm.x, mfp = tm.y;
     int cx = m.x, cy = m.y;
 #define NB_CELL (cy * a.nx + cx)  // tally / density index of the current cell
+    // the base and index a deposit into `cell` goes to: the caller's tally, or the batch's slot
+#define NB_TALLY_AT(cell) \
+  (kBatched ? bt.slab : a.tally), (kBatched ? batch_index(a, bt, PARKED_BATCH, (cell)) : (cell))
     unsigned flags = same_grid(a) ? kFlagSameGrid : 0u;
     PARKED(e) = ew.x;
     PARKED(edep) = 0.0;
     PARKED(origin) = m.w;
+    if constexpr (kBatched) {
+      const int b = (int)batch_of((unsigned)(a.pid0 + (uint64_t)(unsigned)m.w), (unsigned)bt.n,
+                                  (unsigned)bt.nbatches);
+#if NB_PARK_SMEM
+      park.batch[threadIdx.x] = b;
+#else
+      park_batch = b;
+#endif
+    }
     // RNG counter: k_begin_step drew counter 0 (omp3/neutral.c:129); collision number k of
     // this step draws counters 2k-1 and 2k (:235, :294), so the collision count nc is the
     // counter state.
@@ -232,7 +275,7 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live) {
             // them with this facet's own; here they go to the same cell as a reduction of
             // their own (the tally's tolerance covers the different rounding of the sum), which
             // keeps the parked slot out of the per-facet code
-            tally_add<kPreReduce>(a.tally, NB_CELL, PARKED(edep) * a.inv_ntotal);
+            tally_add<kPreReduce>(NB_TALLY_AT(NB_CELL), PARKED(edep) * a.inv_ntotal);
             PARKED(edep) = 0.0;
             flags &= ~kFlagPending;
           }
@@ -260,7 +303,7 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live) {
         dtc -= q_dtc;
         // :321-327 - deposit, flush to the tally (update_tallies, :408-420), reset
         const double edep = deposition(w, d_facet, d.stb, d.heat, nd);
-        tally_add<kPreReduce>(a.tally, NB_CELL, edep * a.inv_ntotal);
+        tally_add<kPreReduce>(NB_TALLY_AT(NB_CELL), edep * a.inv_ntotal);
         x += d_facet * ox;
         y += d_facet * oy;
         // the edge load is consumed here, after the arithmetic it overlapped with
@@ -342,7 +385,7 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live) {
           w *= (1.0 - p_absorb);
           if (e < kMinEnergyOfInterest) {  // :243-252 - the history ends here
             flags |= kFlagDead;
-            tally_add<kPreReduce>(a.tally, NB_CELL, edep * a.inv_ntotal);
+            tally_add<kPreReduce>(NB_TALLY_AT(NB_CELL), edep * a.inv_ntotal);
             break;
           }
           // Energy and direction are unchanged: the lookups of :285-291 return the values
@@ -405,7 +448,7 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live) {
         mfp -= d_census / d.cell_mfp;
         double edep = deposition(w, d_census, d.stb, d.heat, nd);
         if (flags & kFlagPending) edep = PARKED(edep) + edep;
-        tally_add<kPreReduce>(a.tally, NB_CELL, edep * a.inv_ntotal);
+        tally_add<kPreReduce>(NB_TALLY_AT(NB_CELL), edep * a.inv_ntotal);
         dtc = 0.0;
         break;
       }
@@ -437,6 +480,8 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live) {
   flush_totals(a.totals, nf, PARKED(nc), processed, census, died);
 #undef PARKED
 #undef NB_CELL
+#undef NB_TALLY_AT
+#undef PARKED_BATCH
 }
 
 static inline int blocks_for(int n, int threads) { return (n + threads - 1) / threads; }
@@ -444,8 +489,8 @@ static inline int blocks_for(int n, int threads) { return (n + threads - 1) / th
 // `pin`/`pin_bytes` (optional) name the staged cross-section block: the launch then carries an
 // access-policy window that keeps it persisting in L2 (north_star phase 3), while the rest of
 // the kernel's traffic - the tally atomics above all - streams through the remainder.
-int launch_history(const StepArgs& a, const unsigned* n_live, int n_upper, bool fast_div,
-                   bool prereduce, const void* pin, size_t pin_bytes, size_t pin_budget,
+int launch_history(const StepArgs& a, const BatchArgs& bt, const unsigned* n_live, int n_upper,
+                   bool fast_div, bool prereduce, const void* pin, size_t pin_bytes, size_t pin_budget,
                    int smem_pad, cudaStream_t st) {
   if (n_upper <= 0) return 0;
   cudaLaunchConfig_t cfg = {};
@@ -457,9 +502,11 @@ int launch_history(const StepArgs& a, const unsigned* n_live, int n_upper, bool 
     // the number of resident CTAs per SM without touching the code.
     static int granted = 0;
     if (smem_pad > granted) {
-      cudaFuncSetAttribute(k_history<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
-      cudaFuncSetAttribute(k_history<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
-      cudaFuncSetAttribute(k_history<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
+      cudaFuncSetAttribute(k_history<true, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
+      cudaFuncSetAttribute(k_history<true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
+      cudaFuncSetAttribute(k_history<false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
+      cudaFuncSetAttribute(k_history<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
+      cudaFuncSetAttribute(k_history<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
       granted = smem_pad;
     }
     cfg.dynamicSmemBytes = (size_t)smem_pad;
@@ -477,12 +524,22 @@ int launch_history(const StepArgs& a, const unsigned* n_live, int n_upper, bool 
     cfg.attrs = attr;
     cfg.numAttrs = 1;
   }
-  if (prereduce)
-    cudaLaunchKernelEx(&cfg, k_history<true, true>, a, n_live);
-  else if (fast_div)
-    cudaLaunchKernelEx(&cfg, k_history<true, false>, a, n_live);
-  else
-    cudaLaunchKernelEx(&cfg, k_history<false, false>, a, n_live);
+  // A batched bank always runs a batched variant (the host refuses prereduce for it), so the
+  // step graph of a device updates in place from one of its timesteps to the next. Banks with
+  // and without batches alternating on one device change the graph's kernel and re-instantiate
+  // it instead, which is correct and costs an instantiation per switch.
+  if (bt.nbatches > 0) {
+    if (fast_div)
+      cudaLaunchKernelEx(&cfg, k_history<true, false, true>, a, n_live, bt);
+    else
+      cudaLaunchKernelEx(&cfg, k_history<false, false, true>, a, n_live, bt);
+  } else if (prereduce) {
+    cudaLaunchKernelEx(&cfg, k_history<true, true, false>, a, n_live, bt);
+  } else if (fast_div) {
+    cudaLaunchKernelEx(&cfg, k_history<true, false, false>, a, n_live, bt);
+  } else {
+    cudaLaunchKernelEx(&cfg, k_history<false, false, false>, a, n_live, bt);
+  }
   return 1;
 }
 

@@ -134,6 +134,36 @@ struct StepArgs {
   int stagger_at, stagger_share, stagger_min;
 };
 
+// Option tally_batches (tally_batches.cu): with nbatches = B > 0 every deposit of the history
+// kernel goes to the partial tally of the depositing particle's batch instead of
+// StepArgs::tally; batch b is the contiguous pid range shard_split(n, b, B). A kernel
+// parameter of its own behind the existing two: grown, StepArgs would move the offset of the
+// parameter that follows it in every instantiation of k_history, batched or not.
+struct BatchArgs {
+  double* slab;
+  int nbatches;
+  int n;
+};
+
+// Layout of the B partial tallies in the batch slab: batch-major [b][cell] (0) or cell-major
+// [cell][b] (1). Both were built and measured (DESIGN.md 9); the product keeps batch-major.
+// -DNB_TALLY_BATCH_CELL_MAJOR=1 builds the other one for tools/tally_batches_cost.py.
+#ifndef NB_TALLY_BATCH_CELL_MAJOR
+#define NB_TALLY_BATCH_CELL_MAJOR 0
+#endif
+__host__ __device__ __forceinline__ size_t batch_slot(int b, size_t cell, int B, size_t ncells) {
+  return NB_TALLY_BATCH_CELL_MAJOR ? cell * (size_t)B + (size_t)b : (size_t)b * ncells + cell;
+}
+
+// Batch of global pid `pid` among the B contiguous ranges of shard_split(n, b, B) (capi.cu):
+// batch b starts at b * (n / B) + min(b, n % B). The first n % B batches hold n / B + 1
+// particles, the rest n / B. Requires 1 <= B <= n and pid < n.
+__host__ __device__ __forceinline__ unsigned batch_of(unsigned pid, unsigned n, unsigned B) {
+  const unsigned per = n / B, rem = n % B;
+  const unsigned split = rem * (per + 1u);  // particles in the larger batches
+  return pid < split ? pid / (per + 1u) : rem + (pid - split) / per;
+}
+
 // Scratch of the per-step counting sort (pipeline.cu).
 struct SortArgs {
   unsigned* keys;        // [n] sort key of every slot in [0, n_upper)

@@ -19,9 +19,22 @@ int launch_history_direct(const StepArgs& a, cudaStream_t st);
 // `alt`; history = event loop over the sorted live prefix.
 int launch_sort_phase(const StepArgs& a, const SortArgs& s, const BankView& alt,
                       cudaStream_t st);
-int launch_history(const StepArgs& a, const unsigned* n_live, int n_upper, bool fast_div,
-                   bool prereduce, const void* pin, size_t pin_bytes, size_t pin_budget,
-                   int smem_pad, cudaStream_t st);
+// bt.nbatches > 0 runs the batched variant (option tally_batches).
+int launch_history(const StepArgs& a, const BatchArgs& bt, const unsigned* n_live, int n_upper,
+                   bool fast_div, bool prereduce, const void* pin, size_t pin_bytes,
+                   size_t pin_budget, int smem_pad, cudaStream_t st);
+// Batch partial tallies (tally_batches.cu). The slab holds the B partial tallies S_b in the
+// layout of batch_slot() and behind them one more array F of ncells: sum_b S_b as of the last
+// flush. Flush: tally += sum_b S_b - F, F = sum_b S_b (summed in batch order).
+int launch_batch_flush(double* slab, int B, size_t ncells, double* tally, cudaStream_t st);
+// out = the B partial tallies batch-major ([b][cell]), whatever the slab's layout.
+int launch_batch_export(const double* slab, int B, size_t ncells, double* out, cudaStream_t st);
+// relerr[cell] = relative error of the batch mean (n: particles, split into B batches).
+int launch_batch_relerr(const double* slab, int B, size_t ncells, int n, double* relerr,
+                        cudaStream_t st);
+// partial[b * blocks + k] = sum over block k's cells of S_b (blocks = kBatchSumBlocks).
+constexpr int kBatchSumBlocks = 148;
+int launch_batch_sums(const double* slab, int B, size_t ncells, double* partial, cudaStream_t st);
 // Per-step staging of the read-only inputs (stage.cu).
 int launch_stage_cs(const double* keys, const double* vals, int n, double2* kv, int* bucket,
                     unsigned long long bits0, int shift, int nb, const double* twin_keys,

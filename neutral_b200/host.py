@@ -55,7 +55,8 @@ EXPORTED_SYMBOLS = [
     "nb200_bank_capacity", "nb200_bank_gpus", "nb200_bank_append", "nb200_get_option",
     "nb200_bank_set_option", "nb200_bank_solve_finish", "nb200_bank_pending", "nb200_mp_init",
     "nb200_mp_connect", "nb200_mp_finalize", "nb200_tally_sync", "nb200_update_replicas",
-    "nb200_microbench_red",
+    "nb200_microbench_red", "nb200_bank_tally_batches", "nb200_bank_tally_relerr",
+    "nb200_selftest_batch_of",
 ]
 
 #: include/neutral_b200.h
@@ -131,6 +132,10 @@ def load_library(build: bool = False) -> C.CDLL:
     L.nb200_mp_connect.argtypes = [C.c_void_p]
     L.nb200_tally_sync.argtypes = [C.c_void_p]
     L.nb200_microbench_red.argtypes = [C.c_int, C.c_size_t, C.c_int, _dp]
+    L.nb200_bank_tally_batches.argtypes = [_soa_p, C.c_void_p, C.c_size_t]
+    L.nb200_bank_tally_relerr.argtypes = [_soa_p, C.c_void_p, _dp]
+    L.nb200_selftest_batch_of.argtypes = [C.c_uint64, C.c_uint64, C.c_int]
+    L.nb200_selftest_batch_of.restype = C.c_uint
     L.nb200_last_step_stats.argtypes = [_u64p]
     L.nb200_solve_finish.argtypes = [_u64p, _u64p]
     L.nb200_kernel_launches.restype = C.c_uint64
@@ -236,7 +241,8 @@ class Simulation:
     """
 
     def __init__(self, problem: Problem, rank: int = 0, nranks: int = 1,
-                 per_particle_counters: bool = True, quiet: bool = True, ngpus: int = 1):
+                 per_particle_counters: bool = True, quiet: bool = True, ngpus: int = 1,
+                 tally_batches: int = 0):
         self.lib = load_library()
         require_device()
         self.problem = problem
@@ -246,6 +252,9 @@ class Simulation:
         #: GPUs of THIS process the bank is sharded over (option "ngpus"): the library drives
         #: them all behind the same solve_transport_2d call and combines the tally itself
         self.ngpus = ngpus
+        #: batches of the tally statistics (option "tally_batches", 0: none): the bank's
+        #: deposits are kept per contiguous particle range, see :meth:`tally_relative_error`
+        self.tally_batches = tally_batches
         if quiet:
             self.lib.nb200_set_option(b"print", 0)
         self.density = DeviceArray.from_host(problem.density.ravel())
@@ -272,12 +281,12 @@ class Simulation:
         if self.bank is not None:
             self.lib.nb200_bank_free(self.bank)
         self.lib.nb200_set_shard(self.pid0, self.count if self.nranks > 1 else -1)
-        prev = self.lib.nb200_set_option(b"ngpus", self.ngpus)
+        prev = self._set_creation_options()
         out = _soa_p()
         self.bank_bytes = self.lib.inject_particles(
             d.nparticles, d.nx, d.nx, d.ny, 0, s.left, s.bottom, s.width, s.height, 0, 0,
             d.dt, self.edgex.ptr, self.edgey.ptr, d.initial_energy, C.byref(out))
-        self.lib.nb200_set_option(b"ngpus", prev)
+        self._restore_options(prev)
         self.lib.nb200_set_shard(0, -1)
         self.bank = out
         return self.bank_bytes
@@ -289,11 +298,27 @@ class Simulation:
             self.lib.nb200_bank_free(self.bank)
         st = host.as_struct()
         out = _soa_p()
-        prev = self.lib.nb200_set_option(b"ngpus", self.ngpus)
-        _check(self.lib.nb200_bank_create(C.byref(st), self.count, self.pid0, C.byref(out)),
-               "bank_create")
-        self.lib.nb200_set_option(b"ngpus", prev)
+        prev = self._set_creation_options()
+        try:
+            _check(self.lib.nb200_bank_create(C.byref(st), self.count, self.pid0, C.byref(out)),
+                   "bank_create")
+        finally:
+            self._restore_options(prev)
         self.bank = out
+
+    def _set_creation_options(self) -> dict:
+        prev = {}
+        for name, value in ((b"ngpus", self.ngpus), (b"tally_batches", self.tally_batches)):
+            prev[name] = self.lib.nb200_set_option(name, value)
+            if prev[name] == NB200_BAD_OPTION:
+                raise NeutralB200Error(f"option {name.decode()}={value}: "
+                                       f"{self.lib.nb200_last_error().decode()}")
+        return prev
+
+    def _restore_options(self, prev: dict) -> None:
+        for name, value in prev.items():
+            if value != NB200_BAD_OPTION:
+                self.lib.nb200_set_option(name, value)
 
     def bank_to_host(self) -> HostBank:
         host = HostBank.empty(self.count)
@@ -375,6 +400,34 @@ class Simulation:
     # -- results ------------------------------------------------------------------------
     def tally_to_host(self) -> np.ndarray:
         return self.tally.download()
+
+    def tally_batches_to_host(self) -> np.ndarray:
+        """(B, ny, nx) cumulative partial tallies of the B particle batches (option
+        ``tally_batches``); flushes the caller's tally first."""
+        d = self.problem.deck
+        ncells = d.nx * d.ny
+        out = DeviceArray(self.tally_batches * ncells, np.float64)
+        try:
+            rc = self.lib.nb200_bank_tally_batches(self.bank, out.ptr, ncells)
+            if rc != self.tally_batches:
+                raise NeutralB200Error(
+                    f"bank_tally_batches: {self.lib.nb200_last_error().decode()}")
+            return out.download().reshape(self.tally_batches, d.ny, d.nx)
+        finally:
+            out.free()
+
+    def tally_relative_error(self) -> Tuple[np.ndarray, float]:
+        """Relative error of the tally from its batches: (R per cell as (ny, nx), R of the
+        tally total). R = sqrt(s^2 / B) / |m| over the batch estimates x_b = S_b N / n_b."""
+        d = self.problem.deck
+        out = DeviceArray(d.nx * d.ny, np.float64)
+        total = C.c_double(0.0)
+        try:
+            _check(self.lib.nb200_bank_tally_relerr(self.bank, out.ptr, C.byref(total)),
+                   "bank_tally_relerr")
+            return out.download().reshape(d.ny, d.nx), float(total.value)
+        finally:
+            out.free()
 
     def counters_to_host(self) -> np.ndarray:
         """(3, count) cumulative per-particle facets / collisions / census events."""
