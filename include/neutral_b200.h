@@ -365,6 +365,28 @@ int nb200_bank_tally_batches(nb200_particle_soa* particles, double* out_device, 
 int nb200_bank_tally_relerr(nb200_particle_soa* particles, double* relerr_device,
                             double* total_relerr_host);
 
+/* ------------------------------------------------------------------------------------
+ * 7. Track-length flux tally beside the energy-deposition tally. A bank with a flux array
+ *    attached adds w * l / ntotal_particles to flux[celly * nx + cellx] for every flight
+ *    segment of every later timestep: l is the segment's length in the mesh's length unit,
+ *    w the weight the particle carries along it (before an absorption at its end reduces
+ *    it, the weight the energy deposit uses), ntotal_particles the solve_transport_2d
+ *    argument. The array accumulates over timesteps; the caller zeroes it, as the energy
+ *    tally. Divided by the cell's area it is the time-integrated scalar flux per source
+ *    particle. Histories, counts, the bank and the energy tally do not change.
+ *    Refused with an error code: banks sharded over several GPUs or in a multi-process group,
+ *    banks with tally batches, and pipeline = 0 or tally_prereduce = 1 (the bank's effective
+ *    options); with a flux array attached nb200_bank_set_option refuses those two values. A
+ *    fatal error from solve_transport_2d: nx * ny differs from the attached ncells, or the
+ *    process-wide options have since turned pipeline = 0 or tally_prereduce = 1 on.
+ *    deallocate_data of the attached array detaches it; nb200_bank_free drops the attachment;
+ *    nb200_bank_copy copies particles only. The host flavour has no flux tally.
+ * ---------------------------------------------------------------------------------- */
+/* Attaches flux_device (ncells doubles, device memory on the bank's GPU) to the bank, or
+ * detaches the current array when flux_device is null. Returns 0, -4 when timesteps of the bank
+ * are pending, or another negative code (nb200_last_error). */
+int nb200_bank_set_flux_tally(nb200_particle_soa* particles, double* flux_device, size_t ncells);
+
 /* What the history kernel is bound by on facet-dominated decks, measured in place: FP64
  * reductions per second the L2 retires (csrc/microbench.cu; pattern 3 = the peak, 1 = a
  * particle's mesh walk, 0 = random cells, 5 / 6 = 32 / 4 lanes on consecutive cells) into a

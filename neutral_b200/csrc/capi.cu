@@ -79,6 +79,7 @@ uint64_t g_replica_generation = 1;     // bumped by nb200_update_replicas
 int g_shard_first = 0, g_shard_count = -1;  // nb200_set_shard
 std::unordered_set<const void*> g_handles;  // every live bank handle (what `Particle*` may be)
 std::vector<Bank*> g_batched;          // every live bank with tally batches
+std::vector<Bank*> g_flux;             // every live bank with a flux array attached
 
 // What `validate` reports besides the reference's printed lines (SURVEY.md 8f 1).
 struct StepLog {
@@ -565,6 +566,36 @@ Bank* batched_bank_of_tally(const double* tally) {
   return nullptr;
 }
 
+// ------------------------------------------------------------------------- flux tally --
+// `flux` null detaches. The attachment is the bank's own: nb200_bank_copy does not move it.
+void flux_attach(Bank* bank, double* flux, size_t ncells) {
+  g_flux.erase(std::remove(g_flux.begin(), g_flux.end(), bank), g_flux.end());
+  bank->flux = flux;
+  bank->flux_ncells = flux ? ncells : 0;
+  if (flux) g_flux.push_back(bank);
+}
+
+// deallocate_data of an attached array: no later timestep may write into the freed memory.
+void flux_detach_array(const double* buf) {
+  std::vector<Bank*> attached;
+  for (Bank* b : g_flux)
+    if (b->flux == buf) attached.push_back(b);
+  for (Bank* b : attached) flux_attach(b, nullptr, 0);
+}
+
+// Terminates on a timestep the flux kernel cannot serve (before it is enqueued): another mesh,
+// or options changed since the array was attached.
+void flux_check(Bank* bank, const StepRequest& rq, bool grouped) {
+  const size_t ncells = (size_t)rq.nx * (size_t)rq.ny;
+  if (ncells != bank->flux_ncells)
+    terminate("solve_transport_2d: the bank's flux tally has %zu cells, the mesh has %d x %d = "
+              "%zu", bank->flux_ncells, rq.nx, rq.ny, ncells);
+  if (grouped || !single_shard(bank))
+    terminate("solve_transport_2d: a flux tally in a sharded or multi-process run");
+  if (!opt_of(bank, &Options::pipeline) || opt_of(bank, &Options::tally_prereduce))
+    terminate("solve_transport_2d: a flux tally needs pipeline=1 and tally_prereduce=0");
+}
+
 // Uploads host SoA slices into the shards of `bank` (origins from 0 within each shard).
 void upload_host_soa(Bank* bank, const SoaView& host) {
   for (Shard& sh : bank->shards) {
@@ -818,6 +849,7 @@ struct ShardIO {
   double* tally;
   uint64_t *r0, *r1, *r2;
   BatchArgs batches;
+  double* flux;  // track-length flux array, or null
 };
 
 // An event the host will wait on or read a time from. While a timestep is being recorded into
@@ -944,7 +976,7 @@ void record_shard_step(DeviceCtx& c, const Bank* bank, Shard& sh, const StepRequ
     a.stagger_share = opt_of(bank, &Options::stagger_share);
     a.stagger_min = opt_of(bank, &Options::stagger_min);
     const bool fast_div = opt_of(bank, &Options::fast_div) != 0;
-    c.launches += launch_history(a, io.batches, c.d_n_live, s.n_upper, fast_div,
+    c.launches += launch_history(a, io.batches, io.flux, c.d_n_live, s.n_upper, fast_div,
                                  opt_of(bank, &Options::tally_prereduce) != 0,
                                  opt_l2 == 2 ? (const void*)io.tally
                                  : opt_l2    ? (const void*)c.d_cs_stage : nullptr,
@@ -1396,6 +1428,7 @@ void enqueue_step(Bank* bank, const StepRequest& rq) {
     epoch = group->epoch + 1;
   }
   if (bank->batches.B > 0) batches_bind(bank, rq);
+  if (bank->flux) flux_check(bank, rq, group != nullptr);
   PendingStep ps;
   ps.pipeline = opt_of(bank, &Options::pipeline) != 0;
   ps.print = opt_of(bank, &Options::print) != 0;
@@ -1420,6 +1453,7 @@ void enqueue_step(Bank* bank, const StepRequest& rq) {
     io.a_vals = replica_of(c, sh, pd, rq.a_vals, (size_t)rq.a_n);
     io.tally = rq.tally;
     io.batches = BatchArgs{bank->batches.slab, bank->batches.B, bank->n};
+    io.flux = bank->flux;
     // per-particle counters live on the primary GPU, indexed in injection order: a secondary
     // shard reaches its part of them through peer access (one 8-byte update per particle-step)
     const bool counters_ok = sh.dev == pd || (group && group->collective);
@@ -1843,6 +1877,7 @@ extern "C" void deallocate_data(double* buf) {
       if (g->target == buf) g->target = nullptr;
     for (Bank* b : g_batched)
       if (b->batches.target == buf) b->batches.target = nullptr;
+    flux_detach_array(buf);
   }
   cudaFree(buf);
 }
@@ -2282,6 +2317,7 @@ extern "C" int nb200_bank_free(nb200_particle_soa* particles) {
   if (!bank) return -3;
   finish_all(bank);
   batches_release(bank);
+  flux_attach(bank, nullptr, 0);
   if (bank->group) {
     group_flush(*bank->group);
     group_free(bank->group);
@@ -2410,6 +2446,12 @@ extern "C" int nb200_bank_set_option(nb200_particle_soa* particles, const char* 
               "kernel without tally_prereduce has batches)", name, value);
     return NB200_BAD_OPTION;
   }
+  if (bank->flux && ((spec.slot == &Options::pipeline && value == 0) ||
+                     (spec.slot == &Options::tally_prereduce && value != 0))) {
+    set_error("nb200_bank_set_option: %s=%d on a bank with a flux tally attached (only the "
+              "pipelined kernel without tally_prereduce has the flux)", name, value);
+    return NB200_BAD_OPTION;
+  }
   const int prev = opt_of(bank, spec.slot);
   for (auto& o : bank->overrides)
     if (o.first == i) {
@@ -2527,6 +2569,51 @@ extern "C" int nb200_bank_tally_relerr(nb200_particle_soa* particles, double* re
 extern "C" unsigned nb200_selftest_batch_of(uint64_t pid, uint64_t n, int nbatches) {
   if (nbatches < 1 || n > 0x7fffffffull || (uint64_t)nbatches > n || pid >= n) return UINT_MAX;
   return batch_of((unsigned)pid, (unsigned)n, (unsigned)nbatches);
+}
+
+// ------------------------------------------------------------------------- flux tally --
+extern "C" int nb200_bank_set_flux_tally(nb200_particle_soa* particles, double* flux_device,
+                                         size_t ncells) {
+  const char* who = "nb200_bank_set_flux_tally";
+  Bank* bank = bank_of(particles);
+  if (!bank) {
+    set_error("%s: not a bank handle", who);
+    return -3;
+  }
+  if (int rc = refuse_if_pending(bank, who)) return rc;
+  if (!flux_device) {
+    flux_attach(bank, nullptr, 0);
+    return 0;
+  }
+  if (!single_shard(bank) || g_mp) {
+    set_error("%s: a bank sharded over several GPUs or in a multi-process group has no flux "
+              "tally", who);
+    return -3;
+  }
+  if (bank->batches.B > 0) {
+    set_error("%s: a bank with tally_batches has no flux tally", who);
+    return -3;
+  }
+  if (!opt_of(bank, &Options::pipeline) || opt_of(bank, &Options::tally_prereduce)) {
+    set_error("%s: needs pipeline=1 and tally_prereduce=0 (only the pipelined kernel without "
+              "tally_prereduce has the flux)", who);
+    return -3;
+  }
+  if (ncells == 0 || ncells >= (1ull << 31)) {
+    set_error("%s: %zu cells (1 .. 2^31 - 1)", who, ncells);
+    return -3;
+  }
+  cudaPointerAttributes attr{};
+  if (cudaPointerGetAttributes(&attr, flux_device) != cudaSuccess ||
+      (attr.type != cudaMemoryTypeDevice && attr.type != cudaMemoryTypeManaged) ||
+      attr.device != bank->shards[0].dev) {
+    (void)cudaGetLastError();
+    set_error("%s: the flux array is not device memory on the bank's GPU %d", who,
+              bank->shards[0].dev);
+    return -3;
+  }
+  flux_attach(bank, flux_device, ncells);
+  return 0;
 }
 
 extern "C" int nb200_update_replicas(void) {

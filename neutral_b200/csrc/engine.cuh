@@ -222,6 +222,10 @@ struct TallyBatches {
 struct Bank {
   std::vector<Shard> shards;
   TallyBatches batches;
+  // nb200_bank_set_flux_tally: the caller's track-length flux array (device memory on the
+  // bank's GPU, flux_ncells doubles) every timestep also deposits into; null: none.
+  double* flux = nullptr;
+  size_t flux_ncells = 0;
   int n = 0;
   uint64_t pid0 = 0;
   int primary_dev = 0;

@@ -148,15 +148,26 @@ __device__ __forceinline__ int batch_index(const StepArgs& a, const BatchArgs& b
   return i;
 }
 
-template <bool kFastDiv, bool kPreReduce, bool kBatched>
+// kFlux (nb200_bank_set_flux_tally): every flight segment also adds w * length / ntotal to the
+// caller's flux array, at the places the energy deposits go. The track length of collisions
+// since the last flush is parked beside `edep` and flushed with it.
+struct ParkedFlux : Parked {
+  double flux[kHistoryThreads];
+};
+
+// `flux` is a kernel parameter behind the other three for the reason BatchArgs is one: a field
+// appended to StepArgs would move the offsets of the parameters that follow it.
+template <bool kFastDiv, bool kPreReduce, bool kBatched, bool kFlux>
 __global__ void NB_HISTORY_BOUNDS
-k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs bt) {
+k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs bt,
+          double* __restrict__ flux) {
 #if NB_PARK_SMEM
-  __shared__ std::conditional_t<kBatched, ParkedBatched, Parked> park;
+  __shared__ std::conditional_t<kBatched, ParkedBatched,
+                                std::conditional_t<kFlux, ParkedFlux, Parked>> park;
 #define PARKED(name) park.name[threadIdx.x]
 #define PARKED_BATCH parked_batch<kBatched>(park)
 #else
-  double park_e, park_Sig_s, park_p_absorb, park_rho, park_edep;
+  double park_e, park_Sig_s, park_p_absorb, park_rho, park_edep, park_flux;
   int park_origin, park_slot, park_batch = 0;
   unsigned park_nc;
 #define PARKED(name) park_##name
@@ -193,6 +204,7 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs
     unsigned flags = same_grid(a) ? kFlagSameGrid : 0u;
     PARKED(e) = ew.x;
     PARKED(edep) = 0.0;
+    if constexpr (kFlux) PARKED(flux) = 0.0;
     PARKED(origin) = m.w;
     if constexpr (kBatched) {
       const int b = (int)batch_of((unsigned)(a.pid0 + (uint64_t)(unsigned)m.w), (unsigned)bt.n,
@@ -277,6 +289,10 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs
             // keeps the parked slot out of the per-facet code
             tally_add<kPreReduce>(NB_TALLY_AT(NB_CELL), PARKED(edep) * a.inv_ntotal);
             PARKED(edep) = 0.0;
+            if constexpr (kFlux) {
+              tally_add<false>(flux, NB_CELL, PARKED(flux) * a.inv_ntotal);
+              PARKED(flux) = 0.0;
+            }
             flags &= ~kFlagPending;
           }
           if (!kFastDiv) flags &= ~kFlagInvStale;  // no reciprocals to refresh in this variant
@@ -304,6 +320,7 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs
         // :321-327 - deposit, flush to the tally (update_tallies, :408-420), reset
         const double edep = deposition(w, d_facet, d.stb, d.heat, nd);
         tally_add<kPreReduce>(NB_TALLY_AT(NB_CELL), edep * a.inv_ntotal);
+        if constexpr (kFlux) tally_add<false>(flux, NB_CELL, (w * d_facet) * a.inv_ntotal);
         x += d_facet * ox;
         y += d_facet * oy;
         // the edge load is consumed here, after the arithmetic it overlapped with
@@ -368,6 +385,7 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs
         const double e = PARKED(e);
         const double p_absorb = PARKED(p_absorb);
         const double edep = PARKED(edep) + deposition(w, d_coll, d.stb, d.heat, nd);  // :222-225
+        if constexpr (kFlux) PARKED(flux) = PARKED(flux) + w * d_coll;  // before absorption
         x += d_coll * ox;
         y += d_coll * oy;
         double a0, a1;
@@ -386,6 +404,7 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs
           if (e < kMinEnergyOfInterest) {  // :243-252 - the history ends here
             flags |= kFlagDead;
             tally_add<kPreReduce>(NB_TALLY_AT(NB_CELL), edep * a.inv_ntotal);
+            if constexpr (kFlux) tally_add<false>(flux, NB_CELL, PARKED(flux) * a.inv_ntotal);
             break;
           }
           // Energy and direction are unchanged: the lookups of :285-291 return the values
@@ -449,6 +468,11 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs
         double edep = deposition(w, d_census, d.stb, d.heat, nd);
         if (flags & kFlagPending) edep = PARKED(edep) + edep;
         tally_add<kPreReduce>(NB_TALLY_AT(NB_CELL), edep * a.inv_ntotal);
+        if constexpr (kFlux) {
+          double fl = w * d_census;
+          if (flags & kFlagPending) fl = PARKED(flux) + fl;
+          tally_add<false>(flux, NB_CELL, fl * a.inv_ntotal);
+        }
         dtc = 0.0;
         break;
       }
@@ -489,8 +513,8 @@ static inline int blocks_for(int n, int threads) { return (n + threads - 1) / th
 // `pin`/`pin_bytes` (optional) name the staged cross-section block: the launch then carries an
 // access-policy window that keeps it persisting in L2 (north_star phase 3), while the rest of
 // the kernel's traffic - the tally atomics above all - streams through the remainder.
-int launch_history(const StepArgs& a, const BatchArgs& bt, const unsigned* n_live, int n_upper,
-                   bool fast_div, bool prereduce, const void* pin, size_t pin_bytes, size_t pin_budget,
+int launch_history(const StepArgs& a, const BatchArgs& bt, double* flux, const unsigned* n_live,
+                   int n_upper, bool fast_div, bool prereduce, const void* pin, size_t pin_bytes, size_t pin_budget,
                    int smem_pad, cudaStream_t st) {
   if (n_upper <= 0) return 0;
   cudaLaunchConfig_t cfg = {};
@@ -502,11 +526,13 @@ int launch_history(const StepArgs& a, const BatchArgs& bt, const unsigned* n_liv
     // the number of resident CTAs per SM without touching the code.
     static int granted = 0;
     if (smem_pad > granted) {
-      cudaFuncSetAttribute(k_history<true, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
-      cudaFuncSetAttribute(k_history<true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
-      cudaFuncSetAttribute(k_history<false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
-      cudaFuncSetAttribute(k_history<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
-      cudaFuncSetAttribute(k_history<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
+      cudaFuncSetAttribute(k_history<true, true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
+      cudaFuncSetAttribute(k_history<true, false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
+      cudaFuncSetAttribute(k_history<false, false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
+      cudaFuncSetAttribute(k_history<true, false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
+      cudaFuncSetAttribute(k_history<false, false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
+      cudaFuncSetAttribute(k_history<true, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
+      cudaFuncSetAttribute(k_history<false, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
       granted = smem_pad;
     }
     cfg.dynamicSmemBytes = (size_t)smem_pad;
@@ -527,18 +553,24 @@ int launch_history(const StepArgs& a, const BatchArgs& bt, const unsigned* n_liv
   // A batched bank always runs a batched variant (the host refuses prereduce for it), so the
   // step graph of a device updates in place from one of its timesteps to the next. Banks with
   // and without batches alternating on one device change the graph's kernel and re-instantiate
-  // it instead, which is correct and costs an instantiation per switch.
-  if (bt.nbatches > 0) {
+  // it instead, which is correct and costs an instantiation per switch. A bank with a flux
+  // array attached is the same: the host refuses batches and prereduce for it.
+  if (flux) {
     if (fast_div)
-      cudaLaunchKernelEx(&cfg, k_history<true, false, true>, a, n_live, bt);
+      cudaLaunchKernelEx(&cfg, k_history<true, false, false, true>, a, n_live, bt, flux);
     else
-      cudaLaunchKernelEx(&cfg, k_history<false, false, true>, a, n_live, bt);
+      cudaLaunchKernelEx(&cfg, k_history<false, false, false, true>, a, n_live, bt, flux);
+  } else if (bt.nbatches > 0) {
+    if (fast_div)
+      cudaLaunchKernelEx(&cfg, k_history<true, false, true, false>, a, n_live, bt, flux);
+    else
+      cudaLaunchKernelEx(&cfg, k_history<false, false, true, false>, a, n_live, bt, flux);
   } else if (prereduce) {
-    cudaLaunchKernelEx(&cfg, k_history<true, true, false>, a, n_live, bt);
+    cudaLaunchKernelEx(&cfg, k_history<true, true, false, false>, a, n_live, bt, flux);
   } else if (fast_div) {
-    cudaLaunchKernelEx(&cfg, k_history<true, false, false>, a, n_live, bt);
+    cudaLaunchKernelEx(&cfg, k_history<true, false, false, false>, a, n_live, bt, flux);
   } else {
-    cudaLaunchKernelEx(&cfg, k_history<false, false, false>, a, n_live, bt);
+    cudaLaunchKernelEx(&cfg, k_history<false, false, false, false>, a, n_live, bt, flux);
   }
   return 1;
 }

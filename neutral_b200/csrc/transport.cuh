@@ -19,9 +19,10 @@ int launch_history_direct(const StepArgs& a, cudaStream_t st);
 // `alt`; history = event loop over the sorted live prefix.
 int launch_sort_phase(const StepArgs& a, const SortArgs& s, const BankView& alt,
                       cudaStream_t st);
-// bt.nbatches > 0 runs the batched variant (option tally_batches).
-int launch_history(const StepArgs& a, const BatchArgs& bt, const unsigned* n_live, int n_upper,
-                   bool fast_div, bool prereduce, const void* pin, size_t pin_bytes,
+// bt.nbatches > 0 runs the batched variant (option tally_batches); a non-null `flux` the
+// variant that also deposits the track-length flux there (nb200_bank_set_flux_tally).
+int launch_history(const StepArgs& a, const BatchArgs& bt, double* flux, const unsigned* n_live,
+                   int n_upper, bool fast_div, bool prereduce, const void* pin, size_t pin_bytes,
                    size_t pin_budget, int smem_pad, cudaStream_t st);
 // Batch partial tallies (tally_batches.cu). The slab holds the B partial tallies S_b in the
 // layout of batch_slot() and behind them one more array F of ncells: sum_b S_b as of the last

@@ -56,7 +56,7 @@ EXPORTED_SYMBOLS = [
     "nb200_bank_set_option", "nb200_bank_solve_finish", "nb200_bank_pending", "nb200_mp_init",
     "nb200_mp_connect", "nb200_mp_finalize", "nb200_tally_sync", "nb200_update_replicas",
     "nb200_microbench_red", "nb200_bank_tally_batches", "nb200_bank_tally_relerr",
-    "nb200_selftest_batch_of",
+    "nb200_selftest_batch_of", "nb200_bank_set_flux_tally",
 ]
 
 #: include/neutral_b200.h
@@ -136,6 +136,7 @@ def load_library(build: bool = False) -> C.CDLL:
     L.nb200_bank_tally_relerr.argtypes = [_soa_p, C.c_void_p, _dp]
     L.nb200_selftest_batch_of.argtypes = [C.c_uint64, C.c_uint64, C.c_int]
     L.nb200_selftest_batch_of.restype = C.c_uint
+    L.nb200_bank_set_flux_tally.argtypes = [_soa_p, C.c_void_p, C.c_size_t]
     L.nb200_last_step_stats.argtypes = [_u64p]
     L.nb200_solve_finish.argtypes = [_u64p, _u64p]
     L.nb200_kernel_launches.restype = C.c_uint64
@@ -242,7 +243,7 @@ class Simulation:
 
     def __init__(self, problem: Problem, rank: int = 0, nranks: int = 1,
                  per_particle_counters: bool = True, quiet: bool = True, ngpus: int = 1,
-                 tally_batches: int = 0):
+                 tally_batches: int = 0, flux_tally: bool = False):
         self.lib = load_library()
         require_device()
         self.problem = problem
@@ -267,6 +268,9 @@ class Simulation:
             self._cs_arrays += [dk, dv]
             self.cs.append(CrossSection(dk.ptr, dv.ptr, len(keys)))
         self.tally = DeviceArray(d.nx * d.ny, np.float64)
+        #: track-length flux per source particle (nb200_bank_set_flux_tally), attached to every
+        #: bank this simulation creates; see :meth:`scalar_flux`
+        self.flux = DeviceArray(d.nx * d.ny, np.float64) if flux_tally else None
         self.counters = [DeviceArray(max(self.count, 1), np.uint64) for _ in range(3)] \
             if per_particle_counters else None
         self.bank = None
@@ -289,6 +293,7 @@ class Simulation:
         self._restore_options(prev)
         self.lib.nb200_set_shard(0, -1)
         self.bank = out
+        self._attach_flux()
         return self.bank_bytes
 
     def load_bank(self, host: HostBank) -> None:
@@ -305,6 +310,12 @@ class Simulation:
         finally:
             self._restore_options(prev)
         self.bank = out
+        self._attach_flux()
+
+    def _attach_flux(self) -> None:
+        if self.flux is not None:
+            _check(self.lib.nb200_bank_set_flux_tally(self.bank, self.flux.ptr, self.flux.n),
+                   "bank_set_flux_tally")
 
     def _set_creation_options(self) -> dict:
         prev = {}
@@ -429,6 +440,19 @@ class Simulation:
         finally:
             out.free()
 
+    def flux_to_host(self) -> np.ndarray:
+        """(ny, nx) track length per source particle in every cell, summed over timesteps
+        (``flux_tally=True``)."""
+        d = self.problem.deck
+        return self.flux.download().reshape(d.ny, d.nx)
+
+    def scalar_flux(self) -> np.ndarray:
+        """(ny, nx) time-integrated scalar flux per source particle: :meth:`flux_to_host`
+        divided by the cell areas dx_i dy_j."""
+        dx = np.diff(self.problem.edgex)
+        dy = np.diff(self.problem.edgey)
+        return self.flux_to_host() / np.outer(dy, dx)
+
     def counters_to_host(self) -> np.ndarray:
         """(3, count) cumulative per-particle facets / collisions / census events."""
         return np.stack([c.download()[: self.count] for c in self.counters])
@@ -443,7 +467,7 @@ class Simulation:
             self.lib.nb200_bank_free(self.bank)
             self.bank = None
         for a in [self.density, self.edgex, self.edgey, self.tally] + self._cs_arrays + \
-                (self.counters or []):
+                (self.counters or []) + ([self.flux] if self.flux is not None else []):
             a.free()
 
 
