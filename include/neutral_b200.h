@@ -375,7 +375,8 @@ int nb200_bank_tally_relerr(nb200_particle_soa* particles, double* relerr_device
  *    tally. Divided by the cell's area it is the time-integrated scalar flux per source
  *    particle. Histories, counts, the bank and the energy tally do not change.
  *    Refused with an error code: banks sharded over several GPUs or in a multi-process group,
- *    banks with tally batches, and pipeline = 0 or tally_prereduce = 1 (the bank's effective
+ *    banks with tally batches (section 8 gives them a batched flux), and pipeline = 0 or
+ *    tally_prereduce = 1 (the bank's effective
  *    options); with a flux array attached nb200_bank_set_option refuses those two values. A
  *    fatal error from solve_transport_2d: nx * ny differs from the attached ncells, or the
  *    process-wide options have since turned pipeline = 0 or tally_prereduce = 1 on.
@@ -386,6 +387,39 @@ int nb200_bank_tally_relerr(nb200_particle_soa* particles, double* relerr_device
  * detaches the current array when flux_device is null. Returns 0, -4 when timesteps of the bank
  * are pending, or another negative code (nb200_last_error). */
 int nb200_bank_set_flux_tally(nb200_particle_soa* particles, double* flux_device, size_t ncells);
+
+/* ------------------------------------------------------------------------------------
+ * 8. Flux batches: a relative error beside every flux cell. A bank with tally batches
+ *    (section 6) can have a flux array attached through the call below. Its flux deposits
+ *    (section 7) then go to B partial fluxes, one per particle batch of section 6, held by the
+ *    library ((B + 1) * ncells doubles on the bank's GPU, allocated and zeroed when the array
+ *    is attached). The attached array receives what the batches gained lazily, wherever the
+ *    energy tally of a batched bank does: nb200_memcpy_* / nb200_memset_d (flushed first, then
+ *    zeroed) and copy_buffer RECV of it, nb200_tally_sync(NULL or the array), nb200_bank_free,
+ *    a detach, and the two calls below. Afterwards it equals the unbatched flux up to
+ *    summation order. The estimator is section 6's, on the flux batches. Histories, counts,
+ *    the bank and the energy tally and its batches do not change.
+ *    Refused with an error code (-4: timesteps of the bank pending; -3 otherwise): a handle
+ *    that is not a bank, a bank without tally batches, pipeline = 0 or tally_prereduce = 1,
+ *    an array that is not device memory on the bank's GPU, ncells = 0, B * ncells >= 2^31.
+ *    A null array, in this call or in nb200_bank_set_flux_tally, detaches after flushing into
+ *    the old array. deallocate_data of the attached array detaches it without a flush.
+ *    nb200_bank_set_option and solve_transport_2d refuse as in section 7.
+ * ---------------------------------------------------------------------------------- */
+/* Attaches flux_device (ncells doubles, device memory on the bank's GPU) as a batched flux with
+ * the bank's B, or detaches the current array when flux_device is null. Returns 0, -4 when
+ * timesteps of the bank are pending, or another negative code (nb200_last_error). */
+int nb200_bank_set_batched_flux_tally(nb200_particle_soa* particles, double* flux_device,
+                                      size_t ncells);
+/* Flushes, then writes the B cumulative partial fluxes as B consecutive arrays of ncells doubles
+ * (batch-major) to device memory. Returns B, or a negative code: no batched flux attached, no
+ * timestep deposited into it yet, ncells not the attached array's. */
+int nb200_bank_flux_batches(nb200_particle_soa* particles, double* out_device, size_t ncells);
+/* Flushes, then writes R of every flux cell to relerr_device (ncells doubles, device memory)
+ * and R of the flux total to *total_relerr_host. Either may be null. Returns 0 or a negative
+ * code, as nb200_bank_flux_batches. */
+int nb200_bank_flux_relerr(nb200_particle_soa* particles, double* relerr_device,
+                           double* total_relerr_host);
 
 /* What the history kernel is bound by on facet-dominated decks, measured in place: FP64
  * reductions per second the L2 retires (csrc/microbench.cu; pattern 3 = the peak, 1 = a

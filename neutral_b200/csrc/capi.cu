@@ -469,9 +469,9 @@ void batches_attach(Bank* bank, int B) {
   g_batched.push_back(bank);
 }
 
-// Brings the caller's tally up to date: target += sum_b S_b - F, F = sum_b S_b. Synchronous.
-void batches_flush(Bank* bank) {
-  TallyBatches& tb = bank->batches;
+// Brings the target of `tb` up to date (the caller's tally for bank->batches, the attached flux
+// array for bank->flux_batches): target += sum_b S_b - F, F = sum_b S_b. Synchronous.
+void batches_flush(Bank* bank, TallyBatches& tb) {
   if (!tb.dirty || !tb.target) return;
   const Shard& sh = bank->shards[0];
   DeviceGuard guard(sh.dev);
@@ -482,16 +482,15 @@ void batches_flush(Bank* bank) {
   tb.dirty = false;
 }
 
-void batches_release(Bank* bank) {
-  TallyBatches& tb = bank->batches;
+// Flushes `tb` into its target (if it still has one), frees its slab and clears it.
+void batches_release(Bank* bank, TallyBatches& tb) {
   if (tb.B <= 0) return;
-  batches_flush(bank);
+  batches_flush(bank, tb);
   if (tb.slab) {
     DeviceGuard guard(bank->shards[0].dev);
     cudaFree(tb.slab);
   }
   tb = TallyBatches{};
-  g_batched.erase(std::remove(g_batched.begin(), g_batched.end(), bank), g_batched.end());
 }
 
 // Binds the batches to the tally and mesh of a timestep (before it is enqueued): another tally
@@ -511,7 +510,7 @@ void batches_bind(Bank* bank, const StepRequest& rq) {
     terminate("solve_transport_2d: tally_batches=%d over %zu cells needs 2^31 or more tally "
               "slots (the history kernel indexes them with 32 bits)", tb.B, ncells);
   if (tb.target == rq.tally && tb.ncells == ncells) return;
-  batches_flush(bank);
+  batches_flush(bank, tb);
   const Shard& sh = bank->shards[0];
   DeviceGuard guard(sh.dev);
   DeviceCtx& c = ctx_on(sh.dev);
@@ -528,10 +527,9 @@ void batches_bind(Bank* bank, const StepRequest& rq) {
   tb.target = rq.tally;
 }
 
-// R of the tally total: the B batch totals through a fixed-order device reduction, then the
-// estimator in FP64 on the host.
-double batches_total_relerr(Bank* bank) {
-  TallyBatches& tb = bank->batches;
+// R of the total of `tb` (tally or flux): the B batch totals through a fixed-order device
+// reduction, then the estimator in FP64 on the host.
+double batches_total_relerr(Bank* bank, const TallyBatches& tb) {
   const Shard& sh = bank->shards[0];
   DeviceGuard guard(sh.dev);
   DeviceCtx& c = ctx_on(sh.dev);
@@ -568,19 +566,49 @@ Bank* batched_bank_of_tally(const double* tally) {
 
 // ------------------------------------------------------------------------- flux tally --
 // `flux` null detaches. The attachment is the bank's own: nb200_bank_copy does not move it.
-void flux_attach(Bank* bank, double* flux, size_t ncells) {
+// A batched flux of the old attachment is flushed into the old array and its slab freed first.
+// B > 0 attaches a batched flux: deposits go to a zeroed slab of B partial fluxes on the bank's
+// GPU, allocated here. Returns 0, or -2 (error set) when the slab cannot be had.
+int flux_attach(Bank* bank, double* flux, size_t ncells, int B = 0) {
+  batches_release(bank, bank->flux_batches);
   g_flux.erase(std::remove(g_flux.begin(), g_flux.end(), bank), g_flux.end());
+  bank->flux = nullptr;
+  bank->flux_ncells = 0;
+  if (!flux) return 0;
+  if (B > 0) {
+    DeviceGuard guard(bank->shards[0].dev);
+    DeviceCtx& c = ctx_on(bank->shards[0].dev);
+    const size_t bytes = sizeof(double) * (size_t)(B + 1) * ncells;
+    double* slab = nullptr;
+    CU_TRY(cudaMalloc(&slab, bytes));
+    if (cudaError_t err = cudaMemsetAsync(slab, 0, bytes, c.stream)) {
+      cudaFree(slab);
+      set_error("cudaMemsetAsync of the flux batch slab failed: %s", cudaGetErrorString(err));
+      return -2;
+    }
+    // the bank has a batched flux only once its slab is whole
+    TallyBatches& tb = bank->flux_batches;
+    tb.slab = slab;
+    tb.B = B;
+    tb.ncells = ncells;
+    tb.target = flux;
+  }
   bank->flux = flux;
-  bank->flux_ncells = flux ? ncells : 0;
-  if (flux) g_flux.push_back(bank);
+  bank->flux_ncells = ncells;
+  g_flux.push_back(bank);
+  return 0;
 }
 
-// deallocate_data of an attached array: no later timestep may write into the freed memory.
+// deallocate_data of an attached array: no later timestep may write into the freed memory, and
+// nothing is flushed into it.
 void flux_detach_array(const double* buf) {
   std::vector<Bank*> attached;
   for (Bank* b : g_flux)
     if (b->flux == buf) attached.push_back(b);
-  for (Bank* b : attached) flux_attach(b, nullptr, 0);
+  for (Bank* b : attached) {
+    b->flux_batches.target = nullptr;
+    flux_attach(b, nullptr, 0);
+  }
 }
 
 // Terminates on a timestep the flux kernel cannot serve (before it is enqueued): another mesh,
@@ -1337,14 +1365,17 @@ void group_flush(TallyGroup& g) {
 // Any library-mediated look at memory that a group's unflushed contributions belong to
 // flushes first (validate, copy_buffer, the nb200_memcpy / memset helpers).
 void flush_groups_touching(const void* ptr, size_t bytes) {
-  for (Bank* b : g_batched) {
-    const TallyBatches& tb = b->batches;
-    if (!tb.dirty || !tb.target) continue;
+  auto touches = [ptr, bytes](const TallyBatches& tb) {
+    if (!tb.dirty || !tb.target) return false;
     const char* lo = (const char*)tb.target;
     const char* hi = lo + tb.ncells * 8;
     const char* p = (const char*)ptr;
-    if (p < hi && p + bytes > lo) batches_flush(b);
-  }
+    return p < hi && p + bytes > lo;
+  };
+  for (Bank* b : g_batched)
+    if (touches(b->batches)) batches_flush(b, b->batches);
+  for (Bank* b : g_flux)
+    if (touches(b->flux_batches)) batches_flush(b, b->flux_batches);
   for (TallyGroup* g : g_groups) {
     if (!g->dirty || !g->target) continue;
     const char* lo = (const char*)g->target;
@@ -1453,7 +1484,7 @@ void enqueue_step(Bank* bank, const StepRequest& rq) {
     io.a_vals = replica_of(c, sh, pd, rq.a_vals, (size_t)rq.a_n);
     io.tally = rq.tally;
     io.batches = BatchArgs{bank->batches.slab, bank->batches.B, bank->n};
-    io.flux = bank->flux;
+    io.flux = bank->flux_batches.B > 0 ? bank->flux_batches.slab : bank->flux;
     // per-particle counters live on the primary GPU, indexed in injection order: a secondary
     // shard reaches its part of them through peer access (one 8-byte update per particle-step)
     const bool counters_ok = sh.dev == pd || (group && group->collective);
@@ -1475,6 +1506,7 @@ void enqueue_step(Bank* bank, const StepRequest& rq) {
     }
   }
   if (bank->batches.B > 0) bank->batches.dirty = true;
+  if (bank->flux_batches.B > 0) bank->flux_batches.dirty = bank->flux_batches.deposited = true;
   if (group) {
     group->steps_deposited++;
     group->dirty = true;
@@ -1823,7 +1855,7 @@ extern "C" void validate(const int nx, const int ny, const char* params_filename
   if (json && *json) {
     if (Bank* b = batched_bank_of_tally(energy_tally)) {
       batches = b->batches.B;
-      total_relerr = batches_total_relerr(b);
+      total_relerr = batches_total_relerr(b, b->batches);
     }
   }
   printf("\nFinal global_energy_tally %.15e\n", total);
@@ -1872,12 +1904,12 @@ extern "C" void deallocate_data(double* buf) {
   // a tally that a sharded run still owes contributions to is completed before it goes away,
   // and no group keeps pointing at freed memory
   if (buf) {
+    flux_detach_array(buf);
     flush_groups_touching(buf, sizeof(double));
     for (TallyGroup* g : g_groups)
       if (g->target == buf) g->target = nullptr;
     for (Bank* b : g_batched)
       if (b->batches.target == buf) b->batches.target = nullptr;
-    flux_detach_array(buf);
   }
   cudaFree(buf);
 }
@@ -2316,7 +2348,8 @@ extern "C" int nb200_bank_free(nb200_particle_soa* particles) {
   Bank* bank = bank_of(particles);
   if (!bank) return -3;
   finish_all(bank);
-  batches_release(bank);
+  batches_release(bank, bank->batches);
+  g_batched.erase(std::remove(g_batched.begin(), g_batched.end(), bank), g_batched.end());
   flux_attach(bank, nullptr, 0);
   if (bank->group) {
     group_flush(*bank->group);
@@ -2504,7 +2537,9 @@ extern "C" int nb200_tally_sync(double* tally_device) {
   CTX_OR_RETURN(c);
   (void)c;
   for (Bank* b : g_batched)
-    if (!tally_device || b->batches.target == tally_device) batches_flush(b);
+    if (!tally_device || b->batches.target == tally_device) batches_flush(b, b->batches);
+  for (Bank* b : g_flux)
+    if (!tally_device || b->flux == tally_device) batches_flush(b, b->flux_batches);
   for (TallyGroup* g : g_groups)
     if (!tally_device || g->target == tally_device) group_flush(*g);
   return 0;
@@ -2522,7 +2557,7 @@ static Bank* flushed_batches(nb200_particle_soa* particles, const char* who) {
     set_error("%s: no timestep of this bank has deposited into its batches yet", who);
     return nullptr;
   }
-  batches_flush(bank);
+  batches_flush(bank, bank->batches);
   return bank;
 }
 
@@ -2560,7 +2595,7 @@ extern "C" int nb200_bank_tally_relerr(nb200_particle_soa* particles, double* re
     CU_TRY(cudaGetLastError());
     CU_TRY(cudaStreamSynchronize(c.stream));
   }
-  if (total_relerr_host) *total_relerr_host = batches_total_relerr(bank);
+  if (total_relerr_host) *total_relerr_host = batches_total_relerr(bank, tb);
   return 0;
 }
 
@@ -2572,26 +2607,22 @@ extern "C" unsigned nb200_selftest_batch_of(uint64_t pid, uint64_t n, int nbatch
 }
 
 // ------------------------------------------------------------------------- flux tally --
-extern "C" int nb200_bank_set_flux_tally(nb200_particle_soa* particles, double* flux_device,
-                                         size_t ncells) {
-  const char* who = "nb200_bank_set_flux_tally";
-  Bank* bank = bank_of(particles);
-  if (!bank) {
-    set_error("%s: not a bank handle", who);
-    return -3;
-  }
-  if (int rc = refuse_if_pending(bank, who)) return rc;
-  if (!flux_device) {
-    flux_attach(bank, nullptr, 0);
-    return 0;
-  }
+// Why flux_device cannot be attached to the bank (plain, or batched with the bank's B), as an
+// error code with the message set; 0 if it can. Both attach functions check the same things.
+static int refuse_flux_array(Bank* bank, double* flux_device, size_t ncells, bool batched,
+                             const char* who) {
   if (!single_shard(bank) || g_mp) {
     set_error("%s: a bank sharded over several GPUs or in a multi-process group has no flux "
               "tally", who);
     return -3;
   }
-  if (bank->batches.B > 0) {
-    set_error("%s: a bank with tally_batches has no flux tally", who);
+  if (!batched && bank->batches.B > 0) {
+    set_error("%s: a bank with tally_batches has no flux tally (nb200_bank_set_batched_flux_tally "
+              "attaches a batched one)", who);
+    return -3;
+  }
+  if (batched && bank->batches.B <= 0) {
+    set_error("%s: the bank has no tally_batches (a batched flux has the bank's batches)", who);
     return -3;
   }
   if (!opt_of(bank, &Options::pipeline) || opt_of(bank, &Options::tally_prereduce)) {
@@ -2603,6 +2634,11 @@ extern "C" int nb200_bank_set_flux_tally(nb200_particle_soa* particles, double* 
     set_error("%s: %zu cells (1 .. 2^31 - 1)", who, ncells);
     return -3;
   }
+  if (batched && (unsigned long long)ncells * (unsigned long long)bank->batches.B >= (1ull << 31)) {
+    set_error("%s: tally_batches=%d over %zu cells needs 2^31 or more flux slots (the history "
+              "kernel indexes them with 32 bits)", who, bank->batches.B, ncells);
+    return -3;
+  }
   cudaPointerAttributes attr{};
   if (cudaPointerGetAttributes(&attr, flux_device) != cudaSuccess ||
       (attr.type != cudaMemoryTypeDevice && attr.type != cudaMemoryTypeManaged) ||
@@ -2612,7 +2648,83 @@ extern "C" int nb200_bank_set_flux_tally(nb200_particle_soa* particles, double* 
               bank->shards[0].dev);
     return -3;
   }
-  flux_attach(bank, flux_device, ncells);
+  return 0;
+}
+
+extern "C" int nb200_bank_set_flux_tally(nb200_particle_soa* particles, double* flux_device,
+                                         size_t ncells) {
+  const char* who = "nb200_bank_set_flux_tally";
+  Bank* bank = bank_of(particles);
+  if (!bank) {
+    set_error("%s: not a bank handle", who);
+    return -3;
+  }
+  if (int rc = refuse_if_pending(bank, who)) return rc;
+  if (!flux_device) return flux_attach(bank, nullptr, 0);
+  if (int rc = refuse_flux_array(bank, flux_device, ncells, false, who)) return rc;
+  return flux_attach(bank, flux_device, ncells);
+}
+
+extern "C" int nb200_bank_set_batched_flux_tally(nb200_particle_soa* particles,
+                                                 double* flux_device, size_t ncells) {
+  const char* who = "nb200_bank_set_batched_flux_tally";
+  Bank* bank = bank_of(particles);
+  if (!bank) {
+    set_error("%s: not a bank handle", who);
+    return -3;
+  }
+  if (int rc = refuse_if_pending(bank, who)) return rc;
+  if (!flux_device) return flux_attach(bank, nullptr, 0);
+  if (int rc = refuse_flux_array(bank, flux_device, ncells, true, who)) return rc;
+  return flux_attach(bank, flux_device, ncells, bank->batches.B);
+}
+
+// The bank's flux batches, flushed into the attached array; nullptr (error set) if there are none.
+static Bank* flushed_flux_batches(nb200_particle_soa* particles, const char* who) {
+  Bank* bank = bank_of(particles);
+  if (!bank || bank->flux_batches.B <= 0) {
+    set_error("%s: not a bank handle with a batched flux tally attached", who);
+    return nullptr;
+  }
+  if (!bank->flux_batches.deposited) {
+    set_error("%s: no timestep of this bank has deposited into its flux batches yet", who);
+    return nullptr;
+  }
+  batches_flush(bank, bank->flux_batches);
+  return bank;
+}
+
+extern "C" int nb200_bank_flux_batches(nb200_particle_soa* particles, double* out_device,
+                                       size_t ncells) {
+  Bank* bank = flushed_flux_batches(particles, "nb200_bank_flux_batches");
+  if (!bank) return -3;
+  const TallyBatches& tb = bank->flux_batches;
+  if (!out_device || ncells != tb.ncells) {
+    set_error("nb200_bank_flux_batches: the flux batches cover %zu cells, %zu were asked for",
+              tb.ncells, ncells);
+    return -3;
+  }
+  DeviceGuard guard(bank->shards[0].dev);
+  DeviceCtx& c = ctx_on(bank->shards[0].dev);
+  c.launches += launch_batch_export(tb.slab, tb.B, tb.ncells, out_device, c.stream);
+  CU_TRY(cudaGetLastError());
+  CU_TRY(cudaStreamSynchronize(c.stream));
+  return tb.B;
+}
+
+extern "C" int nb200_bank_flux_relerr(nb200_particle_soa* particles, double* relerr_device,
+                                      double* total_relerr_host) {
+  Bank* bank = flushed_flux_batches(particles, "nb200_bank_flux_relerr");
+  if (!bank) return -3;
+  const TallyBatches& tb = bank->flux_batches;
+  DeviceGuard guard(bank->shards[0].dev);
+  DeviceCtx& c = ctx_on(bank->shards[0].dev);
+  if (relerr_device) {
+    c.launches += launch_batch_relerr(tb.slab, tb.B, tb.ncells, bank->n, relerr_device, c.stream);
+    CU_TRY(cudaGetLastError());
+    CU_TRY(cudaStreamSynchronize(c.stream));
+  }
+  if (total_relerr_host) *total_relerr_host = batches_total_relerr(bank, tb);
   return 0;
 }
 

@@ -217,6 +217,7 @@ struct TallyBatches {
   size_t ncells = 0;
   double* target = nullptr;  // the caller-visible tally the batches belong to
   bool dirty = false;        // the batches hold deposits the target has not received
+  bool deposited = false;    // a timestep has deposited into this slab
 };
 
 struct Bank {
@@ -226,6 +227,9 @@ struct Bank {
   // bank's GPU, flux_ncells doubles) every timestep also deposits into; null: none.
   double* flux = nullptr;
   size_t flux_ncells = 0;
+  // nb200_bank_set_batched_flux_tally: B > 0 (the B of `batches`) when the flux deposits go to
+  // B partial fluxes instead; their target is `flux`, their slab is allocated when it attaches.
+  TallyBatches flux_batches;
   int n = 0;
   uint64_t pid0 = 0;
   int primary_dev = 0;

@@ -155,6 +155,12 @@ struct ParkedFlux : Parked {
   double flux[kHistoryThreads];
 };
 
+// kBatched and kFlux together (nb200_bank_set_batched_flux_tally): `flux` is the library's flux
+// batch slab, indexed like the energy batches, and the flux parks beside the batch.
+struct ParkedBatchedFlux : ParkedBatched {
+  double flux[kHistoryThreads];
+};
+
 // `flux` is a kernel parameter behind the other three for the reason BatchArgs is one: a field
 // appended to StepArgs would move the offsets of the parameters that follow it.
 template <bool kFastDiv, bool kPreReduce, bool kBatched, bool kFlux>
@@ -162,7 +168,7 @@ __global__ void NB_HISTORY_BOUNDS
 k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs bt,
           double* __restrict__ flux) {
 #if NB_PARK_SMEM
-  __shared__ std::conditional_t<kBatched, ParkedBatched,
+  __shared__ std::conditional_t<kBatched, std::conditional_t<kFlux, ParkedBatchedFlux, ParkedBatched>,
                                 std::conditional_t<kFlux, ParkedFlux, Parked>> park;
 #define PARKED(name) park.name[threadIdx.x]
 #define PARKED_BATCH parked_batch<kBatched>(park)
@@ -201,6 +207,8 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs
     // the base and index a deposit into `cell` goes to: the caller's tally, or the batch's slot
 #define NB_TALLY_AT(cell) \
   (kBatched ? bt.slab : a.tally), (kBatched ? batch_index(a, bt, PARKED_BATCH, (cell)) : (cell))
+    // ... and a flux deposit: the caller's array, or (batched) the batch's slot of the flux slab
+#define NB_FLUX_AT(cell) flux, (kBatched ? batch_index(a, bt, PARKED_BATCH, (cell)) : (cell))
     unsigned flags = same_grid(a) ? kFlagSameGrid : 0u;
     PARKED(e) = ew.x;
     PARKED(edep) = 0.0;
@@ -290,7 +298,7 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs
             tally_add<kPreReduce>(NB_TALLY_AT(NB_CELL), PARKED(edep) * a.inv_ntotal);
             PARKED(edep) = 0.0;
             if constexpr (kFlux) {
-              tally_add<false>(flux, NB_CELL, PARKED(flux) * a.inv_ntotal);
+              tally_add<false>(NB_FLUX_AT(NB_CELL), PARKED(flux) * a.inv_ntotal);
               PARKED(flux) = 0.0;
             }
             flags &= ~kFlagPending;
@@ -320,7 +328,7 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs
         // :321-327 - deposit, flush to the tally (update_tallies, :408-420), reset
         const double edep = deposition(w, d_facet, d.stb, d.heat, nd);
         tally_add<kPreReduce>(NB_TALLY_AT(NB_CELL), edep * a.inv_ntotal);
-        if constexpr (kFlux) tally_add<false>(flux, NB_CELL, (w * d_facet) * a.inv_ntotal);
+        if constexpr (kFlux) tally_add<false>(NB_FLUX_AT(NB_CELL), (w * d_facet) * a.inv_ntotal);
         x += d_facet * ox;
         y += d_facet * oy;
         // the edge load is consumed here, after the arithmetic it overlapped with
@@ -404,7 +412,7 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs
           if (e < kMinEnergyOfInterest) {  // :243-252 - the history ends here
             flags |= kFlagDead;
             tally_add<kPreReduce>(NB_TALLY_AT(NB_CELL), edep * a.inv_ntotal);
-            if constexpr (kFlux) tally_add<false>(flux, NB_CELL, PARKED(flux) * a.inv_ntotal);
+            if constexpr (kFlux) tally_add<false>(NB_FLUX_AT(NB_CELL), PARKED(flux) * a.inv_ntotal);
             break;
           }
           // Energy and direction are unchanged: the lookups of :285-291 return the values
@@ -471,7 +479,7 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs
         if constexpr (kFlux) {
           double fl = w * d_census;
           if (flags & kFlagPending) fl = PARKED(flux) + fl;
-          tally_add<false>(flux, NB_CELL, fl * a.inv_ntotal);
+          tally_add<false>(NB_FLUX_AT(NB_CELL), fl * a.inv_ntotal);
         }
         dtc = 0.0;
         break;
@@ -505,6 +513,7 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs
 #undef PARKED
 #undef NB_CELL
 #undef NB_TALLY_AT
+#undef NB_FLUX_AT
 #undef PARKED_BATCH
 }
 
@@ -533,6 +542,8 @@ int launch_history(const StepArgs& a, const BatchArgs& bt, double* flux, const u
       cudaFuncSetAttribute(k_history<false, false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
       cudaFuncSetAttribute(k_history<true, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
       cudaFuncSetAttribute(k_history<false, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
+      cudaFuncSetAttribute(k_history<true, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
+      cudaFuncSetAttribute(k_history<false, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
       granted = smem_pad;
     }
     cfg.dynamicSmemBytes = (size_t)smem_pad;
@@ -554,8 +565,14 @@ int launch_history(const StepArgs& a, const BatchArgs& bt, double* flux, const u
   // step graph of a device updates in place from one of its timesteps to the next. Banks with
   // and without batches alternating on one device change the graph's kernel and re-instantiate
   // it instead, which is correct and costs an instantiation per switch. A bank with a flux
-  // array attached is the same: the host refuses batches and prereduce for it.
-  if (flux) {
+  // array attached is the same: the host refuses prereduce for it, and a batched bank's flux is
+  // always batched (its `flux` is the flux batch slab).
+  if (flux && bt.nbatches > 0) {
+    if (fast_div)
+      cudaLaunchKernelEx(&cfg, k_history<true, false, true, true>, a, n_live, bt, flux);
+    else
+      cudaLaunchKernelEx(&cfg, k_history<false, false, true, true>, a, n_live, bt, flux);
+  } else if (flux) {
     if (fast_div)
       cudaLaunchKernelEx(&cfg, k_history<true, false, false, true>, a, n_live, bt, flux);
     else

@@ -56,7 +56,8 @@ EXPORTED_SYMBOLS = [
     "nb200_bank_set_option", "nb200_bank_solve_finish", "nb200_bank_pending", "nb200_mp_init",
     "nb200_mp_connect", "nb200_mp_finalize", "nb200_tally_sync", "nb200_update_replicas",
     "nb200_microbench_red", "nb200_bank_tally_batches", "nb200_bank_tally_relerr",
-    "nb200_selftest_batch_of", "nb200_bank_set_flux_tally",
+    "nb200_selftest_batch_of", "nb200_bank_set_flux_tally", "nb200_bank_set_batched_flux_tally",
+    "nb200_bank_flux_batches", "nb200_bank_flux_relerr",
 ]
 
 #: include/neutral_b200.h
@@ -137,6 +138,9 @@ def load_library(build: bool = False) -> C.CDLL:
     L.nb200_selftest_batch_of.argtypes = [C.c_uint64, C.c_uint64, C.c_int]
     L.nb200_selftest_batch_of.restype = C.c_uint
     L.nb200_bank_set_flux_tally.argtypes = [_soa_p, C.c_void_p, C.c_size_t]
+    L.nb200_bank_set_batched_flux_tally.argtypes = [_soa_p, C.c_void_p, C.c_size_t]
+    L.nb200_bank_flux_batches.argtypes = [_soa_p, C.c_void_p, C.c_size_t]
+    L.nb200_bank_flux_relerr.argtypes = [_soa_p, C.c_void_p, _dp]
     L.nb200_last_step_stats.argtypes = [_u64p]
     L.nb200_solve_finish.argtypes = [_u64p, _u64p]
     L.nb200_kernel_launches.restype = C.c_uint64
@@ -269,7 +273,8 @@ class Simulation:
             self.cs.append(CrossSection(dk.ptr, dv.ptr, len(keys)))
         self.tally = DeviceArray(d.nx * d.ny, np.float64)
         #: track-length flux per source particle (nb200_bank_set_flux_tally), attached to every
-        #: bank this simulation creates; see :meth:`scalar_flux`
+        #: bank this simulation creates; see :meth:`scalar_flux`. With ``tally_batches`` it is
+        #: batched too (nb200_bank_set_batched_flux_tally), see :meth:`flux_relative_error`
         self.flux = DeviceArray(d.nx * d.ny, np.float64) if flux_tally else None
         self.counters = [DeviceArray(max(self.count, 1), np.uint64) for _ in range(3)] \
             if per_particle_counters else None
@@ -313,7 +318,13 @@ class Simulation:
         self._attach_flux()
 
     def _attach_flux(self) -> None:
-        if self.flux is not None:
+        if self.flux is None:
+            return
+        if self.tally_batches:
+            _check(self.lib.nb200_bank_set_batched_flux_tally(self.bank, self.flux.ptr,
+                                                              self.flux.n),
+                   "bank_set_batched_flux_tally")
+        else:
             _check(self.lib.nb200_bank_set_flux_tally(self.bank, self.flux.ptr, self.flux.n),
                    "bank_set_flux_tally")
 
@@ -452,6 +463,36 @@ class Simulation:
         dx = np.diff(self.problem.edgex)
         dy = np.diff(self.problem.edgey)
         return self.flux_to_host() / np.outer(dy, dx)
+
+    def flux_batches_to_host(self) -> np.ndarray:
+        """(B, ny, nx) cumulative partial fluxes of the B particle batches (``flux_tally=True``
+        with ``tally_batches``); flushes the flux array first."""
+        d = self.problem.deck
+        ncells = d.nx * d.ny
+        out = DeviceArray(self.tally_batches * ncells, np.float64)
+        try:
+            rc = self.lib.nb200_bank_flux_batches(self.bank, out.ptr, ncells)
+            if rc != self.tally_batches:
+                raise NeutralB200Error(
+                    f"bank_flux_batches: {self.lib.nb200_last_error().decode()}")
+            return out.download().reshape(self.tally_batches, d.ny, d.nx)
+        finally:
+            out.free()
+
+    def flux_relative_error(self) -> Tuple[np.ndarray, float]:
+        """Relative error of the flux from its batches: (R per cell as (ny, nx), R of the flux
+        total), with the estimator of :meth:`tally_relative_error`. :meth:`scalar_flux` has the
+        same R per cell, because it divides every batch of a cell by the same exact constant,
+        the cell's area."""
+        d = self.problem.deck
+        out = DeviceArray(d.nx * d.ny, np.float64)
+        total = C.c_double(0.0)
+        try:
+            _check(self.lib.nb200_bank_flux_relerr(self.bank, out.ptr, C.byref(total)),
+                   "bank_flux_relerr")
+            return out.download().reshape(d.ny, d.nx), float(total.value)
+        finally:
+            out.free()
 
     def counters_to_host(self) -> np.ndarray:
         """(3, count) cumulative per-particle facets / collisions / census events."""

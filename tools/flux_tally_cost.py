@@ -6,7 +6,12 @@ runs of each the next --runs are timed with CUDA events. Reported: median ms per
 events/s of each, their ratio, and the tally and flux totals (the tally totals of the two must
 agree to summation order).
 
+With --tally-batches B both banks have B tally batches (option tally_batches), and the flux of
+the second is batched too (nb200_bank_set_batched_flux_tally): what the flux batches cost on top
+of the energy batches.
+
     python tools/flux_tally_cost.py --out profiles/r04/flux_tally_cost.json
+    python tools/flux_tally_cost.py --tally-batches 16 --out flux_batches_cost_b16.json
 
 The GPU's name and power limit are written into the same output. Needs a CUDA device.
 """
@@ -38,7 +43,8 @@ def measure(args) -> dict:
     out = {}
     for deck in args.decks:
         prob = build_problem(deck)
-        sims = {flux: Simulation(prob, per_particle_counters=False, flux_tally=flux)
+        sims = {flux: Simulation(prob, per_particle_counters=False, flux_tally=flux,
+                                 tally_batches=args.tally_batches)
                 for flux in (False, True)}
         for sim in sims.values():
             sim.inject()
@@ -87,11 +93,14 @@ def main():
     ap.add_argument("--decks", nargs="+", default=["csp", "split", "stream", "scatter"])
     ap.add_argument("--runs", type=int, default=10)
     ap.add_argument("--warmup", type=int, default=2)
+    ap.add_argument("--tally-batches", type=int, default=0,
+                    help="B > 0: both banks batched, the flux of the second batched too")
     ap.add_argument("--out", default=None, help="JSON file for the results")
     args = ap.parse_args()
     result = {"what": "ms per resident deck run (run_pipelined, CUDA events, median) without "
                       "and with a flux array attached, alternating run by run; events/s",
               **gpu_identity(), "runs": args.runs, "warmup": args.warmup,
+              "tally_batches": args.tally_batches,
               "decks": measure(args)}
     text = json.dumps(result, indent=1)
     print(text)
