@@ -97,6 +97,53 @@ def test_device_cross_section_brackets(gpu_lib, port):
         assert out[i] == port.cs_lookup(keys, values, float(e[i]))
 
 
+def _adversarial_tables():
+    """Tables at the edges of the staged lookup's bucket index (8192 buckets over the leading
+    bits of the key range; stage.cu, cs_params_from_ends)."""
+    rng = np.random.default_rng(23)
+    crowd = np.unique(np.concatenate([
+        1.0e3 * (1.0 + np.arange(10_000) * 1.0e-13),           # within 1e-9 of one value
+        [1.0e-3, 0.5, 7.0e2, 2.0e3, 1.0e6, 1.0e8]]))            # ... and a few far keys
+    one = np.float64(1.0).view(np.uint64)
+    return {
+        "2": np.array([0.5, 3.0]),
+        "3": np.array([1.0e-2, 1.0, 1.0e8]),
+        "8193": np.cumsum(rng.uniform(0.5, 1.5, 8193)),
+        "50000": np.geomspace(1.0e-3, 1.0e8, 50_000),
+        "crowded": crowd,
+        "consecutive": (one + np.arange(3000, dtype=np.uint64)).view(np.float64),  # shift 0
+        "1e-300..1e300": np.geomspace(1.0e-300, 1.0e300, 6000),
+    }
+
+
+@pytest.mark.parametrize("name", list(_adversarial_tables()))
+def test_device_cross_section_brackets_on_adversarial_tables(gpu_lib, port, name):
+    """The staged lookup (bucket index + bisection) against the plain bisection on the device
+    (k_selftest_cs reports -1 where they differ) and the oracle port, bit for bit: at every key,
+    one ulp either side of it, the midpoints, the ends, and outside the table (clamped)."""
+    keys = np.ascontiguousarray(_adversarial_tables()[name])
+    assert np.all(np.diff(keys) > 0.0)
+    values = np.ascontiguousarray(np.random.default_rng(len(keys)).uniform(0.5, 2.0, len(keys)))
+    e = np.concatenate([keys, np.nextafter(keys, 0.0), np.nextafter(keys, np.inf),
+                        0.5 * (keys[:-1] + keys[1:]),
+                        [0.0, 5e-324, 0.5 * keys[0], keys[-1] * 2.0, 1.0e308]])
+    e = np.ascontiguousarray(e)
+    ind = np.zeros(len(e), dtype=np.int32)
+    out = np.zeros(len(e))
+    rc = gpu_lib.nb200_selftest_cs(keys.ctypes.data_as(_dp), values.ctypes.data_as(_dp),
+                                   len(keys), e.ctypes.data_as(_dp), len(e),
+                                   ind.ctypes.data_as(C.POINTER(C.c_int)),
+                                   out.ctypes.data_as(_dp))
+    assert rc == 0
+    assert np.count_nonzero(ind == -1) == 0, "staged and plain lookups differ"
+    want_i = np.array([port.cs_index(keys, float(x)) for x in e])
+    want_v = np.array([port.cs_lookup(keys, values, float(x)) for x in e])
+    bad = np.flatnonzero(ind != want_i)
+    assert len(bad) == 0, [(e[i].hex(), ind[i], want_i[i]) for i in bad[:5]]
+    bad = np.flatnonzero(out.view(np.uint64) != want_v.view(np.uint64))
+    assert len(bad) == 0, [(e[i].hex(), out[i], want_v[i]) for i in bad[:5]]
+
+
 def test_reciprocal_division_is_ieee_division(gpu_lib):
     """The event loop divides by loop-invariant divisors (speed, cell mean free path) through
     their correctly rounded reciprocals with a Markstein correction step; the quotient must
