@@ -224,7 +224,9 @@ int nb200_memset_d(void* dst_device, int value, size_t bytes);
 int nb200_synchronize(void);
 
 /* dst[i] += src[i] on the device: combines per-step tally deltas of a particle-sharded run
- * (after the all-reduce of the deltas, SURVEY.md 8e). */
+ * (after the all-reduce of the deltas, SURVEY.md 8e). dst and src need only the 8-byte
+ * alignment of a double (e.g. base + 1 element); 16-byte aligned pointers take a vector path
+ * with the same result. */
 int nb200_accumulate(double* dst_device, const double* src_device, size_t n);
 /* The same, and src[i] = 0 afterwards (the delta buffer is ready for its next timestep). */
 int nb200_accumulate_clear(double* dst_device, double* src_device, size_t n);
@@ -319,6 +321,9 @@ uint64_t nb200_kernel_launches(void);
  *      - one process per GPU (torchrun, MPI): nb200_set_shard + nb200_mp_init on every rank,
  *        exchange the blobs with whatever the host has (torch.distributed.all_gather, MPI),
  *        nb200_mp_connect. From then on solve_transport_2d on that GPU takes part in the group.
+ *    The tally of a sharded run, like that of a single-GPU one, may be any 8-byte aligned
+ *    double array (e.g. base + 1 element): the gather into it takes 16-byte accesses only
+ *    when the tally is 16-byte aligned.
  * ---------------------------------------------------------------------------------- */
 /* Allocates this rank's part of the group for a tally of `ncells` doubles on the current GPU
  * and writes NB200_MP_BLOB_BYTES bytes the peers need into blob_out. */

@@ -110,16 +110,24 @@ k_reduce_fold(const GroupView g, double* __restrict__ owned, unsigned long long 
 
 
 // All-gather fused with the accumulation into the caller-visible tally: slice by slice,
-// straight out of the owners' memory.
+// straight out of the owners' memory. The caller's tally need only be 8-byte aligned; the
+// owned slices are 256-byte aligned and every slice starts at an even cell (chunk is even), so
+// one test of `tally` picks the 16-byte or the scalar loop for the whole grid.
 __global__ void __launch_bounds__(256)
 k_gather_owned(const GroupView g, double* __restrict__ tally, unsigned long long epoch) {
   SyncBlock* mine = g.sync[g.rank];
   const size_t stride = (size_t)gridDim.x * blockDim.x;
+  const bool vec = ((uintptr_t)tally & 15) == 0;
   for (int d = 0; d < g.nranks; ++d) {
     const size_t begin = (size_t)d * g.chunk;
     if (begin >= g.ncells) break;
     const size_t end = begin + g.chunk < g.ncells ? begin + g.chunk : g.ncells;
     const size_t count = end - begin;
+    if (!vec) {
+      for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += stride)
+        tally[begin + i] += __ldcv(g.src[d] + i);
+      continue;
+    }
     const size_t pairs = count >> 1;
     double2* t2 = reinterpret_cast<double2*>(tally + begin);
     const double2* s2 = reinterpret_cast<const double2*>(g.src[d]);

@@ -316,9 +316,16 @@ __global__ void k_selftest_cs(const double* keys, const double* vals, int n_entr
   out[i] = v_staged;
 }
 
-// dst += src over the tally mesh (combining per-step tally deltas of a sharded run).
+// dst += src over the tally mesh (combining per-step tally deltas of a sharded run). 16-byte
+// accesses when both pointers allow them, a scalar loop when either is only 8-byte aligned.
 __global__ void k_accumulate(double* __restrict__ dst, const double* __restrict__ src,
                              size_t n) {
+  if ((((uintptr_t)dst | (uintptr_t)src) & 15) != 0) {
+    const size_t stride = (size_t)gridDim.x * blockDim.x;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
+      dst[i] += src[i];
+    return;
+  }
   size_t i = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) * 2;
   const size_t stride = (size_t)gridDim.x * blockDim.x * 2;
   for (; i + 1 < n; i += stride) {
@@ -334,6 +341,14 @@ __global__ void k_accumulate(double* __restrict__ dst, const double* __restrict_
 // dst += src; src = 0: folds a reduced per-step delta into the cumulative tally and leaves the
 // delta buffer ready for its next timestep in the same pass.
 __global__ void k_accumulate_clear(double* __restrict__ dst, double* __restrict__ src, size_t n) {
+  if ((((uintptr_t)dst | (uintptr_t)src) & 15) != 0) {
+    const size_t stride = (size_t)gridDim.x * blockDim.x;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+      dst[i] += src[i];
+      src[i] = 0.0;
+    }
+    return;
+  }
   size_t i = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) * 2;
   const size_t stride = (size_t)gridDim.x * blockDim.x * 2;
   for (; i + 1 < n; i += stride) {
