@@ -426,6 +426,34 @@ int nb200_bank_flux_batches(nb200_particle_soa* particles, double* out_device, s
 int nb200_bank_flux_relerr(nb200_particle_soa* particles, double* relerr_device,
                            double* total_relerr_host);
 
+/* ------------------------------------------------------------------------------------
+ * 9. Energy-group flux: the track-length flux of section 7 split into caller-given energy
+ *    groups. The caller gives G + 1 edges E_0 < E_1 < ... < E_G in eV (the unit of the deck's
+ *    initial_energy), 1 <= G <= 256, and a device array of G * ncells doubles, group-major.
+ *    Every flight segment of every later timestep adds w * l / ntotal_particles to
+ *    flux[g * ncells + celly * nx + cellx], g the group with E_g <= e < E_{g+1}, e the energy
+ *    the particle flies with along the segment; w and l are those of section 7. A segment whose
+ *    energy is outside [E_0, E_G) is not scored. Histories, counts, the bank and the energy
+ *    tally do not change. The edges are copied into a device buffer the library owns.
+ *    A bank has at most one flux attachment: this call replaces a plain flux (section 7), and
+ *    nb200_bank_set_flux_tally replaces a group flux. A null array, in either call, detaches
+ *    whichever is attached. deallocate_data of the attached array detaches it;
+ *    nb200_bank_free drops the attachment; nb200_bank_copy copies particles only.
+ *    Refused with an error code (-4: timesteps of the bank pending; -3 otherwise): G < 1 or
+ *    G > 256, edges that are not finite and strictly increasing (these two are checked on the
+ *    host before anything else), a handle that is not a bank, a bank with tally batches, a bank
+ *    sharded over several GPUs or in a multi-process group, pipeline = 0 or tally_prereduce = 1
+ *    (the bank's effective options), an array that is not device memory on the bank's GPU,
+ *    ncells = 0, G * ncells >= 2^31. nb200_bank_set_option and solve_transport_2d refuse as
+ *    in section 7.
+ * ---------------------------------------------------------------------------------- */
+/* Attaches flux_device (ngroups * ncells doubles, device memory on the bank's GPU) as a group
+ * flux over the ngroups + 1 energy edges at edges_host, or detaches the current flux array when
+ * flux_device is null (edges_host and ngroups are then ignored). Returns 0, -4 when timesteps of
+ * the bank are pending, or another negative code (nb200_last_error). */
+int nb200_bank_set_group_flux_tally(nb200_particle_soa* particles, double* flux_device,
+                                    size_t ncells, const double* edges_host, int ngroups);
+
 /* What the history kernel is bound by on facet-dominated decks, measured in place: FP64
  * reductions per second the L2 retires (csrc/microbench.cu; pattern 3 = the peak, 1 = a
  * particle's mesh walk, 0 = random cells, 5 / 6 = 32 / 4 lanes on consecutive cells) into a

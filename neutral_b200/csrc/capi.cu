@@ -14,6 +14,7 @@
 #include <time.h>
 
 #include <algorithm>
+#include <cmath>
 #include <string>
 #include <unordered_set>
 #include <vector>
@@ -80,6 +81,7 @@ int g_shard_first = 0, g_shard_count = -1;  // nb200_set_shard
 std::unordered_set<const void*> g_handles;  // every live bank handle (what `Particle*` may be)
 std::vector<Bank*> g_batched;          // every live bank with tally batches
 std::vector<Bank*> g_flux;             // every live bank with a flux array attached
+constexpr int kMaxFluxGroups = 256;    // energy groups of a group flux (nb200_bank_set_group_flux_tally)
 
 // What `validate` reports besides the reference's printed lines (SURVEY.md 8f 1).
 struct StepLog {
@@ -568,13 +570,38 @@ Bank* batched_bank_of_tally(const double* tally) {
 // `flux` null detaches. The attachment is the bank's own: nb200_bank_copy does not move it.
 // A batched flux of the old attachment is flushed into the old array and its slab freed first.
 // B > 0 attaches a batched flux: deposits go to a zeroed slab of B partial fluxes on the bank's
-// GPU, allocated here. Returns 0, or -2 (error set) when the slab cannot be had.
-int flux_attach(Bank* bank, double* flux, size_t ncells, int B = 0) {
+// GPU, allocated here. G > 0 attaches a group flux (G * ncells doubles) whose G + 1 edges are
+// copied from `edges` (host memory) into a device buffer of the bank. Returns 0, or -2 (error
+// set) when the slab or the edge buffer cannot be had.
+int flux_attach(Bank* bank, double* flux, size_t ncells, int B = 0, const double* edges = nullptr,
+                int G = 0) {
   batches_release(bank, bank->flux_batches);
   g_flux.erase(std::remove(g_flux.begin(), g_flux.end(), bank), g_flux.end());
   bank->flux = nullptr;
   bank->flux_ncells = 0;
+  if (bank->flux_edges) {
+    DeviceGuard guard(bank->shards[0].dev);
+    cudaFree(bank->flux_edges);  // synchronises: no timestep still reads them
+    bank->flux_edges = nullptr;
+  }
+  bank->flux_groups = 0;
   if (!flux) return 0;
+  if (G > 0) {
+    DeviceGuard guard(bank->shards[0].dev);
+    DeviceCtx& c = ctx_on(bank->shards[0].dev);
+    const size_t bytes = sizeof(double) * (size_t)(G + 1);
+    double* d_edges = nullptr;
+    CU_TRY(cudaMalloc(&d_edges, bytes));
+    cudaError_t err = cudaMemcpyAsync(d_edges, edges, bytes, cudaMemcpyHostToDevice, c.stream);
+    if (err == cudaSuccess) err = cudaStreamSynchronize(c.stream);
+    if (err != cudaSuccess) {
+      cudaFree(d_edges);
+      set_error("copying the energy edges to the device failed: %s", cudaGetErrorString(err));
+      return -2;
+    }
+    bank->flux_edges = d_edges;
+    bank->flux_groups = G;
+  }
   if (B > 0) {
     DeviceGuard guard(bank->shards[0].dev);
     DeviceCtx& c = ctx_on(bank->shards[0].dev);
@@ -878,6 +905,7 @@ struct ShardIO {
   uint64_t *r0, *r1, *r2;
   BatchArgs batches;
   double* flux;  // track-length flux array, or null
+  GroupArgs groups;  // its energy groups (ngroups > 0: `flux` is a group flux)
 };
 
 // An event the host will wait on or read a time from. While a timestep is being recorded into
@@ -1004,7 +1032,7 @@ void record_shard_step(DeviceCtx& c, const Bank* bank, Shard& sh, const StepRequ
     a.stagger_share = opt_of(bank, &Options::stagger_share);
     a.stagger_min = opt_of(bank, &Options::stagger_min);
     const bool fast_div = opt_of(bank, &Options::fast_div) != 0;
-    c.launches += launch_history(a, io.batches, io.flux, c.d_n_live, s.n_upper, fast_div,
+    c.launches += launch_history(a, io.batches, io.flux, io.groups, c.d_n_live, s.n_upper, fast_div,
                                  opt_of(bank, &Options::tally_prereduce) != 0,
                                  opt_l2 == 2 ? (const void*)io.tally
                                  : opt_l2    ? (const void*)c.d_cs_stage : nullptr,
@@ -1485,6 +1513,7 @@ void enqueue_step(Bank* bank, const StepRequest& rq) {
     io.tally = rq.tally;
     io.batches = BatchArgs{bank->batches.slab, bank->batches.B, bank->n};
     io.flux = bank->flux_batches.B > 0 ? bank->flux_batches.slab : bank->flux;
+    io.groups = GroupArgs{bank->flux_edges, bank->flux_groups};
     // per-particle counters live on the primary GPU, indexed in injection order: a secondary
     // shard reaches its part of them through peer access (one 8-byte update per particle-step)
     const bool counters_ok = sh.dev == pd || (group && group->collective);
@@ -2677,6 +2706,49 @@ extern "C" int nb200_bank_set_batched_flux_tally(nb200_particle_soa* particles,
   if (!flux_device) return flux_attach(bank, nullptr, 0);
   if (int rc = refuse_flux_array(bank, flux_device, ncells, true, who)) return rc;
   return flux_attach(bank, flux_device, ncells, bank->batches.B);
+}
+
+// Why `edges` (G + 1 host doubles) cannot be a group flux's energy edges, as -3 with the message
+// set; 0 if they can. Host arguments only: checked before anything needs a device.
+static int refuse_group_edges(const double* edges, int ngroups, const char* who) {
+  if (ngroups < 1 || ngroups > kMaxFluxGroups) {
+    set_error("%s: ngroups = %d (1 .. %d)", who, ngroups, kMaxFluxGroups);
+    return -3;
+  }
+  if (!edges) {
+    set_error("%s: no energy edges", who);
+    return -3;
+  }
+  for (int g = 0; g <= ngroups; ++g) {
+    if (!std::isfinite(edges[g]) || (g > 0 && !(edges[g] > edges[g - 1]))) {
+      set_error("%s: the energy edges must be finite and strictly increasing (edge %d is %.17g)",
+                who, g, edges[g]);
+      return -3;
+    }
+  }
+  return 0;
+}
+
+extern "C" int nb200_bank_set_group_flux_tally(nb200_particle_soa* particles, double* flux_device,
+                                               size_t ncells, const double* edges_host,
+                                               int ngroups) {
+  const char* who = "nb200_bank_set_group_flux_tally";
+  if (flux_device)
+    if (int rc = refuse_group_edges(edges_host, ngroups, who)) return rc;
+  Bank* bank = bank_of(particles);
+  if (!bank) {
+    set_error("%s: not a bank handle", who);
+    return -3;
+  }
+  if (int rc = refuse_if_pending(bank, who)) return rc;
+  if (!flux_device) return flux_attach(bank, nullptr, 0);
+  if (int rc = refuse_flux_array(bank, flux_device, ncells, false, who)) return rc;
+  if ((unsigned long long)ncells * (unsigned long long)ngroups >= (1ull << 31)) {
+    set_error("%s: %d groups over %zu cells need 2^31 or more flux slots (the history kernel "
+              "indexes them with 32 bits)", who, ngroups, ncells);
+    return -3;
+  }
+  return flux_attach(bank, flux_device, ncells, 0, edges_host, ngroups);
 }
 
 // The bank's flux batches, flushed into the attached array; nullptr (error set) if there are none.

@@ -230,6 +230,10 @@ struct Bank {
   // nb200_bank_set_batched_flux_tally: B > 0 (the B of `batches`) when the flux deposits go to
   // B partial fluxes instead; their target is `flux`, their slab is allocated when it attaches.
   TallyBatches flux_batches;
+  // nb200_bank_set_group_flux_tally: G > 0 when `flux` holds G energy groups of flux_ncells
+  // cells each (group-major); the G + 1 edges are in flux_edges, device memory the bank owns.
+  double* flux_edges = nullptr;
+  int flux_groups = 0;
   int n = 0;
   uint64_t pid0 = 0;
   int primary_dev = 0;

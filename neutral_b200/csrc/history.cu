@@ -31,7 +31,7 @@
 // Compiled with -fmad=false: the only fused operations are the explicit fma() of nb_log,
 // div_by_known and the cores.
 #include <type_traits>
-#ifdef NB_ASSERT_BATCH_SLOT
+#if defined(NB_ASSERT_BATCH_SLOT) || defined(NB_ASSERT_GROUP_SLOT)
 #include <cassert>
 #endif
 
@@ -161,23 +161,74 @@ struct ParkedBatchedFlux : ParkedBatched {
   double flux[kHistoryThreads];
 };
 
+// kGroups with kFlux (nb200_bank_set_group_flux_tally): `flux` is G group-major arrays of the
+// mesh, and a segment goes to the group of the energy it flies with. The group is a property of
+// the flight: found by bisection at the start of the history and after every scatter, and
+// parked beside the flux. -1 (an energy outside the edges) deposits nothing.
+struct ParkedGroupFlux : ParkedFlux {
+  int group[kHistoryThreads];
+};
+
+template <bool kGroups, class P>
+__device__ __forceinline__ int parked_group(const P& park) {
+  if constexpr (kGroups) return park.group[threadIdx.x];
+  else return 0;
+}
+
+template <bool kGroups, class P>
+__device__ __forceinline__ void park_group(P& park, int g) {
+  if constexpr (kGroups) park.group[threadIdx.x] = g;
+}
+
+// g with edges[g] <= e < edges[g + 1], or -1 when e is outside [edges[0], edges[G]) (or NaN).
+// The G + 1 <= 257 edges are read through the read-only path and stay in L1.
+__device__ __forceinline__ int energy_group(const GroupArgs& gr, double e) {
+  if (!(e >= __ldg(gr.edges) && e < __ldg(gr.edges + gr.ngroups))) return -1;
+  int lo = 0, hi = gr.ngroups;  // edges[lo] <= e < edges[hi]
+  while (hi - lo > 1) {
+    const int mid = (lo + hi) >> 1;
+    if (__ldg(gr.edges + mid) <= e) lo = mid;
+    else hi = mid;
+  }
+  return lo;
+}
+
+// Index of `cell` of group g in the flux array (32 bits: the host refuses G * ncells >= 2^31).
+__device__ __forceinline__ int group_index(const StepArgs& a, const GroupArgs& gr, int g,
+                                           int cell) {
+  const int ncells = a.nx * a.ny;
+  const int i = g * ncells + cell;
+#ifdef NB_ASSERT_GROUP_SLOT  // checking build: NB200_DEFINES=-DNB_ASSERT_GROUP_SLOT
+  assert(g >= 0 && g < gr.ngroups && cell >= 0 && cell < ncells && i >= 0 &&
+         i < gr.ngroups * ncells);
+#endif
+  return i;
+}
+
 // `flux` is a kernel parameter behind the other three for the reason BatchArgs is one: a field
-// appended to StepArgs would move the offsets of the parameters that follow it.
-template <bool kFastDiv, bool kPreReduce, bool kBatched, bool kFlux>
+// appended to StepArgs would move the offsets of the parameters that follow it; `grp` follows
+// `flux` for the same reason.
+template <bool kFastDiv, bool kPreReduce, bool kBatched, bool kFlux, bool kGroups = false>
 __global__ void NB_HISTORY_BOUNDS
 k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs bt,
-          double* __restrict__ flux) {
+          double* __restrict__ flux, const GroupArgs grp) {
 #if NB_PARK_SMEM
-  __shared__ std::conditional_t<kBatched, std::conditional_t<kFlux, ParkedBatchedFlux, ParkedBatched>,
-                                std::conditional_t<kFlux, ParkedFlux, Parked>> park;
+  __shared__ std::conditional_t<
+      kBatched, std::conditional_t<kFlux, ParkedBatchedFlux, ParkedBatched>,
+      std::conditional_t<kFlux, std::conditional_t<kGroups, ParkedGroupFlux, ParkedFlux>, Parked>>
+      park;
 #define PARKED(name) park.name[threadIdx.x]
 #define PARKED_BATCH parked_batch<kBatched>(park)
+#define PARKED_GROUP parked_group<kGroups>(park)
+#define PARK_GROUP(g) park_group<kGroups>(park, (g))
 #else
   double park_e, park_Sig_s, park_p_absorb, park_rho, park_edep, park_flux;
-  int park_origin, park_slot, park_batch = 0;
+  int park_origin, park_slot, park_batch = 0, park_group = 0;
   unsigned park_nc;
 #define PARKED(name) park_##name
 #define PARKED_BATCH park_batch
+#define PARKED_GROUP park_group
+#define PARK_GROUP(g) (park_group = (g))
 #endif
   const unsigned live = n_live[0];
   unsigned nf = 0, census = 0, processed = 0, died = 0;
@@ -207,12 +258,21 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs
     // the base and index a deposit into `cell` goes to: the caller's tally, or the batch's slot
 #define NB_TALLY_AT(cell) \
   (kBatched ? bt.slab : a.tally), (kBatched ? batch_index(a, bt, PARKED_BATCH, (cell)) : (cell))
-    // ... and a flux deposit: the caller's array, or (batched) the batch's slot of the flux slab
-#define NB_FLUX_AT(cell) flux, (kBatched ? batch_index(a, bt, PARKED_BATCH, (cell)) : (cell))
+    // ... and a flux deposit: the caller's array (the group's slice of it for a group flux), or
+    // (batched) the batch's slot of the flux slab
+#define NB_FLUX_AT(cell)                                      \
+  flux, (kBatched  ? batch_index(a, bt, PARKED_BATCH, (cell)) \
+         : kGroups ? group_index(a, grp, PARKED_GROUP, (cell)) : (cell))
+    // ... through this, which makes no deposit while the particle is outside the energy groups
+#define NB_FLUX_ADD(cell, value)                                                    \
+  do {                                                                              \
+    if (!kGroups || PARKED_GROUP >= 0) tally_add<false>(NB_FLUX_AT(cell), (value)); \
+  } while (0)
     unsigned flags = same_grid(a) ? kFlagSameGrid : 0u;
     PARKED(e) = ew.x;
     PARKED(edep) = 0.0;
     if constexpr (kFlux) PARKED(flux) = 0.0;
+    if constexpr (kGroups) PARK_GROUP(energy_group(grp, ew.x));
     PARKED(origin) = m.w;
     if constexpr (kBatched) {
       const int b = (int)batch_of((unsigned)(a.pid0 + (uint64_t)(unsigned)m.w), (unsigned)bt.n,
@@ -298,7 +358,7 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs
             tally_add<kPreReduce>(NB_TALLY_AT(NB_CELL), PARKED(edep) * a.inv_ntotal);
             PARKED(edep) = 0.0;
             if constexpr (kFlux) {
-              tally_add<false>(NB_FLUX_AT(NB_CELL), PARKED(flux) * a.inv_ntotal);
+              NB_FLUX_ADD(NB_CELL, PARKED(flux) * a.inv_ntotal);
               PARKED(flux) = 0.0;
             }
             flags &= ~kFlagPending;
@@ -328,7 +388,7 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs
         // :321-327 - deposit, flush to the tally (update_tallies, :408-420), reset
         const double edep = deposition(w, d_facet, d.stb, d.heat, nd);
         tally_add<kPreReduce>(NB_TALLY_AT(NB_CELL), edep * a.inv_ntotal);
-        if constexpr (kFlux) tally_add<false>(NB_FLUX_AT(NB_CELL), (w * d_facet) * a.inv_ntotal);
+        if constexpr (kFlux) NB_FLUX_ADD(NB_CELL, (w * d_facet) * a.inv_ntotal);
         x += d_facet * ox;
         y += d_facet * oy;
         // the edge load is consumed here, after the arithmetic it overlapped with
@@ -412,7 +472,7 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs
           if (e < kMinEnergyOfInterest) {  // :243-252 - the history ends here
             flags |= kFlagDead;
             tally_add<kPreReduce>(NB_TALLY_AT(NB_CELL), edep * a.inv_ntotal);
-            if constexpr (kFlux) tally_add<false>(NB_FLUX_AT(NB_CELL), PARKED(flux) * a.inv_ntotal);
+            if constexpr (kFlux) NB_FLUX_ADD(NB_CELL, PARKED(flux) * a.inv_ntotal);
             break;
           }
           // Energy and direction are unchanged: the lookups of :285-291 return the values
@@ -463,6 +523,17 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs
             ey = target_edge(a.edgey, cy, axis_step(oy));
             mfp = neglog / PARKED(Sig_s);
           }
+          if constexpr (kGroups) {
+            // PARKED(e) holds the new energy. The parked flux (this collision's segment and
+            // those of the collisions before it in this cell) flew at the old one: into the
+            // old group with it, before the new group is parked.
+            const int g = energy_group(grp, PARKED(e));
+            if (g != PARKED_GROUP) {
+              NB_FLUX_ADD(NB_CELL, PARKED(flux) * a.inv_ntotal);
+              PARKED(flux) = 0.0;
+              PARK_GROUP(g);
+            }
+          }
         }
         PARKED(edep) = edep;
         flags |= kFlagPending;
@@ -479,7 +550,7 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs
         if constexpr (kFlux) {
           double fl = w * d_census;
           if (flags & kFlagPending) fl = PARKED(flux) + fl;
-          tally_add<false>(NB_FLUX_AT(NB_CELL), fl * a.inv_ntotal);
+          NB_FLUX_ADD(NB_CELL, fl * a.inv_ntotal);
         }
         dtc = 0.0;
         break;
@@ -514,7 +585,10 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs
 #undef NB_CELL
 #undef NB_TALLY_AT
 #undef NB_FLUX_AT
+#undef NB_FLUX_ADD
 #undef PARKED_BATCH
+#undef PARKED_GROUP
+#undef PARK_GROUP
 }
 
 static inline int blocks_for(int n, int threads) { return (n + threads - 1) / threads; }
@@ -522,7 +596,8 @@ static inline int blocks_for(int n, int threads) { return (n + threads - 1) / th
 // `pin`/`pin_bytes` (optional) name the staged cross-section block: the launch then carries an
 // access-policy window that keeps it persisting in L2 (north_star phase 3), while the rest of
 // the kernel's traffic - the tally atomics above all - streams through the remainder.
-int launch_history(const StepArgs& a, const BatchArgs& bt, double* flux, const unsigned* n_live,
+int launch_history(const StepArgs& a, const BatchArgs& bt, double* flux, const GroupArgs& grp,
+                   const unsigned* n_live,
                    int n_upper, bool fast_div, bool prereduce, const void* pin, size_t pin_bytes, size_t pin_budget,
                    int smem_pad, cudaStream_t st) {
   if (n_upper <= 0) return 0;
@@ -544,6 +619,8 @@ int launch_history(const StepArgs& a, const BatchArgs& bt, double* flux, const u
       cudaFuncSetAttribute(k_history<false, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
       cudaFuncSetAttribute(k_history<true, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
       cudaFuncSetAttribute(k_history<false, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
+      cudaFuncSetAttribute(k_history<true, false, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
+      cudaFuncSetAttribute(k_history<false, false, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
       granted = smem_pad;
     }
     cfg.dynamicSmemBytes = (size_t)smem_pad;
@@ -566,28 +643,34 @@ int launch_history(const StepArgs& a, const BatchArgs& bt, double* flux, const u
   // and without batches alternating on one device change the graph's kernel and re-instantiate
   // it instead, which is correct and costs an instantiation per switch. A bank with a flux
   // array attached is the same: the host refuses prereduce for it, and a batched bank's flux is
-  // always batched (its `flux` is the flux batch slab).
-  if (flux && bt.nbatches > 0) {
+  // always batched (its `flux` is the flux batch slab). A group flux is neither batched nor
+  // prereduced (the host refuses both), and its kernel is one more switch of the same kind.
+  if (flux && grp.ngroups > 0) {
     if (fast_div)
-      cudaLaunchKernelEx(&cfg, k_history<true, false, true, true>, a, n_live, bt, flux);
+      cudaLaunchKernelEx(&cfg, k_history<true, false, false, true, true>, a, n_live, bt, flux, grp);
     else
-      cudaLaunchKernelEx(&cfg, k_history<false, false, true, true>, a, n_live, bt, flux);
+      cudaLaunchKernelEx(&cfg, k_history<false, false, false, true, true>, a, n_live, bt, flux, grp);
+  } else if (flux && bt.nbatches > 0) {
+    if (fast_div)
+      cudaLaunchKernelEx(&cfg, k_history<true, false, true, true>, a, n_live, bt, flux, grp);
+    else
+      cudaLaunchKernelEx(&cfg, k_history<false, false, true, true>, a, n_live, bt, flux, grp);
   } else if (flux) {
     if (fast_div)
-      cudaLaunchKernelEx(&cfg, k_history<true, false, false, true>, a, n_live, bt, flux);
+      cudaLaunchKernelEx(&cfg, k_history<true, false, false, true>, a, n_live, bt, flux, grp);
     else
-      cudaLaunchKernelEx(&cfg, k_history<false, false, false, true>, a, n_live, bt, flux);
+      cudaLaunchKernelEx(&cfg, k_history<false, false, false, true>, a, n_live, bt, flux, grp);
   } else if (bt.nbatches > 0) {
     if (fast_div)
-      cudaLaunchKernelEx(&cfg, k_history<true, false, true, false>, a, n_live, bt, flux);
+      cudaLaunchKernelEx(&cfg, k_history<true, false, true, false>, a, n_live, bt, flux, grp);
     else
-      cudaLaunchKernelEx(&cfg, k_history<false, false, true, false>, a, n_live, bt, flux);
+      cudaLaunchKernelEx(&cfg, k_history<false, false, true, false>, a, n_live, bt, flux, grp);
   } else if (prereduce) {
-    cudaLaunchKernelEx(&cfg, k_history<true, true, false, false>, a, n_live, bt, flux);
+    cudaLaunchKernelEx(&cfg, k_history<true, true, false, false>, a, n_live, bt, flux, grp);
   } else if (fast_div) {
-    cudaLaunchKernelEx(&cfg, k_history<true, false, false, false>, a, n_live, bt, flux);
+    cudaLaunchKernelEx(&cfg, k_history<true, false, false, false>, a, n_live, bt, flux, grp);
   } else {
-    cudaLaunchKernelEx(&cfg, k_history<false, false, false, false>, a, n_live, bt, flux);
+    cudaLaunchKernelEx(&cfg, k_history<false, false, false, false>, a, n_live, bt, flux, grp);
   }
   return 1;
 }

@@ -145,6 +145,15 @@ struct BatchArgs {
   int n;
 };
 
+// nb200_bank_set_group_flux_tally: with ngroups = G > 0 the flux deposits go to
+// flux[g * ncells + cell], g the energy group with edges[g] <= e < edges[g + 1] (G + 1 edges in
+// device memory); none outside [edges[0], edges[G]). A kernel parameter of its own behind the
+// flux array, for the reason BatchArgs is one.
+struct GroupArgs {
+  const double* edges;
+  int ngroups;
+};
+
 // Layout of the B partial tallies in the batch slab: batch-major [b][cell] (0) or cell-major
 // [cell][b] (1). Both were built and measured (DESIGN.md 9); the product keeps batch-major.
 // -DNB_TALLY_BATCH_CELL_MAJOR=1 builds the other one for tools/tally_batches_cost.py.

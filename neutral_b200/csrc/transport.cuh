@@ -20,8 +20,10 @@ int launch_history_direct(const StepArgs& a, cudaStream_t st);
 int launch_sort_phase(const StepArgs& a, const SortArgs& s, const BankView& alt,
                       cudaStream_t st);
 // bt.nbatches > 0 runs the batched variant (option tally_batches); a non-null `flux` the
-// variant that also deposits the track-length flux there (nb200_bank_set_flux_tally).
-int launch_history(const StepArgs& a, const BatchArgs& bt, double* flux, const unsigned* n_live,
+// variant that also deposits the track-length flux there (nb200_bank_set_flux_tally), and with
+// grp.ngroups > 0 into the flux's energy groups (nb200_bank_set_group_flux_tally).
+int launch_history(const StepArgs& a, const BatchArgs& bt, double* flux, const GroupArgs& grp,
+                   const unsigned* n_live,
                    int n_upper, bool fast_div, bool prereduce, const void* pin, size_t pin_bytes,
                    size_t pin_budget, int smem_pad, cudaStream_t st);
 // Batch partial tallies (tally_batches.cu). The slab holds the B partial tallies S_b in the

@@ -57,7 +57,7 @@ EXPORTED_SYMBOLS = [
     "nb200_mp_connect", "nb200_mp_finalize", "nb200_tally_sync", "nb200_update_replicas",
     "nb200_microbench_red", "nb200_bank_tally_batches", "nb200_bank_tally_relerr",
     "nb200_selftest_batch_of", "nb200_bank_set_flux_tally", "nb200_bank_set_batched_flux_tally",
-    "nb200_bank_flux_batches", "nb200_bank_flux_relerr",
+    "nb200_bank_flux_batches", "nb200_bank_flux_relerr", "nb200_bank_set_group_flux_tally",
 ]
 
 #: include/neutral_b200.h
@@ -141,6 +141,8 @@ def load_library(build: bool = False) -> C.CDLL:
     L.nb200_bank_set_batched_flux_tally.argtypes = [_soa_p, C.c_void_p, C.c_size_t]
     L.nb200_bank_flux_batches.argtypes = [_soa_p, C.c_void_p, C.c_size_t]
     L.nb200_bank_flux_relerr.argtypes = [_soa_p, C.c_void_p, _dp]
+    L.nb200_bank_set_group_flux_tally.argtypes = [_soa_p, C.c_void_p, C.c_size_t, C.c_void_p,
+                                                  C.c_int]
     L.nb200_last_step_stats.argtypes = [_u64p]
     L.nb200_solve_finish.argtypes = [_u64p, _u64p]
     L.nb200_kernel_launches.restype = C.c_uint64
@@ -247,8 +249,18 @@ class Simulation:
 
     def __init__(self, problem: Problem, rank: int = 0, nranks: int = 1,
                  per_particle_counters: bool = True, quiet: bool = True, ngpus: int = 1,
-                 tally_batches: int = 0, flux_tally: bool = False):
+                 tally_batches: int = 0, flux_tally: bool = False, flux_groups=None):
         self.lib = load_library()
+        #: energy edges of the group flux (nb200_bank_set_group_flux_tally), or None
+        self.flux_edges = None
+        if flux_groups is not None:
+            if flux_tally or tally_batches:
+                raise NeutralB200Error("flux_groups cannot be combined with flux_tally or "
+                                       "tally_batches (a bank has one flux, and a group flux "
+                                       "has no batches)")
+            self.flux_edges = np.array(flux_groups, dtype=np.float64)
+            if self.flux_edges.ndim != 1 or self.flux_edges.size < 2:
+                raise NeutralB200Error("flux_groups: G + 1 >= 2 energy edges in eV, increasing")
         require_device()
         self.problem = problem
         d = problem.deck
@@ -276,6 +288,10 @@ class Simulation:
         #: bank this simulation creates; see :meth:`scalar_flux`. With ``tally_batches`` it is
         #: batched too (nb200_bank_set_batched_flux_tally), see :meth:`flux_relative_error`
         self.flux = DeviceArray(d.nx * d.ny, np.float64) if flux_tally else None
+        if self.flux_edges is not None:
+            #: with ``flux_groups``: the group flux, G arrays of the mesh (group-major), see
+            #: :meth:`group_flux_to_host`
+            self.flux = DeviceArray((self.flux_edges.size - 1) * d.nx * d.ny, np.float64)
         self.counters = [DeviceArray(max(self.count, 1), np.uint64) for _ in range(3)] \
             if per_particle_counters else None
         self.bank = None
@@ -320,7 +336,12 @@ class Simulation:
     def _attach_flux(self) -> None:
         if self.flux is None:
             return
-        if self.tally_batches:
+        if self.flux_edges is not None:
+            ncells = self.problem.deck.nx * self.problem.deck.ny
+            _check(self.lib.nb200_bank_set_group_flux_tally(
+                self.bank, self.flux.ptr, ncells, self.flux_edges.ctypes.data,
+                self.flux_edges.size - 1), "bank_set_group_flux_tally")
+        elif self.tally_batches:
             _check(self.lib.nb200_bank_set_batched_flux_tally(self.bank, self.flux.ptr,
                                                               self.flux.n),
                    "bank_set_batched_flux_tally")
@@ -463,6 +484,19 @@ class Simulation:
         dx = np.diff(self.problem.edgex)
         dy = np.diff(self.problem.edgey)
         return self.flux_to_host() / np.outer(dy, dx)
+
+    def group_flux_to_host(self) -> np.ndarray:
+        """(G, ny, nx) track length per source particle in every cell and energy group
+        ``flux_groups[g] <= e < flux_groups[g + 1]``, summed over timesteps."""
+        d = self.problem.deck
+        return self.flux.download().reshape(self.flux_edges.size - 1, d.ny, d.nx)
+
+    def group_scalar_flux(self) -> np.ndarray:
+        """(G, ny, nx) time-integrated scalar flux per source particle in every energy group:
+        :meth:`group_flux_to_host` divided by the cell areas dx_i dy_j."""
+        dx = np.diff(self.problem.edgex)
+        dy = np.diff(self.problem.edgey)
+        return self.group_flux_to_host() / np.outer(dy, dx)
 
     def flux_batches_to_host(self) -> np.ndarray:
         """(B, ny, nx) cumulative partial fluxes of the B particle batches (``flux_tally=True``

@@ -10,8 +10,14 @@ With --tally-batches B both banks have B tally batches (option tally_batches), a
 the second is batched too (nb200_bank_set_batched_flux_tally): what the flux batches cost on top
 of the energy batches.
 
+With --groups G [G ...] each G adds one more configuration to the alternation: a group flux
+(nb200_bank_set_group_flux_tally) over G logarithmic energy groups from 1e-3 eV to twice the
+deck's initial energy, which cover every energy the deck reaches. Its rows carry the flux summed
+over the groups, and their ratio to the run without flux.
+
     python tools/flux_tally_cost.py --out profiles/r04/flux_tally_cost.json
     python tools/flux_tally_cost.py --tally-batches 16 --out flux_batches_cost_b16.json
+    python tools/flux_tally_cost.py --groups 8 32 --out profiles/r05/group_flux_cost.json
 
 The GPU's name and power limit are written into the same output. Needs a CUDA device.
 """
@@ -43,17 +49,21 @@ def measure(args) -> dict:
     out = {}
     for deck in args.decks:
         prob = build_problem(deck)
+        e0 = prob.deck.initial_energy
         sims = {flux: Simulation(prob, per_particle_counters=False, flux_tally=flux,
                                  tally_batches=args.tally_batches)
                 for flux in (False, True)}
+        for g in args.groups:
+            sims[f"groups_{g}"] = Simulation(prob, per_particle_counters=False,
+                                             flux_groups=np.geomspace(1.0e-3, 2.0 * e0, g + 1))
         for sim in sims.values():
             sim.inject()
         injected = sims[False].bank_to_host()
         st = injected.as_struct()
         snap = _soa_p()
         _check(lib.nb200_bank_create(C.byref(st), len(injected), 0, C.byref(snap)), "snapshot")
-        ms = {False: [], True: []}
-        events = {False: [], True: []}
+        ms = {k: [] for k in sims}
+        events = {k: [] for k in sims}
         for i in range(args.warmup + args.runs):
             for flux, sim in sims.items():
                 _check(lib.nb200_bank_copy(sim.bank, snap), "bank_copy")
@@ -73,12 +83,16 @@ def measure(args) -> dict:
         row = {}
         for flux, sim in sims.items():
             med = statistics.median(ms[flux])
-            row["flux" if flux else "no_flux"] = {
+            name = flux if isinstance(flux, str) else "flux" if flux else "no_flux"
+            row[name] = {
                 "ms_per_deck_run": med, "ms_min": min(ms[flux]), "ms_max": max(ms[flux]),
                 "events_per_s": statistics.median(events[flux]) / (med / 1e3),
                 "runs": len(ms[flux]), "tally_total": float(np.sum(sim.tally_to_host()))}
-            if flux:
-                row["flux"]["flux_total"] = float(np.sum(sim.flux_to_host()))
+            if flux is True:
+                row[name]["flux_total"] = float(np.sum(sim.flux_to_host()))
+            elif flux:
+                row[name]["flux_total"] = float(np.sum(sim.group_flux_to_host()))
+                row[name]["ratio"] = med / statistics.median(ms[False])
         row["ratio"] = row["flux"]["ms_per_deck_run"] / row["no_flux"]["ms_per_deck_run"]
         out[deck] = row
         print(deck, json.dumps(row), flush=True)
@@ -95,12 +109,17 @@ def main():
     ap.add_argument("--warmup", type=int, default=2)
     ap.add_argument("--tally-batches", type=int, default=0,
                     help="B > 0: both banks batched, the flux of the second batched too")
+    ap.add_argument("--groups", type=int, nargs="*", default=[],
+                    help="G ...: one more configuration per G, a group flux over G log groups")
     ap.add_argument("--out", default=None, help="JSON file for the results")
     args = ap.parse_args()
+    if args.groups and args.tally_batches:
+        ap.error("--groups: a group flux has no tally batches")
     result = {"what": "ms per resident deck run (run_pipelined, CUDA events, median) without "
-                      "and with a flux array attached, alternating run by run; events/s",
+                      "and with a flux array attached (plain, and a group flux per --groups G), "
+                      "alternating run by run; events/s",
               **gpu_identity(), "runs": args.runs, "warmup": args.warmup,
-              "tally_batches": args.tally_batches,
+              "tally_batches": args.tally_batches, "groups": args.groups,
               "decks": measure(args)}
     text = json.dumps(result, indent=1)
     print(text)
