@@ -454,6 +454,49 @@ int nb200_bank_flux_relerr(nb200_particle_soa* particles, double* relerr_device,
 int nb200_bank_set_group_flux_tally(nb200_particle_soa* particles, double* flux_device,
                                     size_t ncells, const double* edges_host, int ngroups);
 
+/* ------------------------------------------------------------------------------------
+ * 10. Group flux batches: a relative error beside every group of every flux cell, and of
+ *    every group's total over the mesh (the error bar of the spectrum). A bank with tally
+ *    batches (section 6) can have a group flux (section 9) attached through the call below:
+ *    G * ncells doubles, group-major, over G + 1 edges as in section 9. Its group-flux
+ *    deposits then go to B partial group fluxes, one per particle batch of section 6, held by
+ *    the library ((B + 1) * G * ncells doubles on the bank's GPU, allocated and zeroed when the
+ *    array is attached). The attached array receives what the batches gained lazily, wherever
+ *    a batched flux of section 8 does. The estimator is section 6's, on the group flux batches.
+ *    Histories, counts, the bank and the energy tally and its batches do not change.
+ *    A bank has at most one flux attachment: each of the four attach calls (sections 7 to 10)
+ *    replaces whatever is attached, after flushing a batched one into its old array; a null
+ *    array detaches the same way. deallocate_data of the attached array detaches it without a
+ *    flush. nb200_bank_flux_batches and nb200_bank_flux_relerr refuse a batched group flux,
+ *    and nb200_bank_set_group_flux_tally still refuses a bank with tally batches.
+ *    Refused with an error code (-4: timesteps of the bank pending; -3 otherwise): G < 1 or
+ *    G > 256, edges that are not finite and strictly increasing (these two are checked on the
+ *    host before anything else), a handle that is not a bank, a bank without tally batches, a
+ *    bank sharded over several GPUs or in a multi-process group, pipeline = 0 or
+ *    tally_prereduce = 1 (the bank's effective options), an array that is not device memory on
+ *    the bank's GPU, ncells = 0, B * G * ncells >= 2^31. nb200_bank_set_option and
+ *    solve_transport_2d refuse as in section 7.
+ * ---------------------------------------------------------------------------------- */
+/* Attaches flux_device (ngroups * ncells doubles, device memory on the bank's GPU) as a batched
+ * group flux over the ngroups + 1 energy edges at edges_host, with the bank's B, or detaches the
+ * current flux array when flux_device is null (edges_host and ngroups are then ignored).
+ * Returns 0, -4 when timesteps of the bank are pending, or another negative code
+ * (nb200_last_error). */
+int nb200_bank_set_batched_group_flux_tally(nb200_particle_soa* particles, double* flux_device,
+                                            size_t ncells, const double* edges_host, int ngroups);
+/* Flushes, then writes the B cumulative partial group fluxes batch-major to device memory:
+ * out[(b * ngroups + g) * ncells + cell]. Returns B, or a negative code: no batched group flux
+ * attached, no timestep deposited into it yet, ncells or ngroups not the attached array's. */
+int nb200_bank_group_flux_batches(nb200_particle_soa* particles, double* out_device,
+                                  size_t ncells, int ngroups);
+/* Flushes, then writes R of every group of every cell to relerr_device (ngroups * ncells
+ * doubles, group-major, device memory), R of every group's total over the mesh to
+ * group_relerr_host (ngroups doubles) and R of the grand total to *total_relerr_host. Each may
+ * be null. Returns 0 or a negative code: no batched group flux attached, no timestep deposited
+ * into it yet. */
+int nb200_bank_group_flux_relerr(nb200_particle_soa* particles, double* relerr_device,
+                                 double* group_relerr_host, double* total_relerr_host);
+
 /* What the history kernel is bound by on facet-dominated decks, measured in place: FP64
  * reductions per second the L2 retires (csrc/microbench.cu; pattern 3 = the peak, 1 = a
  * particle's mesh walk, 0 = random cells, 5 / 6 = 32 / 4 lanes on consecutive cells) into a

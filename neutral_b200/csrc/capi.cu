@@ -529,35 +529,53 @@ void batches_bind(Bank* bank, const StepRequest& rq) {
   tb.target = rq.tally;
 }
 
+// R over the B batch totals t_b of one quantity: x_b = t_b * N / n_b, in batch order.
+static double batch_totals_relerr(const Bank* bank, const std::vector<double>& t) {
+  const int B = (int)t.size();
+  std::vector<double> x(B);
+  double sum = 0.0;
+  for (int b = 0; b < B; ++b) {
+    const int nb = bank->n / B + (b < bank->n % B ? 1 : 0);
+    x[b] = t[b] * (double)bank->n / (double)nb;
+    sum += x[b];
+  }
+  const double m = sum / (double)B;
+  double ss = 0.0;
+  for (int b = 0; b < B; ++b) ss += (x[b] - m) * (x[b] - m);
+  const double var = ss / (double)(B - 1);
+  return m == 0.0 ? 0.0 : sqrt(var / (double)B) / fabs(m);
+}
+
 // R of the total of `tb` (tally or flux): the B batch totals through a fixed-order device
-// reduction, then the estimator in FP64 on the host.
-double batches_total_relerr(Bank* bank, const TallyBatches& tb) {
+// reduction, then the estimator in FP64 on the host. With G > 1 the cells of every batch are G
+// equal, consecutive segments (the groups of a batched group flux): `group_relerr` (G doubles,
+// optional) gets R of every segment's total, and a batch's total is the sum of its G segment
+// totals in group order.
+double batches_total_relerr(Bank* bank, const TallyBatches& tb, int G = 1,
+                            double* group_relerr = nullptr) {
   const Shard& sh = bank->shards[0];
   DeviceGuard guard(sh.dev);
   DeviceCtx& c = ctx_on(sh.dev);
-  const size_t np = (size_t)tb.B * kBatchSumBlocks;
+  const size_t np = (size_t)tb.B * G * kBatchSumBlocks;
   double* d_partial = nullptr;
   CU_FATAL(cudaMalloc(&d_partial, sizeof(double) * np));
-  c.launches += launch_batch_sums(tb.slab, tb.B, tb.ncells, d_partial, c.stream);
+  c.launches += launch_batch_sums(tb.slab, tb.B, tb.ncells, G, d_partial, c.stream);
   std::vector<double> h(np);
   CU_FATAL(cudaMemcpyAsync(h.data(), d_partial, sizeof(double) * np, cudaMemcpyDeviceToHost,
                            c.stream));
   CU_FATAL(cudaStreamSynchronize(c.stream));
   cudaFree(d_partial);
-  std::vector<double> x(tb.B);
-  double sum = 0.0;
-  for (int b = 0; b < tb.B; ++b) {
-    double t = 0.0;
-    for (int k = 0; k < kBatchSumBlocks; ++k) t += h[(size_t)b * kBatchSumBlocks + k];
-    const int nb = bank->n / tb.B + (b < bank->n % tb.B ? 1 : 0);
-    x[b] = t * (double)bank->n / (double)nb;
-    sum += x[b];
+  std::vector<double> total(tb.B, 0.0), seg(tb.B);
+  for (int g = 0; g < G; ++g) {
+    for (int b = 0; b < tb.B; ++b) {
+      double t = 0.0;
+      for (int k = 0; k < kBatchSumBlocks; ++k) t += h[((size_t)b * G + g) * kBatchSumBlocks + k];
+      seg[b] = t;
+      total[b] += t;
+    }
+    if (group_relerr) group_relerr[g] = batch_totals_relerr(bank, seg);
   }
-  const double m = sum / (double)tb.B;
-  double ss = 0.0;
-  for (int b = 0; b < tb.B; ++b) ss += (x[b] - m) * (x[b] - m);
-  const double var = ss / (double)(tb.B - 1);
-  return m == 0.0 ? 0.0 : sqrt(var / (double)tb.B) / fabs(m);
+  return batch_totals_relerr(bank, total);
 }
 
 Bank* batched_bank_of_tally(const double* tally) {
@@ -571,8 +589,9 @@ Bank* batched_bank_of_tally(const double* tally) {
 // A batched flux of the old attachment is flushed into the old array and its slab freed first.
 // B > 0 attaches a batched flux: deposits go to a zeroed slab of B partial fluxes on the bank's
 // GPU, allocated here. G > 0 attaches a group flux (G * ncells doubles) whose G + 1 edges are
-// copied from `edges` (host memory) into a device buffer of the bank. Returns 0, or -2 (error
-// set) when the slab or the edge buffer cannot be had.
+// copied from `edges` (host memory) into a device buffer of the bank; both attach a batched
+// group flux, whose B partial fluxes are G * ncells doubles each. Returns 0, or -2 (error set)
+// when the slab or the edge buffer cannot be had.
 int flux_attach(Bank* bank, double* flux, size_t ncells, int B = 0, const double* edges = nullptr,
                 int G = 0) {
   batches_release(bank, bank->flux_batches);
@@ -605,7 +624,10 @@ int flux_attach(Bank* bank, double* flux, size_t ncells, int B = 0, const double
   if (B > 0) {
     DeviceGuard guard(bank->shards[0].dev);
     DeviceCtx& c = ctx_on(bank->shards[0].dev);
-    const size_t bytes = sizeof(double) * (size_t)(B + 1) * ncells;
+    // the slab of a batched group flux is a batched flux of G * ncells "cells": batch-major
+    // (b, g, cell), so that every batch sweep serves it unchanged
+    const size_t slots = (size_t)(G > 0 ? G : 1) * ncells;
+    const size_t bytes = sizeof(double) * (size_t)(B + 1) * slots;
     double* slab = nullptr;
     CU_TRY(cudaMalloc(&slab, bytes));
     if (cudaError_t err = cudaMemsetAsync(slab, 0, bytes, c.stream)) {
@@ -617,7 +639,7 @@ int flux_attach(Bank* bank, double* flux, size_t ncells, int B = 0, const double
     TallyBatches& tb = bank->flux_batches;
     tb.slab = slab;
     tb.B = B;
-    tb.ncells = ncells;
+    tb.ncells = slots;
     tb.target = flux;
   }
   bank->flux = flux;
@@ -2742,6 +2764,11 @@ extern "C" int nb200_bank_set_group_flux_tally(nb200_particle_soa* particles, do
   }
   if (int rc = refuse_if_pending(bank, who)) return rc;
   if (!flux_device) return flux_attach(bank, nullptr, 0);
+  if (bank->batches.B > 0) {
+    set_error("%s: a bank with tally_batches has no unbatched group flux "
+              "(nb200_bank_set_batched_group_flux_tally attaches a batched one)", who);
+    return -3;
+  }
   if (int rc = refuse_flux_array(bank, flux_device, ncells, false, who)) return rc;
   if ((unsigned long long)ncells * (unsigned long long)ngroups >= (1ull << 31)) {
     set_error("%s: %d groups over %zu cells need 2^31 or more flux slots (the history kernel "
@@ -2751,11 +2778,47 @@ extern "C" int nb200_bank_set_group_flux_tally(nb200_particle_soa* particles, do
   return flux_attach(bank, flux_device, ncells, 0, edges_host, ngroups);
 }
 
-// The bank's flux batches, flushed into the attached array; nullptr (error set) if there are none.
-static Bank* flushed_flux_batches(nb200_particle_soa* particles, const char* who) {
+extern "C" int nb200_bank_set_batched_group_flux_tally(nb200_particle_soa* particles,
+                                                       double* flux_device, size_t ncells,
+                                                       const double* edges_host, int ngroups) {
+  const char* who = "nb200_bank_set_batched_group_flux_tally";
+  if (flux_device)
+    if (int rc = refuse_group_edges(edges_host, ngroups, who)) return rc;
   Bank* bank = bank_of(particles);
+  if (!bank) {
+    set_error("%s: not a bank handle", who);
+    return -3;
+  }
+  if (int rc = refuse_if_pending(bank, who)) return rc;
+  if (!flux_device) return flux_attach(bank, nullptr, 0);
+  if (int rc = refuse_flux_array(bank, flux_device, ncells, true, who)) return rc;
+  const int B = bank->batches.B;
+  if ((unsigned long long)B * (unsigned long long)ngroups * (unsigned long long)ncells >=
+      (1ull << 31)) {
+    set_error("%s: tally_batches=%d and %d groups over %zu cells need 2^31 or more flux slots "
+              "(the history kernel indexes them with 32 bits)", who, B, ngroups, ncells);
+    return -3;
+  }
+  return flux_attach(bank, flux_device, ncells, B, edges_host, ngroups);
+}
+
+// The bank's flux batches (a batched group flux's when `grouped`), flushed into the attached
+// array; nullptr (error set) if there are none. Each read call serves one kind, so that its
+// `ncells` has one meaning.
+static Bank* flushed_flux_batches(nb200_particle_soa* particles, const char* who,
+                                  bool grouped = false) {
+  Bank* bank = bank_of(particles);
+  if (grouped && (!bank || bank->flux_batches.B <= 0 || bank->flux_groups <= 0)) {
+    set_error("%s: not a bank handle with a batched group flux tally attached", who);
+    return nullptr;
+  }
   if (!bank || bank->flux_batches.B <= 0) {
     set_error("%s: not a bank handle with a batched flux tally attached", who);
+    return nullptr;
+  }
+  if (!grouped && bank->flux_groups > 0) {
+    set_error("%s: the bank's batched flux is a group flux (nb200_bank_group_flux_batches and "
+              "nb200_bank_group_flux_relerr read it)", who);
     return nullptr;
   }
   if (!bank->flux_batches.deposited) {
@@ -2797,6 +2860,44 @@ extern "C" int nb200_bank_flux_relerr(nb200_particle_soa* particles, double* rel
     CU_TRY(cudaStreamSynchronize(c.stream));
   }
   if (total_relerr_host) *total_relerr_host = batches_total_relerr(bank, tb);
+  return 0;
+}
+
+extern "C" int nb200_bank_group_flux_batches(nb200_particle_soa* particles, double* out_device,
+                                             size_t ncells, int ngroups) {
+  const char* who = "nb200_bank_group_flux_batches";
+  Bank* bank = flushed_flux_batches(particles, who, true);
+  if (!bank) return -3;
+  const TallyBatches& tb = bank->flux_batches;
+  if (!out_device || ncells != bank->flux_ncells || ngroups != bank->flux_groups) {
+    set_error("%s: the group flux batches cover %d groups of %zu cells, %d groups of %zu cells "
+              "were asked for", who, bank->flux_groups, bank->flux_ncells, ngroups, ncells);
+    return -3;
+  }
+  DeviceGuard guard(bank->shards[0].dev);
+  DeviceCtx& c = ctx_on(bank->shards[0].dev);
+  c.launches += launch_batch_export(tb.slab, tb.B, tb.ncells, out_device, c.stream);
+  CU_TRY(cudaGetLastError());
+  CU_TRY(cudaStreamSynchronize(c.stream));
+  return tb.B;
+}
+
+extern "C" int nb200_bank_group_flux_relerr(nb200_particle_soa* particles, double* relerr_device,
+                                            double* group_relerr_host, double* total_relerr_host) {
+  Bank* bank = flushed_flux_batches(particles, "nb200_bank_group_flux_relerr", true);
+  if (!bank) return -3;
+  const TallyBatches& tb = bank->flux_batches;
+  DeviceGuard guard(bank->shards[0].dev);
+  DeviceCtx& c = ctx_on(bank->shards[0].dev);
+  if (relerr_device) {
+    c.launches += launch_batch_relerr(tb.slab, tb.B, tb.ncells, bank->n, relerr_device, c.stream);
+    CU_TRY(cudaGetLastError());
+    CU_TRY(cudaStreamSynchronize(c.stream));
+  }
+  if (group_relerr_host || total_relerr_host) {
+    const double total = batches_total_relerr(bank, tb, bank->flux_groups, group_relerr_host);
+    if (total_relerr_host) *total_relerr_host = total;
+  }
   return 0;
 }
 

@@ -232,6 +232,8 @@ struct Bank {
   TallyBatches flux_batches;
   // nb200_bank_set_group_flux_tally: G > 0 when `flux` holds G energy groups of flux_ncells
   // cells each (group-major); the G + 1 edges are in flux_edges, device memory the bank owns.
+  // With flux_batches too (nb200_bank_set_batched_group_flux_tally) the batches cover
+  // flux_batches.ncells = G * flux_ncells slots; flux_ncells stays the mesh's cell count.
   double* flux_edges = nullptr;
   int flux_groups = 0;
   int n = 0;

@@ -205,6 +205,28 @@ __device__ __forceinline__ int group_index(const StepArgs& a, const GroupArgs& g
   return i;
 }
 
+// kBatched, kFlux and kGroups together (nb200_bank_set_batched_group_flux_tally): `flux` is the
+// library's flux batch slab of B batches of G group-major arrays of the mesh; batch and group
+// park side by side.
+struct ParkedBatchedGroupFlux : ParkedBatchedFlux {
+  int group[kHistoryThreads];
+};
+
+// Index of `cell` of group g of batch b in that slab: batch_slot over G * ncells "cells", so
+// the batch sweeps of tally_batches.cu serve it as a batched flux of G * ncells cells (32 bits:
+// the host refuses B * G * ncells >= 2^31).
+__device__ __forceinline__ int batched_group_index(const StepArgs& a, const BatchArgs& bt,
+                                                   const GroupArgs& gr, int b, int g, int cell) {
+  const int ncells = a.nx * a.ny;
+  const int i = (int)batch_slot(b, (size_t)(unsigned)(g * ncells + cell), bt.nbatches,
+                                (size_t)(gr.ngroups * ncells));
+#if defined(NB_ASSERT_BATCH_SLOT) || defined(NB_ASSERT_GROUP_SLOT)
+  assert(b >= 0 && b < bt.nbatches && g >= 0 && g < gr.ngroups && cell >= 0 && cell < ncells &&
+         i >= 0 && (long long)i < (long long)bt.nbatches * gr.ngroups * ncells);
+#endif
+  return i;
+}
+
 // `flux` is a kernel parameter behind the other three for the reason BatchArgs is one: a field
 // appended to StepArgs would move the offsets of the parameters that follow it; `grp` follows
 // `flux` for the same reason.
@@ -214,7 +236,9 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs
           double* __restrict__ flux, const GroupArgs grp) {
 #if NB_PARK_SMEM
   __shared__ std::conditional_t<
-      kBatched, std::conditional_t<kFlux, ParkedBatchedFlux, ParkedBatched>,
+      kBatched,
+      std::conditional_t<kFlux, std::conditional_t<kGroups, ParkedBatchedGroupFlux, ParkedBatchedFlux>,
+                         ParkedBatched>,
       std::conditional_t<kFlux, std::conditional_t<kGroups, ParkedGroupFlux, ParkedFlux>, Parked>>
       park;
 #define PARKED(name) park.name[threadIdx.x]
@@ -259,10 +283,11 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs
 #define NB_TALLY_AT(cell) \
   (kBatched ? bt.slab : a.tally), (kBatched ? batch_index(a, bt, PARKED_BATCH, (cell)) : (cell))
     // ... and a flux deposit: the caller's array (the group's slice of it for a group flux), or
-    // (batched) the batch's slot of the flux slab
-#define NB_FLUX_AT(cell)                                      \
-  flux, (kBatched  ? batch_index(a, bt, PARKED_BATCH, (cell)) \
-         : kGroups ? group_index(a, grp, PARKED_GROUP, (cell)) : (cell))
+    // (batched) the batch's slot of the flux slab (of the batch's group slice for a group flux)
+#define NB_FLUX_AT(cell)                                                                      \
+  flux, (kBatched && kGroups ? batched_group_index(a, bt, grp, PARKED_BATCH, PARKED_GROUP, (cell)) \
+         : kBatched          ? batch_index(a, bt, PARKED_BATCH, (cell))                       \
+         : kGroups           ? group_index(a, grp, PARKED_GROUP, (cell)) : (cell))
     // ... through this, which makes no deposit while the particle is outside the energy groups
 #define NB_FLUX_ADD(cell, value)                                                    \
   do {                                                                              \
@@ -621,6 +646,8 @@ int launch_history(const StepArgs& a, const BatchArgs& bt, double* flux, const G
       cudaFuncSetAttribute(k_history<false, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
       cudaFuncSetAttribute(k_history<true, false, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
       cudaFuncSetAttribute(k_history<false, false, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
+      cudaFuncSetAttribute(k_history<true, false, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
+      cudaFuncSetAttribute(k_history<false, false, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
       granted = smem_pad;
     }
     cfg.dynamicSmemBytes = (size_t)smem_pad;
@@ -643,9 +670,15 @@ int launch_history(const StepArgs& a, const BatchArgs& bt, double* flux, const G
   // and without batches alternating on one device change the graph's kernel and re-instantiate
   // it instead, which is correct and costs an instantiation per switch. A bank with a flux
   // array attached is the same: the host refuses prereduce for it, and a batched bank's flux is
-  // always batched (its `flux` is the flux batch slab). A group flux is neither batched nor
-  // prereduced (the host refuses both), and its kernel is one more switch of the same kind.
-  if (flux && grp.ngroups > 0) {
+  // always batched (its `flux` is the flux batch slab). A group flux is never prereduced (the
+  // host refuses it); on a batched bank it is always batched too, and either kernel is one more
+  // switch of the same kind.
+  if (flux && grp.ngroups > 0 && bt.nbatches > 0) {
+    if (fast_div)
+      cudaLaunchKernelEx(&cfg, k_history<true, false, true, true, true>, a, n_live, bt, flux, grp);
+    else
+      cudaLaunchKernelEx(&cfg, k_history<false, false, true, true, true>, a, n_live, bt, flux, grp);
+  } else if (flux && grp.ngroups > 0) {
     if (fast_div)
       cudaLaunchKernelEx(&cfg, k_history<true, false, false, true, true>, a, n_live, bt, flux, grp);
     else

@@ -61,15 +61,19 @@ k_batch_relerr(const double* __restrict__ slab, int B, size_t ncells, int n,
   }
 }
 
-// One batch per blockIdx.y; a fixed grid, so that the host's sum of the partials is the same
-// sum in the same order every time.
+// One batch per blockIdx.y and one of the nseg equal, consecutive segments of its cells per
+// blockIdx.z; a fixed grid, so that the host's sum of the partials is the same sum in the same
+// order every time. nseg = 1 is the whole batch.
 __global__ void __launch_bounds__(256)
-k_batch_sums(const double* __restrict__ slab, int B, size_t ncells, double* __restrict__ partial) {
+k_batch_sums(const double* __restrict__ slab, int B, size_t ncells, int nseg,
+             double* __restrict__ partial) {
   const int b = blockIdx.y;
+  const size_t seg = ncells / (size_t)nseg;
+  const size_t first = (size_t)blockIdx.z * seg;
   double s = 0.0;
-  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < ncells;
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < seg;
        i += (size_t)gridDim.x * blockDim.x)
-    s += slab[batch_slot(b, i, B, ncells)];
+    s += slab[batch_slot(b, first + i, B, ncells)];
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
   __shared__ double warp_part[8];
@@ -78,7 +82,7 @@ k_batch_sums(const double* __restrict__ slab, int B, size_t ncells, double* __re
   if (threadIdx.x == 0) {
     double t = 0.0;
     for (int w = 0; w < (int)(blockDim.x >> 5); ++w) t += warp_part[w];
-    partial[(size_t)b * gridDim.x + blockIdx.x] = t;
+    partial[((size_t)b * gridDim.z + blockIdx.z) * gridDim.x + blockIdx.x] = t;
   }
 }
 
@@ -98,8 +102,9 @@ int launch_batch_relerr(const double* slab, int B, size_t ncells, int n, double*
   return 1;
 }
 
-int launch_batch_sums(const double* slab, int B, size_t ncells, double* partial, cudaStream_t st) {
-  k_batch_sums<<<dim3(kBatchSumBlocks, B), 256, 0, st>>>(slab, B, ncells, partial);
+int launch_batch_sums(const double* slab, int B, size_t ncells, int nseg, double* partial,
+                      cudaStream_t st) {
+  k_batch_sums<<<dim3(kBatchSumBlocks, B, nseg), 256, 0, st>>>(slab, B, ncells, nseg, partial);
   return 1;
 }
 

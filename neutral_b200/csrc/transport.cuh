@@ -35,9 +35,12 @@ int launch_batch_export(const double* slab, int B, size_t ncells, double* out, c
 // relerr[cell] = relative error of the batch mean (n: particles, split into B batches).
 int launch_batch_relerr(const double* slab, int B, size_t ncells, int n, double* relerr,
                         cudaStream_t st);
-// partial[b * blocks + k] = sum over block k's cells of S_b (blocks = kBatchSumBlocks).
+// partial[(b * nseg + g) * blocks + k] = sum over block k's cells of segment g of S_b
+// (blocks = kBatchSumBlocks): the cells of a batch split into nseg equal, consecutive segments
+// (nseg divides ncells; 1: the whole batch, G: the groups of a batched group flux).
 constexpr int kBatchSumBlocks = 148;
-int launch_batch_sums(const double* slab, int B, size_t ncells, double* partial, cudaStream_t st);
+int launch_batch_sums(const double* slab, int B, size_t ncells, int nseg, double* partial,
+                      cudaStream_t st);
 // Per-step staging of the read-only inputs (stage.cu).
 int launch_stage_cs(const double* keys, const double* vals, int n, double2* kv, int* bucket,
                     unsigned long long bits0, int shift, int nb, const double* twin_keys,

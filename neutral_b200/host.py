@@ -58,6 +58,8 @@ EXPORTED_SYMBOLS = [
     "nb200_microbench_red", "nb200_bank_tally_batches", "nb200_bank_tally_relerr",
     "nb200_selftest_batch_of", "nb200_bank_set_flux_tally", "nb200_bank_set_batched_flux_tally",
     "nb200_bank_flux_batches", "nb200_bank_flux_relerr", "nb200_bank_set_group_flux_tally",
+    "nb200_bank_set_batched_group_flux_tally", "nb200_bank_group_flux_batches",
+    "nb200_bank_group_flux_relerr",
 ]
 
 #: include/neutral_b200.h
@@ -143,6 +145,10 @@ def load_library(build: bool = False) -> C.CDLL:
     L.nb200_bank_flux_relerr.argtypes = [_soa_p, C.c_void_p, _dp]
     L.nb200_bank_set_group_flux_tally.argtypes = [_soa_p, C.c_void_p, C.c_size_t, C.c_void_p,
                                                   C.c_int]
+    L.nb200_bank_set_batched_group_flux_tally.argtypes = [_soa_p, C.c_void_p, C.c_size_t,
+                                                          C.c_void_p, C.c_int]
+    L.nb200_bank_group_flux_batches.argtypes = [_soa_p, C.c_void_p, C.c_size_t, C.c_int]
+    L.nb200_bank_group_flux_relerr.argtypes = [_soa_p, C.c_void_p, C.c_void_p, _dp]
     L.nb200_last_step_stats.argtypes = [_u64p]
     L.nb200_solve_finish.argtypes = [_u64p, _u64p]
     L.nb200_kernel_launches.restype = C.c_uint64
@@ -249,15 +255,22 @@ class Simulation:
 
     def __init__(self, problem: Problem, rank: int = 0, nranks: int = 1,
                  per_particle_counters: bool = True, quiet: bool = True, ngpus: int = 1,
-                 tally_batches: int = 0, flux_tally: bool = False, flux_groups=None):
+                 tally_batches: int = 0, flux_tally: bool = False, flux_groups=None,
+                 group_flux_batches: bool = False):
         self.lib = load_library()
         #: energy edges of the group flux (nb200_bank_set_group_flux_tally), or None
         self.flux_edges = None
+        #: the group flux is batched (nb200_bank_set_batched_group_flux_tally), see
+        #: :meth:`group_flux_relative_error`
+        self.group_flux_batches = group_flux_batches
+        if group_flux_batches and (flux_groups is None or not tally_batches or flux_tally):
+            raise NeutralB200Error("group_flux_batches needs flux_groups and tally_batches, "
+                                   "without flux_tally")
         if flux_groups is not None:
-            if flux_tally or tally_batches:
-                raise NeutralB200Error("flux_groups cannot be combined with flux_tally or "
-                                       "tally_batches (a bank has one flux, and a group flux "
-                                       "has no batches)")
+            if flux_tally or (tally_batches and not group_flux_batches):
+                raise NeutralB200Error("flux_groups cannot be combined with flux_tally, nor with "
+                                       "tally_batches unless group_flux_batches=True (a bank has "
+                                       "one flux)")
             self.flux_edges = np.array(flux_groups, dtype=np.float64)
             if self.flux_edges.ndim != 1 or self.flux_edges.size < 2:
                 raise NeutralB200Error("flux_groups: G + 1 >= 2 energy edges in eV, increasing")
@@ -336,7 +349,12 @@ class Simulation:
     def _attach_flux(self) -> None:
         if self.flux is None:
             return
-        if self.flux_edges is not None:
+        if self.group_flux_batches:
+            ncells = self.problem.deck.nx * self.problem.deck.ny
+            _check(self.lib.nb200_bank_set_batched_group_flux_tally(
+                self.bank, self.flux.ptr, ncells, self.flux_edges.ctypes.data,
+                self.flux_edges.size - 1), "bank_set_batched_group_flux_tally")
+        elif self.flux_edges is not None:
             ncells = self.problem.deck.nx * self.problem.deck.ny
             _check(self.lib.nb200_bank_set_group_flux_tally(
                 self.bank, self.flux.ptr, ncells, self.flux_edges.ctypes.data,
@@ -525,6 +543,40 @@ class Simulation:
             _check(self.lib.nb200_bank_flux_relerr(self.bank, out.ptr, C.byref(total)),
                    "bank_flux_relerr")
             return out.download().reshape(d.ny, d.nx), float(total.value)
+        finally:
+            out.free()
+
+    def group_flux_batches_to_host(self) -> np.ndarray:
+        """(B, G, ny, nx) cumulative partial group fluxes of the B particle batches
+        (``group_flux_batches=True``); flushes the group flux array first."""
+        d = self.problem.deck
+        ncells = d.nx * d.ny
+        G = self.flux_edges.size - 1
+        out = DeviceArray(self.tally_batches * G * ncells, np.float64)
+        try:
+            rc = self.lib.nb200_bank_group_flux_batches(self.bank, out.ptr, ncells, G)
+            if rc != self.tally_batches:
+                raise NeutralB200Error(
+                    f"bank_group_flux_batches: {self.lib.nb200_last_error().decode()}")
+            return out.download().reshape(self.tally_batches, G, d.ny, d.nx)
+        finally:
+            out.free()
+
+    def group_flux_relative_error(self) -> Tuple[np.ndarray, np.ndarray, float]:
+        """Relative error of the group flux from its batches (``group_flux_batches=True``):
+        (R per group and cell as (G, ny, nx), R of every group's total over the mesh as (G,),
+        R of the grand total), with the estimator of :meth:`tally_relative_error`. The R per
+        group is the error bar of the spectrum."""
+        d = self.problem.deck
+        G = self.flux_edges.size - 1
+        out = DeviceArray(G * d.nx * d.ny, np.float64)
+        groups = np.zeros(G)
+        total = C.c_double(0.0)
+        try:
+            _check(self.lib.nb200_bank_group_flux_relerr(self.bank, out.ptr, groups.ctypes.data,
+                                                         C.byref(total)),
+                   "bank_group_flux_relerr")
+            return out.download().reshape(G, d.ny, d.nx), groups, float(total.value)
         finally:
             out.free()
 

@@ -13,11 +13,14 @@ of the energy batches.
 With --groups G [G ...] each G adds one more configuration to the alternation: a group flux
 (nb200_bank_set_group_flux_tally) over G logarithmic energy groups from 1e-3 eV to twice the
 deck's initial energy, which cover every energy the deck reaches. Its rows carry the flux summed
-over the groups, and their ratio to the run without flux.
+over the groups, and their ratio to the run without flux. With --tally-batches B as well, every
+bank of the alternation is batched: no flux, a batched plain flux, and one batched group flux per
+G (nb200_bank_set_batched_group_flux_tally), whose slab holds (B + 1) * G * ncells doubles.
 
     python tools/flux_tally_cost.py --out profiles/r04/flux_tally_cost.json
     python tools/flux_tally_cost.py --tally-batches 16 --out flux_batches_cost_b16.json
     python tools/flux_tally_cost.py --groups 8 32 --out profiles/r05/group_flux_cost.json
+    python tools/flux_tally_cost.py --tally-batches 16 --groups 8 --out batched_group_b16.json
 
 The GPU's name and power limit are written into the same output. Needs a CUDA device.
 """
@@ -55,7 +58,9 @@ def measure(args) -> dict:
                 for flux in (False, True)}
         for g in args.groups:
             sims[f"groups_{g}"] = Simulation(prob, per_particle_counters=False,
-                                             flux_groups=np.geomspace(1.0e-3, 2.0 * e0, g + 1))
+                                             flux_groups=np.geomspace(1.0e-3, 2.0 * e0, g + 1),
+                                             tally_batches=args.tally_batches,
+                                             group_flux_batches=args.tally_batches > 0)
         for sim in sims.values():
             sim.inject()
         injected = sims[False].bank_to_host()
@@ -110,11 +115,10 @@ def main():
     ap.add_argument("--tally-batches", type=int, default=0,
                     help="B > 0: both banks batched, the flux of the second batched too")
     ap.add_argument("--groups", type=int, nargs="*", default=[],
-                    help="G ...: one more configuration per G, a group flux over G log groups")
+                    help="G ...: one more configuration per G, a group flux over G log groups "
+                         "(batched with --tally-batches)")
     ap.add_argument("--out", default=None, help="JSON file for the results")
     args = ap.parse_args()
-    if args.groups and args.tally_batches:
-        ap.error("--groups: a group flux has no tally batches")
     result = {"what": "ms per resident deck run (run_pipelined, CUDA events, median) without "
                       "and with a flux array attached (plain, and a group flux per --groups G), "
                       "alternating run by run; events/s",
