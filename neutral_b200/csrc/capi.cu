@@ -472,7 +472,7 @@ void batches_attach(Bank* bank, int B) {
 }
 
 // Brings the target of `tb` up to date (the caller's tally for bank->batches, the attached flux
-// array for bank->flux_batches): target += sum_b S_b - F, F = sum_b S_b. Synchronous.
+// array for bank->flux.batches): target += sum_b S_b - F, F = sum_b S_b. Synchronous.
 void batches_flush(Bank* bank, TallyBatches& tb) {
   if (!tb.dirty || !tb.target) return;
   const Shard& sh = bank->shards[0];
@@ -546,16 +546,23 @@ static double batch_totals_relerr(const Bank* bank, const std::vector<double>& t
   return m == 0.0 ? 0.0 : sqrt(var / (double)B) / fabs(m);
 }
 
-// R of the total of `tb` (tally or flux): the B batch totals through a fixed-order device
-// reduction, then the estimator in FP64 on the host. With G > 1 the cells of every batch are G
-// equal, consecutive segments (the groups of a batched group flux): `group_relerr` (G doubles,
-// optional) gets R of every segment's total, and a batch's total is the sum of its G segment
-// totals in group order.
-double batches_total_relerr(Bank* bank, const TallyBatches& tb, int G = 1,
-                            double* group_relerr = nullptr) {
+// Relative errors of `tb` (tally or flux). `relerr_device` (optional, tb.ncells doubles on the
+// bank's GPU) gets R of every slot. `total` (optional) gets R of the total: the B batch totals
+// through a fixed-order device reduction, then the estimator in FP64 on the host. With G > 1 the
+// cells of every batch are G equal, consecutive segments (the groups of a batched group flux):
+// `group_relerr` (G doubles, optional) gets R of every segment's total, and a batch's total is
+// the sum of its G segment totals in group order. Returns 0, or -2 (error set).
+int batches_relerr(Bank* bank, const TallyBatches& tb, double* relerr_device, int G,
+                   double* group_relerr, double* total) {
   const Shard& sh = bank->shards[0];
   DeviceGuard guard(sh.dev);
   DeviceCtx& c = ctx_on(sh.dev);
+  if (relerr_device) {
+    c.launches += launch_batch_relerr(tb.slab, tb.B, tb.ncells, bank->n, relerr_device, c.stream);
+    CU_TRY(cudaGetLastError());
+    CU_TRY(cudaStreamSynchronize(c.stream));
+  }
+  if (!group_relerr && !total) return 0;
   const size_t np = (size_t)tb.B * G * kBatchSumBlocks;
   double* d_partial = nullptr;
   CU_FATAL(cudaMalloc(&d_partial, sizeof(double) * np));
@@ -565,17 +572,18 @@ double batches_total_relerr(Bank* bank, const TallyBatches& tb, int G = 1,
                            c.stream));
   CU_FATAL(cudaStreamSynchronize(c.stream));
   cudaFree(d_partial);
-  std::vector<double> total(tb.B, 0.0), seg(tb.B);
+  std::vector<double> sum(tb.B, 0.0), seg(tb.B);
   for (int g = 0; g < G; ++g) {
     for (int b = 0; b < tb.B; ++b) {
       double t = 0.0;
       for (int k = 0; k < kBatchSumBlocks; ++k) t += h[((size_t)b * G + g) * kBatchSumBlocks + k];
       seg[b] = t;
-      total[b] += t;
+      sum[b] += t;
     }
     if (group_relerr) group_relerr[g] = batch_totals_relerr(bank, seg);
   }
-  return batch_totals_relerr(bank, total);
+  if (total) *total = batch_totals_relerr(bank, sum);
+  return 0;
 }
 
 Bank* batched_bank_of_tally(const double* tally) {
@@ -594,16 +602,14 @@ Bank* batched_bank_of_tally(const double* tally) {
 // when the slab or the edge buffer cannot be had.
 int flux_attach(Bank* bank, double* flux, size_t ncells, int B = 0, const double* edges = nullptr,
                 int G = 0) {
-  batches_release(bank, bank->flux_batches);
+  FluxTally& f = bank->flux;
+  batches_release(bank, f.batches);
   g_flux.erase(std::remove(g_flux.begin(), g_flux.end(), bank), g_flux.end());
-  bank->flux = nullptr;
-  bank->flux_ncells = 0;
-  if (bank->flux_edges) {
+  if (f.edges) {
     DeviceGuard guard(bank->shards[0].dev);
-    cudaFree(bank->flux_edges);  // synchronises: no timestep still reads them
-    bank->flux_edges = nullptr;
+    cudaFree(f.edges);  // synchronises: no timestep still reads them
   }
-  bank->flux_groups = 0;
+  f = FluxTally{};
   if (!flux) return 0;
   if (G > 0) {
     DeviceGuard guard(bank->shards[0].dev);
@@ -618,8 +624,8 @@ int flux_attach(Bank* bank, double* flux, size_t ncells, int B = 0, const double
       set_error("copying the energy edges to the device failed: %s", cudaGetErrorString(err));
       return -2;
     }
-    bank->flux_edges = d_edges;
-    bank->flux_groups = G;
+    f.edges = d_edges;
+    f.groups = G;
   }
   if (B > 0) {
     DeviceGuard guard(bank->shards[0].dev);
@@ -636,14 +642,13 @@ int flux_attach(Bank* bank, double* flux, size_t ncells, int B = 0, const double
       return -2;
     }
     // the bank has a batched flux only once its slab is whole
-    TallyBatches& tb = bank->flux_batches;
-    tb.slab = slab;
-    tb.B = B;
-    tb.ncells = slots;
-    tb.target = flux;
+    f.batches.slab = slab;
+    f.batches.B = B;
+    f.batches.ncells = slots;
+    f.batches.target = flux;
   }
-  bank->flux = flux;
-  bank->flux_ncells = ncells;
+  f.target = flux;
+  f.ncells = ncells;
   g_flux.push_back(bank);
   return 0;
 }
@@ -653,9 +658,9 @@ int flux_attach(Bank* bank, double* flux, size_t ncells, int B = 0, const double
 void flux_detach_array(const double* buf) {
   std::vector<Bank*> attached;
   for (Bank* b : g_flux)
-    if (b->flux == buf) attached.push_back(b);
+    if (b->flux.target == buf) attached.push_back(b);
   for (Bank* b : attached) {
-    b->flux_batches.target = nullptr;
+    b->flux.batches.target = nullptr;
     flux_attach(b, nullptr, 0);
   }
 }
@@ -664,9 +669,9 @@ void flux_detach_array(const double* buf) {
 // or options changed since the array was attached.
 void flux_check(Bank* bank, const StepRequest& rq, bool grouped) {
   const size_t ncells = (size_t)rq.nx * (size_t)rq.ny;
-  if (ncells != bank->flux_ncells)
+  if (ncells != bank->flux.ncells)
     terminate("solve_transport_2d: the bank's flux tally has %zu cells, the mesh has %d x %d = "
-              "%zu", bank->flux_ncells, rq.nx, rq.ny, ncells);
+              "%zu", bank->flux.ncells, rq.nx, rq.ny, ncells);
   if (grouped || !single_shard(bank))
     terminate("solve_transport_2d: a flux tally in a sharded or multi-process run");
   if (!opt_of(bank, &Options::pipeline) || opt_of(bank, &Options::tally_prereduce))
@@ -1425,7 +1430,7 @@ void flush_groups_touching(const void* ptr, size_t bytes) {
   for (Bank* b : g_batched)
     if (touches(b->batches)) batches_flush(b, b->batches);
   for (Bank* b : g_flux)
-    if (touches(b->flux_batches)) batches_flush(b, b->flux_batches);
+    if (touches(b->flux.batches)) batches_flush(b, b->flux.batches);
   for (TallyGroup* g : g_groups) {
     if (!g->dirty || !g->target) continue;
     const char* lo = (const char*)g->target;
@@ -1509,7 +1514,7 @@ void enqueue_step(Bank* bank, const StepRequest& rq) {
     epoch = group->epoch + 1;
   }
   if (bank->batches.B > 0) batches_bind(bank, rq);
-  if (bank->flux) flux_check(bank, rq, group != nullptr);
+  if (bank->flux.target) flux_check(bank, rq, group != nullptr);
   PendingStep ps;
   ps.pipeline = opt_of(bank, &Options::pipeline) != 0;
   ps.print = opt_of(bank, &Options::print) != 0;
@@ -1534,8 +1539,8 @@ void enqueue_step(Bank* bank, const StepRequest& rq) {
     io.a_vals = replica_of(c, sh, pd, rq.a_vals, (size_t)rq.a_n);
     io.tally = rq.tally;
     io.batches = BatchArgs{bank->batches.slab, bank->batches.B, bank->n};
-    io.flux = bank->flux_batches.B > 0 ? bank->flux_batches.slab : bank->flux;
-    io.groups = GroupArgs{bank->flux_edges, bank->flux_groups};
+    io.flux = bank->flux.batches.B > 0 ? bank->flux.batches.slab : bank->flux.target;
+    io.groups = GroupArgs{bank->flux.edges, bank->flux.groups};
     // per-particle counters live on the primary GPU, indexed in injection order: a secondary
     // shard reaches its part of them through peer access (one 8-byte update per particle-step)
     const bool counters_ok = sh.dev == pd || (group && group->collective);
@@ -1556,8 +1561,8 @@ void enqueue_step(Bank* bank, const StepRequest& rq) {
       enqueue_shard_step(c, bank, sh, rq, io, slot, nullptr, 0);
     }
   }
-  if (bank->batches.B > 0) bank->batches.dirty = true;
-  if (bank->flux_batches.B > 0) bank->flux_batches.dirty = bank->flux_batches.deposited = true;
+  for (TallyBatches* tb : {&bank->batches, &bank->flux.batches})
+    if (tb->B > 0) tb->dirty = tb->deposited = true;
   if (group) {
     group->steps_deposited++;
     group->dirty = true;
@@ -1906,7 +1911,7 @@ extern "C" void validate(const int nx, const int ny, const char* params_filename
   if (json && *json) {
     if (Bank* b = batched_bank_of_tally(energy_tally)) {
       batches = b->batches.B;
-      total_relerr = batches_total_relerr(b, b->batches);
+      batches_relerr(b, b->batches, nullptr, 1, nullptr, &total_relerr);
     }
   }
   printf("\nFinal global_energy_tally %.15e\n", total);
@@ -2530,8 +2535,8 @@ extern "C" int nb200_bank_set_option(nb200_particle_soa* particles, const char* 
               "kernel without tally_prereduce has batches)", name, value);
     return NB200_BAD_OPTION;
   }
-  if (bank->flux && ((spec.slot == &Options::pipeline && value == 0) ||
-                     (spec.slot == &Options::tally_prereduce && value != 0))) {
+  if (bank->flux.target && ((spec.slot == &Options::pipeline && value == 0) ||
+                            (spec.slot == &Options::tally_prereduce && value != 0))) {
     set_error("nb200_bank_set_option: %s=%d on a bank with a flux tally attached (only the "
               "pipelined kernel without tally_prereduce has the flux)", name, value);
     return NB200_BAD_OPTION;
@@ -2590,40 +2595,47 @@ extern "C" int nb200_tally_sync(double* tally_device) {
   for (Bank* b : g_batched)
     if (!tally_device || b->batches.target == tally_device) batches_flush(b, b->batches);
   for (Bank* b : g_flux)
-    if (!tally_device || b->flux == tally_device) batches_flush(b, b->flux_batches);
+    if (!tally_device || b->flux.target == tally_device) batches_flush(b, b->flux.batches);
   for (TallyGroup* g : g_groups)
     if (!tally_device || g->target == tally_device) group_flush(*g);
   return 0;
 }
 
 // ------------------------------------------------------------------------ tally batches --
-// The bank's batched state, flushed into the caller's tally; nullptr (error set) if there is none.
-static Bank* flushed_batches(nb200_particle_soa* particles, const char* who) {
-  Bank* bank = bank_of(particles);
-  if (!bank || bank->batches.B <= 0) {
-    set_error("%s: not a bank handle created with tally_batches", who);
+// The batches a read call serves: the deposition batches (nb200_bank_tally_*), a batched plain
+// flux (nb200_bank_flux_*) or a batched group flux (nb200_bank_group_flux_*). Each call serves
+// one kind, so that its `ncells` has one meaning.
+enum class BatchKind { kTally, kFlux, kGroupFlux };
+
+// The bank's batches of that kind, flushed into their target; nullptr (error set) if there are
+// none.
+static TallyBatches* flushed_batches(Bank* bank, BatchKind kind, const char* who) {
+  const bool tally = kind == BatchKind::kTally, grouped = kind == BatchKind::kGroupFlux;
+  TallyBatches* tb = !bank ? nullptr : tally ? &bank->batches : &bank->flux.batches;
+  if (!tb || tb->B <= 0 || (grouped && bank->flux.groups <= 0)) {
+    set_error(tally     ? "%s: not a bank handle created with tally_batches"
+              : grouped ? "%s: not a bank handle with a batched group flux tally attached"
+                        : "%s: not a bank handle with a batched flux tally attached",
+              who);
     return nullptr;
   }
-  if (!bank->batches.slab) {
-    set_error("%s: no timestep of this bank has deposited into its batches yet", who);
+  if (kind == BatchKind::kFlux && bank->flux.groups > 0) {
+    set_error("%s: the bank's batched flux is a group flux (nb200_bank_group_flux_batches and "
+              "nb200_bank_group_flux_relerr read it)", who);
     return nullptr;
   }
-  batches_flush(bank, bank->batches);
-  return bank;
+  if (!tb->deposited) {
+    set_error(tally ? "%s: no timestep of this bank has deposited into its batches yet"
+                    : "%s: no timestep of this bank has deposited into its flux batches yet",
+              who);
+    return nullptr;
+  }
+  batches_flush(bank, *tb);
+  return tb;
 }
 
-extern "C" int nb200_bank_tally_batches(nb200_particle_soa* particles, double* out_device,
-                                        size_t ncells) {
-  CTX_OR_RETURN(c0);
-  (void)c0;
-  Bank* bank = flushed_batches(particles, "nb200_bank_tally_batches");
-  if (!bank) return -3;
-  const TallyBatches& tb = bank->batches;
-  if (!out_device || ncells != tb.ncells) {
-    set_error("nb200_bank_tally_batches: the batches cover %zu cells, %zu were asked for",
-              tb.ncells, ncells);
-    return -3;
-  }
+// out_device = the B partial arrays of `tb`, batch-major. Returns B, or -2 (error set).
+static int export_batches(Bank* bank, const TallyBatches& tb, double* out_device) {
   DeviceGuard guard(bank->shards[0].dev);
   DeviceCtx& c = ctx_on(bank->shards[0].dev);
   c.launches += launch_batch_export(tb.slab, tb.B, tb.ncells, out_device, c.stream);
@@ -2632,22 +2644,29 @@ extern "C" int nb200_bank_tally_batches(nb200_particle_soa* particles, double* o
   return tb.B;
 }
 
+extern "C" int nb200_bank_tally_batches(nb200_particle_soa* particles, double* out_device,
+                                        size_t ncells) {
+  CTX_OR_RETURN(c0);
+  (void)c0;
+  Bank* bank = bank_of(particles);
+  TallyBatches* tb = flushed_batches(bank, BatchKind::kTally, "nb200_bank_tally_batches");
+  if (!tb) return -3;
+  if (!out_device || ncells != tb->ncells) {
+    set_error("nb200_bank_tally_batches: the batches cover %zu cells, %zu were asked for",
+              tb->ncells, ncells);
+    return -3;
+  }
+  return export_batches(bank, *tb, out_device);
+}
+
 extern "C" int nb200_bank_tally_relerr(nb200_particle_soa* particles, double* relerr_device,
                                        double* total_relerr_host) {
   CTX_OR_RETURN(c0);
   (void)c0;
-  Bank* bank = flushed_batches(particles, "nb200_bank_tally_relerr");
-  if (!bank) return -3;
-  const TallyBatches& tb = bank->batches;
-  DeviceGuard guard(bank->shards[0].dev);
-  DeviceCtx& c = ctx_on(bank->shards[0].dev);
-  if (relerr_device) {
-    c.launches += launch_batch_relerr(tb.slab, tb.B, tb.ncells, bank->n, relerr_device, c.stream);
-    CU_TRY(cudaGetLastError());
-    CU_TRY(cudaStreamSynchronize(c.stream));
-  }
-  if (total_relerr_host) *total_relerr_host = batches_total_relerr(bank, tb);
-  return 0;
+  Bank* bank = bank_of(particles);
+  TallyBatches* tb = flushed_batches(bank, BatchKind::kTally, "nb200_bank_tally_relerr");
+  if (!tb) return -3;
+  return batches_relerr(bank, *tb, relerr_device, 1, nullptr, total_relerr_host);
 }
 
 // Host-side evaluation of the history kernel's pid -> batch map (pure integer arithmetic), for
@@ -2659,7 +2678,7 @@ extern "C" unsigned nb200_selftest_batch_of(uint64_t pid, uint64_t n, int nbatch
 
 // ------------------------------------------------------------------------- flux tally --
 // Why flux_device cannot be attached to the bank (plain, or batched with the bank's B), as an
-// error code with the message set; 0 if it can. Both attach functions check the same things.
+// error code with the message set; 0 if it can.
 static int refuse_flux_array(Bank* bank, double* flux_device, size_t ncells, bool batched,
                              const char* who) {
   if (!single_shard(bank) || g_mp) {
@@ -2685,11 +2704,6 @@ static int refuse_flux_array(Bank* bank, double* flux_device, size_t ncells, boo
     set_error("%s: %zu cells (1 .. 2^31 - 1)", who, ncells);
     return -3;
   }
-  if (batched && (unsigned long long)ncells * (unsigned long long)bank->batches.B >= (1ull << 31)) {
-    set_error("%s: tally_batches=%d over %zu cells needs 2^31 or more flux slots (the history "
-              "kernel indexes them with 32 bits)", who, bank->batches.B, ncells);
-    return -3;
-  }
   cudaPointerAttributes attr{};
   if (cudaPointerGetAttributes(&attr, flux_device) != cudaSuccess ||
       (attr.type != cudaMemoryTypeDevice && attr.type != cudaMemoryTypeManaged) ||
@@ -2700,34 +2714,6 @@ static int refuse_flux_array(Bank* bank, double* flux_device, size_t ncells, boo
     return -3;
   }
   return 0;
-}
-
-extern "C" int nb200_bank_set_flux_tally(nb200_particle_soa* particles, double* flux_device,
-                                         size_t ncells) {
-  const char* who = "nb200_bank_set_flux_tally";
-  Bank* bank = bank_of(particles);
-  if (!bank) {
-    set_error("%s: not a bank handle", who);
-    return -3;
-  }
-  if (int rc = refuse_if_pending(bank, who)) return rc;
-  if (!flux_device) return flux_attach(bank, nullptr, 0);
-  if (int rc = refuse_flux_array(bank, flux_device, ncells, false, who)) return rc;
-  return flux_attach(bank, flux_device, ncells);
-}
-
-extern "C" int nb200_bank_set_batched_flux_tally(nb200_particle_soa* particles,
-                                                 double* flux_device, size_t ncells) {
-  const char* who = "nb200_bank_set_batched_flux_tally";
-  Bank* bank = bank_of(particles);
-  if (!bank) {
-    set_error("%s: not a bank handle", who);
-    return -3;
-  }
-  if (int rc = refuse_if_pending(bank, who)) return rc;
-  if (!flux_device) return flux_attach(bank, nullptr, 0);
-  if (int rc = refuse_flux_array(bank, flux_device, ncells, true, who)) return rc;
-  return flux_attach(bank, flux_device, ncells, bank->batches.B);
 }
 
 // Why `edges` (G + 1 host doubles) cannot be a group flux's energy edges, as -3 with the message
@@ -2751,31 +2737,53 @@ static int refuse_group_edges(const double* edges, int ngroups, const char* who)
   return 0;
 }
 
-extern "C" int nb200_bank_set_group_flux_tally(nb200_particle_soa* particles, double* flux_device,
-                                               size_t ncells, const double* edges_host,
-                                               int ngroups) {
-  const char* who = "nb200_bank_set_group_flux_tally";
-  if (flux_device)
-    if (int rc = refuse_group_edges(edges_host, ngroups, who)) return rc;
+// The four nb200_bank_set_*flux_tally calls: attaches `flux` (null: detaches) to the bank, a
+// batched flux with the bank's batches when `batched`, a group flux of G > 0 groups over the
+// caller's edges (already checked by refuse_group_edges).
+static int set_flux_tally(nb200_particle_soa* particles, double* flux, size_t ncells,
+                          const double* edges, int G, bool batched, const char* who) {
   Bank* bank = bank_of(particles);
   if (!bank) {
     set_error("%s: not a bank handle", who);
     return -3;
   }
   if (int rc = refuse_if_pending(bank, who)) return rc;
-  if (!flux_device) return flux_attach(bank, nullptr, 0);
-  if (bank->batches.B > 0) {
+  if (!flux) return flux_attach(bank, nullptr, 0);
+  if (G > 0 && !batched && bank->batches.B > 0) {
     set_error("%s: a bank with tally_batches has no unbatched group flux "
               "(nb200_bank_set_batched_group_flux_tally attaches a batched one)", who);
     return -3;
   }
-  if (int rc = refuse_flux_array(bank, flux_device, ncells, false, who)) return rc;
-  if ((unsigned long long)ncells * (unsigned long long)ngroups >= (1ull << 31)) {
-    set_error("%s: %d groups over %zu cells need 2^31 or more flux slots (the history kernel "
-              "indexes them with 32 bits)", who, ngroups, ncells);
+  if (int rc = refuse_flux_array(bank, flux, ncells, batched, who)) return rc;
+  const int B = batched ? bank->batches.B : 0;
+  if ((unsigned long long)std::max(B, 1) * (unsigned long long)std::max(G, 1) * ncells >=
+      (1ull << 31)) {
+    set_error("%s: tally_batches=%d and %d groups over %zu cells need 2^31 or more flux slots "
+              "(the history kernel indexes them with 32 bits)", who, B, G, ncells);
     return -3;
   }
-  return flux_attach(bank, flux_device, ncells, 0, edges_host, ngroups);
+  return flux_attach(bank, flux, ncells, B, edges, G);
+}
+
+extern "C" int nb200_bank_set_flux_tally(nb200_particle_soa* particles, double* flux_device,
+                                         size_t ncells) {
+  return set_flux_tally(particles, flux_device, ncells, nullptr, 0, false,
+                        "nb200_bank_set_flux_tally");
+}
+
+extern "C" int nb200_bank_set_batched_flux_tally(nb200_particle_soa* particles,
+                                                 double* flux_device, size_t ncells) {
+  return set_flux_tally(particles, flux_device, ncells, nullptr, 0, true,
+                        "nb200_bank_set_batched_flux_tally");
+}
+
+extern "C" int nb200_bank_set_group_flux_tally(nb200_particle_soa* particles, double* flux_device,
+                                               size_t ncells, const double* edges_host,
+                                               int ngroups) {
+  const char* who = "nb200_bank_set_group_flux_tally";
+  if (flux_device)
+    if (int rc = refuse_group_edges(edges_host, ngroups, who)) return rc;
+  return set_flux_tally(particles, flux_device, ncells, edges_host, ngroups, false, who);
 }
 
 extern "C" int nb200_bank_set_batched_group_flux_tally(nb200_particle_soa* particles,
@@ -2784,121 +2792,52 @@ extern "C" int nb200_bank_set_batched_group_flux_tally(nb200_particle_soa* parti
   const char* who = "nb200_bank_set_batched_group_flux_tally";
   if (flux_device)
     if (int rc = refuse_group_edges(edges_host, ngroups, who)) return rc;
-  Bank* bank = bank_of(particles);
-  if (!bank) {
-    set_error("%s: not a bank handle", who);
-    return -3;
-  }
-  if (int rc = refuse_if_pending(bank, who)) return rc;
-  if (!flux_device) return flux_attach(bank, nullptr, 0);
-  if (int rc = refuse_flux_array(bank, flux_device, ncells, true, who)) return rc;
-  const int B = bank->batches.B;
-  if ((unsigned long long)B * (unsigned long long)ngroups * (unsigned long long)ncells >=
-      (1ull << 31)) {
-    set_error("%s: tally_batches=%d and %d groups over %zu cells need 2^31 or more flux slots "
-              "(the history kernel indexes them with 32 bits)", who, B, ngroups, ncells);
-    return -3;
-  }
-  return flux_attach(bank, flux_device, ncells, B, edges_host, ngroups);
-}
-
-// The bank's flux batches (a batched group flux's when `grouped`), flushed into the attached
-// array; nullptr (error set) if there are none. Each read call serves one kind, so that its
-// `ncells` has one meaning.
-static Bank* flushed_flux_batches(nb200_particle_soa* particles, const char* who,
-                                  bool grouped = false) {
-  Bank* bank = bank_of(particles);
-  if (grouped && (!bank || bank->flux_batches.B <= 0 || bank->flux_groups <= 0)) {
-    set_error("%s: not a bank handle with a batched group flux tally attached", who);
-    return nullptr;
-  }
-  if (!bank || bank->flux_batches.B <= 0) {
-    set_error("%s: not a bank handle with a batched flux tally attached", who);
-    return nullptr;
-  }
-  if (!grouped && bank->flux_groups > 0) {
-    set_error("%s: the bank's batched flux is a group flux (nb200_bank_group_flux_batches and "
-              "nb200_bank_group_flux_relerr read it)", who);
-    return nullptr;
-  }
-  if (!bank->flux_batches.deposited) {
-    set_error("%s: no timestep of this bank has deposited into its flux batches yet", who);
-    return nullptr;
-  }
-  batches_flush(bank, bank->flux_batches);
-  return bank;
+  return set_flux_tally(particles, flux_device, ncells, edges_host, ngroups, true, who);
 }
 
 extern "C" int nb200_bank_flux_batches(nb200_particle_soa* particles, double* out_device,
                                        size_t ncells) {
-  Bank* bank = flushed_flux_batches(particles, "nb200_bank_flux_batches");
-  if (!bank) return -3;
-  const TallyBatches& tb = bank->flux_batches;
-  if (!out_device || ncells != tb.ncells) {
+  Bank* bank = bank_of(particles);
+  TallyBatches* tb = flushed_batches(bank, BatchKind::kFlux, "nb200_bank_flux_batches");
+  if (!tb) return -3;
+  if (!out_device || ncells != tb->ncells) {
     set_error("nb200_bank_flux_batches: the flux batches cover %zu cells, %zu were asked for",
-              tb.ncells, ncells);
+              tb->ncells, ncells);
     return -3;
   }
-  DeviceGuard guard(bank->shards[0].dev);
-  DeviceCtx& c = ctx_on(bank->shards[0].dev);
-  c.launches += launch_batch_export(tb.slab, tb.B, tb.ncells, out_device, c.stream);
-  CU_TRY(cudaGetLastError());
-  CU_TRY(cudaStreamSynchronize(c.stream));
-  return tb.B;
+  return export_batches(bank, *tb, out_device);
 }
 
 extern "C" int nb200_bank_flux_relerr(nb200_particle_soa* particles, double* relerr_device,
                                       double* total_relerr_host) {
-  Bank* bank = flushed_flux_batches(particles, "nb200_bank_flux_relerr");
-  if (!bank) return -3;
-  const TallyBatches& tb = bank->flux_batches;
-  DeviceGuard guard(bank->shards[0].dev);
-  DeviceCtx& c = ctx_on(bank->shards[0].dev);
-  if (relerr_device) {
-    c.launches += launch_batch_relerr(tb.slab, tb.B, tb.ncells, bank->n, relerr_device, c.stream);
-    CU_TRY(cudaGetLastError());
-    CU_TRY(cudaStreamSynchronize(c.stream));
-  }
-  if (total_relerr_host) *total_relerr_host = batches_total_relerr(bank, tb);
-  return 0;
+  Bank* bank = bank_of(particles);
+  TallyBatches* tb = flushed_batches(bank, BatchKind::kFlux, "nb200_bank_flux_relerr");
+  if (!tb) return -3;
+  return batches_relerr(bank, *tb, relerr_device, 1, nullptr, total_relerr_host);
 }
 
 extern "C" int nb200_bank_group_flux_batches(nb200_particle_soa* particles, double* out_device,
                                              size_t ncells, int ngroups) {
   const char* who = "nb200_bank_group_flux_batches";
-  Bank* bank = flushed_flux_batches(particles, who, true);
-  if (!bank) return -3;
-  const TallyBatches& tb = bank->flux_batches;
-  if (!out_device || ncells != bank->flux_ncells || ngroups != bank->flux_groups) {
+  Bank* bank = bank_of(particles);
+  TallyBatches* tb = flushed_batches(bank, BatchKind::kGroupFlux, who);
+  if (!tb) return -3;
+  const FluxTally& f = bank->flux;
+  if (!out_device || ncells != f.ncells || ngroups != f.groups) {
     set_error("%s: the group flux batches cover %d groups of %zu cells, %d groups of %zu cells "
-              "were asked for", who, bank->flux_groups, bank->flux_ncells, ngroups, ncells);
+              "were asked for", who, f.groups, f.ncells, ngroups, ncells);
     return -3;
   }
-  DeviceGuard guard(bank->shards[0].dev);
-  DeviceCtx& c = ctx_on(bank->shards[0].dev);
-  c.launches += launch_batch_export(tb.slab, tb.B, tb.ncells, out_device, c.stream);
-  CU_TRY(cudaGetLastError());
-  CU_TRY(cudaStreamSynchronize(c.stream));
-  return tb.B;
+  return export_batches(bank, *tb, out_device);
 }
 
 extern "C" int nb200_bank_group_flux_relerr(nb200_particle_soa* particles, double* relerr_device,
                                             double* group_relerr_host, double* total_relerr_host) {
-  Bank* bank = flushed_flux_batches(particles, "nb200_bank_group_flux_relerr", true);
-  if (!bank) return -3;
-  const TallyBatches& tb = bank->flux_batches;
-  DeviceGuard guard(bank->shards[0].dev);
-  DeviceCtx& c = ctx_on(bank->shards[0].dev);
-  if (relerr_device) {
-    c.launches += launch_batch_relerr(tb.slab, tb.B, tb.ncells, bank->n, relerr_device, c.stream);
-    CU_TRY(cudaGetLastError());
-    CU_TRY(cudaStreamSynchronize(c.stream));
-  }
-  if (group_relerr_host || total_relerr_host) {
-    const double total = batches_total_relerr(bank, tb, bank->flux_groups, group_relerr_host);
-    if (total_relerr_host) *total_relerr_host = total;
-  }
-  return 0;
+  Bank* bank = bank_of(particles);
+  TallyBatches* tb = flushed_batches(bank, BatchKind::kGroupFlux, "nb200_bank_group_flux_relerr");
+  if (!tb) return -3;
+  return batches_relerr(bank, *tb, relerr_device, bank->flux.groups, group_relerr_host,
+                        total_relerr_host);
 }
 
 extern "C" int nb200_update_replicas(void) {

@@ -220,22 +220,25 @@ struct TallyBatches {
   bool deposited = false;    // a timestep has deposited into this slab
 };
 
+// The track-length flux a bank's timesteps also deposit into (nb200_bank_set_*flux_tally).
+struct FluxTally {
+  // the caller's flux array (device memory on the bank's GPU); null: none
+  double* target = nullptr;
+  size_t ncells = 0;  // the mesh's cells
+  // G > 0: `target` holds G energy groups of `ncells` cells each (group-major), whose G + 1
+  // edges are in `edges`, device memory the bank owns
+  int groups = 0;
+  double* edges = nullptr;
+  // B > 0 (the B of the bank's tally batches): the deposits go to B partial fluxes of
+  // max(G, 1) * ncells slots each instead; their target is `target`, their slab is allocated
+  // when the flux attaches
+  TallyBatches batches;
+};
+
 struct Bank {
   std::vector<Shard> shards;
   TallyBatches batches;
-  // nb200_bank_set_flux_tally: the caller's track-length flux array (device memory on the
-  // bank's GPU, flux_ncells doubles) every timestep also deposits into; null: none.
-  double* flux = nullptr;
-  size_t flux_ncells = 0;
-  // nb200_bank_set_batched_flux_tally: B > 0 (the B of `batches`) when the flux deposits go to
-  // B partial fluxes instead; their target is `flux`, their slab is allocated when it attaches.
-  TallyBatches flux_batches;
-  // nb200_bank_set_group_flux_tally: G > 0 when `flux` holds G energy groups of flux_ncells
-  // cells each (group-major); the G + 1 edges are in flux_edges, device memory the bank owns.
-  // With flux_batches too (nb200_bank_set_batched_group_flux_tally) the batches cover
-  // flux_batches.ncells = G * flux_ncells slots; flux_ncells stays the mesh's cell count.
-  double* flux_edges = nullptr;
-  int flux_groups = 0;
+  FluxTally flux;
   int n = 0;
   uint64_t pid0 = 0;
   int primary_dev = 0;

@@ -30,7 +30,8 @@
 //
 // Compiled with -fmad=false: the only fused operations are the explicit fma() of nb_log,
 // div_by_known and the cores.
-#include <type_traits>
+#include <cstdio>
+#include <cstdlib>
 #if defined(NB_ASSERT_BATCH_SLOT) || defined(NB_ASSERT_GROUP_SLOT)
 #include <cassert>
 #endif
@@ -124,50 +125,35 @@ extern "C" unsigned nb200_selftest_dispatch_group(unsigned cta, unsigned n_live,
   return dispatch_group(a, cta, n_live, n_coll);
 }
 
+// The parked state of a variant (ParkedAs): `Parked`, then one array per tally option the
+// variant has, in the order batch, flux, group. A mixin whose option is off is an empty base
+// and takes no space.
+//
 // kBatched (option tally_batches): every deposit goes to the partial tally of the particle's
 // batch (StepArgs::batch_slab). The batch follows from the global pid, once per history; it
 // is parked beside `origin` and turned into an address at each deposit.
-struct ParkedBatched : Parked {
-  int batch[kHistoryThreads];
-};
+template <bool> struct BatchPark {};
+template <> struct BatchPark<true> { int batch[kHistoryThreads]; };
+// kFlux (nb200_bank_set_flux_tally): every flight segment also adds w * length / ntotal to the
+// caller's flux array, at the places the energy deposits go. The track length of collisions
+// since the last flush is parked beside `edep` and flushed with it.
+template <bool> struct FluxPark {};
+template <> struct FluxPark<true> { double flux[kHistoryThreads]; };
+// kGroups with kFlux (nb200_bank_set_group_flux_tally): `flux` is G group-major arrays of the
+// mesh, and a segment goes to the group of the energy it flies with. The group is a property of
+// the flight: found by bisection at the start of the history and after every scatter, and
+// parked beside the flux. -1 (an energy outside the edges) deposits nothing.
+template <bool> struct GroupPark {};
+template <> struct GroupPark<true> { int group[kHistoryThreads]; };
+
+template <bool kBatched, bool kFlux, bool kGroups>
+struct ParkedAs : Parked, BatchPark<kBatched>, FluxPark<kFlux>, GroupPark<kGroups> {};
 
 template <bool kBatched, class P>
 __device__ __forceinline__ int parked_batch(const P& park) {
   if constexpr (kBatched) return park.batch[threadIdx.x];
   else return 0;
 }
-
-// Index of `cell` of batch b in the slab (32 bits: the host refuses B * ncells >= 2^31).
-__device__ __forceinline__ int batch_index(const StepArgs& a, const BatchArgs& bt, int b,
-                                           int cell) {
-  const int i = (int)batch_slot(b, (size_t)(unsigned)cell, bt.nbatches, (size_t)(a.nx * a.ny));
-#ifdef NB_ASSERT_BATCH_SLOT  // checking build: NB200_DEFINES=-DNB_ASSERT_BATCH_SLOT
-  assert(b >= 0 && b < bt.nbatches && cell >= 0 && cell < a.nx * a.ny && i >= 0 &&
-         i < bt.nbatches * a.nx * a.ny);
-#endif
-  return i;
-}
-
-// kFlux (nb200_bank_set_flux_tally): every flight segment also adds w * length / ntotal to the
-// caller's flux array, at the places the energy deposits go. The track length of collisions
-// since the last flush is parked beside `edep` and flushed with it.
-struct ParkedFlux : Parked {
-  double flux[kHistoryThreads];
-};
-
-// kBatched and kFlux together (nb200_bank_set_batched_flux_tally): `flux` is the library's flux
-// batch slab, indexed like the energy batches, and the flux parks beside the batch.
-struct ParkedBatchedFlux : ParkedBatched {
-  double flux[kHistoryThreads];
-};
-
-// kGroups with kFlux (nb200_bank_set_group_flux_tally): `flux` is G group-major arrays of the
-// mesh, and a segment goes to the group of the energy it flies with. The group is a property of
-// the flight: found by bisection at the start of the history and after every scatter, and
-// parked beside the flux. -1 (an energy outside the edges) deposits nothing.
-struct ParkedGroupFlux : ParkedFlux {
-  int group[kHistoryThreads];
-};
 
 template <bool kGroups, class P>
 __device__ __forceinline__ int parked_group(const P& park) {
@@ -193,54 +179,37 @@ __device__ __forceinline__ int energy_group(const GroupArgs& gr, double e) {
   return lo;
 }
 
-// Index of `cell` of group g in the flux array (32 bits: the host refuses G * ncells >= 2^31).
-__device__ __forceinline__ int group_index(const StepArgs& a, const GroupArgs& gr, int g,
-                                           int cell) {
+// Index of `cell` (of group g with kGroups) in the array a deposit goes to: i = g * ncells + cell
+// in the caller's G group-major arrays of the mesh, or with kBatched slot i of batch b in the
+// batch slab, batch_slot over G * ncells "cells", so that the batch sweeps of tally_batches.cu
+// serve a batched group flux as a batched flux of G * ncells cells. 32 bits: the host refuses
+// max(B, 1) * max(G, 1) * ncells >= 2^31.
+template <bool kBatched, bool kGroups>
+__device__ __forceinline__ int slot_index(const StepArgs& a, const BatchArgs& bt,
+                                          const GroupArgs& gr, int b, int g, int cell) {
   const int ncells = a.nx * a.ny;
-  const int i = g * ncells + cell;
-#ifdef NB_ASSERT_GROUP_SLOT  // checking build: NB200_DEFINES=-DNB_ASSERT_GROUP_SLOT
-  assert(g >= 0 && g < gr.ngroups && cell >= 0 && cell < ncells && i >= 0 &&
-         i < gr.ngroups * ncells);
-#endif
-  return i;
-}
-
-// kBatched, kFlux and kGroups together (nb200_bank_set_batched_group_flux_tally): `flux` is the
-// library's flux batch slab of B batches of G group-major arrays of the mesh; batch and group
-// park side by side.
-struct ParkedBatchedGroupFlux : ParkedBatchedFlux {
-  int group[kHistoryThreads];
-};
-
-// Index of `cell` of group g of batch b in that slab: batch_slot over G * ncells "cells", so
-// the batch sweeps of tally_batches.cu serve it as a batched flux of G * ncells cells (32 bits:
-// the host refuses B * G * ncells >= 2^31).
-__device__ __forceinline__ int batched_group_index(const StepArgs& a, const BatchArgs& bt,
-                                                   const GroupArgs& gr, int b, int g, int cell) {
-  const int ncells = a.nx * a.ny;
-  const int i = (int)batch_slot(b, (size_t)(unsigned)(g * ncells + cell), bt.nbatches,
-                                (size_t)(gr.ngroups * ncells));
+  const int i = kGroups ? g * ncells + cell : cell;
+  const int s = kBatched ? (int)batch_slot(b, (size_t)(unsigned)i, bt.nbatches,
+                                           (size_t)(kGroups ? gr.ngroups * ncells : ncells))
+                         : i;
 #if defined(NB_ASSERT_BATCH_SLOT) || defined(NB_ASSERT_GROUP_SLOT)
-  assert(b >= 0 && b < bt.nbatches && g >= 0 && g < gr.ngroups && cell >= 0 && cell < ncells &&
-         i >= 0 && (long long)i < (long long)bt.nbatches * gr.ngroups * ncells);
+  // checking build: NB200_DEFINES="-DNB_ASSERT_BATCH_SLOT -DNB_ASSERT_GROUP_SLOT"
+  const int B = kBatched ? bt.nbatches : 1, G = kGroups ? gr.ngroups : 1;
+  assert((!kBatched || (b >= 0 && b < B)) && (!kGroups || (g >= 0 && g < G)) && cell >= 0 &&
+         cell < ncells && s >= 0 && (long long)s < (long long)B * G * ncells);
 #endif
-  return i;
+  return s;
 }
 
 // `flux` is a kernel parameter behind the other three for the reason BatchArgs is one: a field
 // appended to StepArgs would move the offsets of the parameters that follow it; `grp` follows
 // `flux` for the same reason.
-template <bool kFastDiv, bool kPreReduce, bool kBatched, bool kFlux, bool kGroups = false>
+template <bool kFastDiv, bool kPreReduce, bool kBatched, bool kFlux, bool kGroups>
 __global__ void NB_HISTORY_BOUNDS
 k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs bt,
           double* __restrict__ flux, const GroupArgs grp) {
 #if NB_PARK_SMEM
-  __shared__ std::conditional_t<
-      kBatched,
-      std::conditional_t<kFlux, std::conditional_t<kGroups, ParkedBatchedGroupFlux, ParkedBatchedFlux>,
-                         ParkedBatched>,
-      std::conditional_t<kFlux, std::conditional_t<kGroups, ParkedGroupFlux, ParkedFlux>, Parked>>
-      park;
+  __shared__ ParkedAs<kBatched, kFlux, kGroups> park;
 #define PARKED(name) park.name[threadIdx.x]
 #define PARKED_BATCH parked_batch<kBatched>(park)
 #define PARKED_GROUP parked_group<kGroups>(park)
@@ -281,13 +250,11 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs
 #define NB_CELL (cy * a.nx + cx)  // tally / density index of the current cell
     // the base and index a deposit into `cell` goes to: the caller's tally, or the batch's slot
 #define NB_TALLY_AT(cell) \
-  (kBatched ? bt.slab : a.tally), (kBatched ? batch_index(a, bt, PARKED_BATCH, (cell)) : (cell))
+  (kBatched ? bt.slab : a.tally), slot_index<kBatched, false>(a, bt, grp, PARKED_BATCH, 0, (cell))
     // ... and a flux deposit: the caller's array (the group's slice of it for a group flux), or
     // (batched) the batch's slot of the flux slab (of the batch's group slice for a group flux)
-#define NB_FLUX_AT(cell)                                                                      \
-  flux, (kBatched && kGroups ? batched_group_index(a, bt, grp, PARKED_BATCH, PARKED_GROUP, (cell)) \
-         : kBatched          ? batch_index(a, bt, PARKED_BATCH, (cell))                       \
-         : kGroups           ? group_index(a, grp, PARKED_GROUP, (cell)) : (cell))
+#define NB_FLUX_AT(cell) \
+  flux, slot_index<kBatched, kGroups>(a, bt, grp, PARKED_BATCH, PARKED_GROUP, (cell))
     // ... through this, which makes no deposit while the particle is outside the energy groups
 #define NB_FLUX_ADD(cell, value)                                                    \
   do {                                                                              \
@@ -618,6 +585,25 @@ k_history(const StepArgs a, const unsigned* __restrict__ n_live, const BatchArgs
 
 static inline int blocks_for(int n, int threads) { return (n + threads - 1) / threads; }
 
+// Every instantiation of k_history, by its template arguments. Prereduction has one variant
+// (with the fast divisions, unbatched and without a flux); every other combination of the
+// options exists with and without the fast divisions.
+struct HistoryVariant {
+  bool fast_div, prereduce, batched, flux, groups;
+  void (*fn)(StepArgs, const unsigned*, BatchArgs, double*, GroupArgs);
+};
+#define NB_VARIANT(f, p, b, x, g) {f, p, b, x, g, &k_history<f, p, b, x, g>}
+static const HistoryVariant kHistoryVariants[] = {
+    NB_VARIANT(true, true, false, false, false),
+    NB_VARIANT(true, false, false, false, false),  NB_VARIANT(false, false, false, false, false),
+    NB_VARIANT(true, false, true, false, false),   NB_VARIANT(false, false, true, false, false),
+    NB_VARIANT(true, false, false, true, false),   NB_VARIANT(false, false, false, true, false),
+    NB_VARIANT(true, false, true, true, false),    NB_VARIANT(false, false, true, true, false),
+    NB_VARIANT(true, false, false, true, true),    NB_VARIANT(false, false, false, true, true),
+    NB_VARIANT(true, false, true, true, true),     NB_VARIANT(false, false, true, true, true),
+};
+#undef NB_VARIANT
+
 // `pin`/`pin_bytes` (optional) name the staged cross-section block: the launch then carries an
 // access-policy window that keeps it persisting in L2 (north_star phase 3), while the rest of
 // the kernel's traffic - the tally atomics above all - streams through the remainder.
@@ -635,19 +621,8 @@ int launch_history(const StepArgs& a, const BatchArgs& bt, double* flux, const G
     // the number of resident CTAs per SM without touching the code.
     static int granted = 0;
     if (smem_pad > granted) {
-      cudaFuncSetAttribute(k_history<true, true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
-      cudaFuncSetAttribute(k_history<true, false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
-      cudaFuncSetAttribute(k_history<false, false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
-      cudaFuncSetAttribute(k_history<true, false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
-      cudaFuncSetAttribute(k_history<false, false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
-      cudaFuncSetAttribute(k_history<true, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
-      cudaFuncSetAttribute(k_history<false, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
-      cudaFuncSetAttribute(k_history<true, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
-      cudaFuncSetAttribute(k_history<false, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
-      cudaFuncSetAttribute(k_history<true, false, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
-      cudaFuncSetAttribute(k_history<false, false, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
-      cudaFuncSetAttribute(k_history<true, false, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
-      cudaFuncSetAttribute(k_history<false, false, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
+      for (const HistoryVariant& v : kHistoryVariants)
+        cudaFuncSetAttribute(v.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_pad);
       granted = smem_pad;
     }
     cfg.dynamicSmemBytes = (size_t)smem_pad;
@@ -673,39 +648,22 @@ int launch_history(const StepArgs& a, const BatchArgs& bt, double* flux, const G
   // always batched (its `flux` is the flux batch slab). A group flux is never prereduced (the
   // host refuses it); on a batched bank it is always batched too, and either kernel is one more
   // switch of the same kind.
-  if (flux && grp.ngroups > 0 && bt.nbatches > 0) {
-    if (fast_div)
-      cudaLaunchKernelEx(&cfg, k_history<true, false, true, true, true>, a, n_live, bt, flux, grp);
-    else
-      cudaLaunchKernelEx(&cfg, k_history<false, false, true, true, true>, a, n_live, bt, flux, grp);
-  } else if (flux && grp.ngroups > 0) {
-    if (fast_div)
-      cudaLaunchKernelEx(&cfg, k_history<true, false, false, true, true>, a, n_live, bt, flux, grp);
-    else
-      cudaLaunchKernelEx(&cfg, k_history<false, false, false, true, true>, a, n_live, bt, flux, grp);
-  } else if (flux && bt.nbatches > 0) {
-    if (fast_div)
-      cudaLaunchKernelEx(&cfg, k_history<true, false, true, true>, a, n_live, bt, flux, grp);
-    else
-      cudaLaunchKernelEx(&cfg, k_history<false, false, true, true>, a, n_live, bt, flux, grp);
-  } else if (flux) {
-    if (fast_div)
-      cudaLaunchKernelEx(&cfg, k_history<true, false, false, true>, a, n_live, bt, flux, grp);
-    else
-      cudaLaunchKernelEx(&cfg, k_history<false, false, false, true>, a, n_live, bt, flux, grp);
-  } else if (bt.nbatches > 0) {
-    if (fast_div)
-      cudaLaunchKernelEx(&cfg, k_history<true, false, true, false>, a, n_live, bt, flux, grp);
-    else
-      cudaLaunchKernelEx(&cfg, k_history<false, false, true, false>, a, n_live, bt, flux, grp);
-  } else if (prereduce) {
-    cudaLaunchKernelEx(&cfg, k_history<true, true, false, false>, a, n_live, bt, flux, grp);
-  } else if (fast_div) {
-    cudaLaunchKernelEx(&cfg, k_history<true, false, false, false>, a, n_live, bt, flux, grp);
-  } else {
-    cudaLaunchKernelEx(&cfg, k_history<false, false, false, false>, a, n_live, bt, flux, grp);
+  // The key: energy edges without a flux array are ignored, batches or a flux override
+  // prereduce, and prereduce runs the fast divisions whatever fast_div says.
+  const bool batched = bt.nbatches > 0, fluxed = flux != nullptr;
+  const bool groups = fluxed && grp.ngroups > 0;
+  const bool pre = prereduce && !batched && !fluxed;
+  const bool fast = pre || fast_div;
+  for (const HistoryVariant& v : kHistoryVariants) {
+    if (v.fast_div == fast && v.prereduce == pre && v.batched == batched && v.flux == fluxed &&
+        v.groups == groups) {
+      cudaLaunchKernelEx(&cfg, v.fn, a, n_live, bt, flux, grp);
+      return 1;
+    }
   }
-  return 1;
+  // not reached: the table holds every key formed above
+  fprintf(stderr, "launch_history: no k_history variant for this key\n");
+  abort();
 }
 
 }  // namespace nb

@@ -462,33 +462,41 @@ class Simulation:
     def tally_to_host(self) -> np.ndarray:
         return self.tally.download()
 
+    def _batches_to_host(self, name: str, shape: tuple, *args) -> np.ndarray:
+        """``nb200_bank_<name>(bank, out, *args)``: the B partial arrays of one kind of batches,
+        exported into a scratch device buffer and downloaded as (B,) + ``shape``."""
+        out = DeviceArray(self.tally_batches * int(np.prod(shape)), np.float64)
+        try:
+            rc = getattr(self.lib, f"nb200_bank_{name}")(self.bank, out.ptr, *args)
+            if rc != self.tally_batches:
+                raise NeutralB200Error(f"bank_{name}: {self.lib.nb200_last_error().decode()}")
+            return out.download().reshape((self.tally_batches,) + shape)
+        finally:
+            out.free()
+
+    def _relative_error(self, name: str, shape: tuple, *args) -> Tuple[np.ndarray, float]:
+        """``nb200_bank_<name>(bank, relerr, *args, &total)``: (R per slot, downloaded as
+        ``shape``, R of the total)."""
+        out = DeviceArray(int(np.prod(shape)), np.float64)
+        total = C.c_double(0.0)
+        try:
+            _check(getattr(self.lib, f"nb200_bank_{name}")(self.bank, out.ptr, *args,
+                                                           C.byref(total)), f"bank_{name}")
+            return out.download().reshape(shape), float(total.value)
+        finally:
+            out.free()
+
     def tally_batches_to_host(self) -> np.ndarray:
         """(B, ny, nx) cumulative partial tallies of the B particle batches (option
         ``tally_batches``); flushes the caller's tally first."""
         d = self.problem.deck
-        ncells = d.nx * d.ny
-        out = DeviceArray(self.tally_batches * ncells, np.float64)
-        try:
-            rc = self.lib.nb200_bank_tally_batches(self.bank, out.ptr, ncells)
-            if rc != self.tally_batches:
-                raise NeutralB200Error(
-                    f"bank_tally_batches: {self.lib.nb200_last_error().decode()}")
-            return out.download().reshape(self.tally_batches, d.ny, d.nx)
-        finally:
-            out.free()
+        return self._batches_to_host("tally_batches", (d.ny, d.nx), d.nx * d.ny)
 
     def tally_relative_error(self) -> Tuple[np.ndarray, float]:
         """Relative error of the tally from its batches: (R per cell as (ny, nx), R of the
         tally total). R = sqrt(s^2 / B) / |m| over the batch estimates x_b = S_b N / n_b."""
         d = self.problem.deck
-        out = DeviceArray(d.nx * d.ny, np.float64)
-        total = C.c_double(0.0)
-        try:
-            _check(self.lib.nb200_bank_tally_relerr(self.bank, out.ptr, C.byref(total)),
-                   "bank_tally_relerr")
-            return out.download().reshape(d.ny, d.nx), float(total.value)
-        finally:
-            out.free()
+        return self._relative_error("tally_relerr", (d.ny, d.nx))
 
     def flux_to_host(self) -> np.ndarray:
         """(ny, nx) track length per source particle in every cell, summed over timesteps
@@ -520,16 +528,7 @@ class Simulation:
         """(B, ny, nx) cumulative partial fluxes of the B particle batches (``flux_tally=True``
         with ``tally_batches``); flushes the flux array first."""
         d = self.problem.deck
-        ncells = d.nx * d.ny
-        out = DeviceArray(self.tally_batches * ncells, np.float64)
-        try:
-            rc = self.lib.nb200_bank_flux_batches(self.bank, out.ptr, ncells)
-            if rc != self.tally_batches:
-                raise NeutralB200Error(
-                    f"bank_flux_batches: {self.lib.nb200_last_error().decode()}")
-            return out.download().reshape(self.tally_batches, d.ny, d.nx)
-        finally:
-            out.free()
+        return self._batches_to_host("flux_batches", (d.ny, d.nx), d.nx * d.ny)
 
     def flux_relative_error(self) -> Tuple[np.ndarray, float]:
         """Relative error of the flux from its batches: (R per cell as (ny, nx), R of the flux
@@ -537,30 +536,14 @@ class Simulation:
         same R per cell, because it divides every batch of a cell by the same exact constant,
         the cell's area."""
         d = self.problem.deck
-        out = DeviceArray(d.nx * d.ny, np.float64)
-        total = C.c_double(0.0)
-        try:
-            _check(self.lib.nb200_bank_flux_relerr(self.bank, out.ptr, C.byref(total)),
-                   "bank_flux_relerr")
-            return out.download().reshape(d.ny, d.nx), float(total.value)
-        finally:
-            out.free()
+        return self._relative_error("flux_relerr", (d.ny, d.nx))
 
     def group_flux_batches_to_host(self) -> np.ndarray:
         """(B, G, ny, nx) cumulative partial group fluxes of the B particle batches
         (``group_flux_batches=True``); flushes the group flux array first."""
         d = self.problem.deck
-        ncells = d.nx * d.ny
         G = self.flux_edges.size - 1
-        out = DeviceArray(self.tally_batches * G * ncells, np.float64)
-        try:
-            rc = self.lib.nb200_bank_group_flux_batches(self.bank, out.ptr, ncells, G)
-            if rc != self.tally_batches:
-                raise NeutralB200Error(
-                    f"bank_group_flux_batches: {self.lib.nb200_last_error().decode()}")
-            return out.download().reshape(self.tally_batches, G, d.ny, d.nx)
-        finally:
-            out.free()
+        return self._batches_to_host("group_flux_batches", (G, d.ny, d.nx), d.nx * d.ny, G)
 
     def group_flux_relative_error(self) -> Tuple[np.ndarray, np.ndarray, float]:
         """Relative error of the group flux from its batches (``group_flux_batches=True``):
@@ -569,16 +552,10 @@ class Simulation:
         group is the error bar of the spectrum."""
         d = self.problem.deck
         G = self.flux_edges.size - 1
-        out = DeviceArray(G * d.nx * d.ny, np.float64)
         groups = np.zeros(G)
-        total = C.c_double(0.0)
-        try:
-            _check(self.lib.nb200_bank_group_flux_relerr(self.bank, out.ptr, groups.ctypes.data,
-                                                         C.byref(total)),
-                   "bank_group_flux_relerr")
-            return out.download().reshape(G, d.ny, d.nx), groups, float(total.value)
-        finally:
-            out.free()
+        per_cell, total = self._relative_error("group_flux_relerr", (G, d.ny, d.nx),
+                                               groups.ctypes.data)
+        return per_cell, groups, total
 
     def counters_to_host(self) -> np.ndarray:
         """(3, count) cumulative per-particle facets / collisions / census events."""
